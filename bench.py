@@ -9,7 +9,9 @@ with NCCL all-reduce when N > 1.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
 
-Prints ONE JSON line (rank 0).  `value` is device-timed with inputs resident in HBM; `e2e` goes
+Prints ONE JSON line (rank 0).  `--dump-outputs DIR` also writes what the resident step returned in its last timed
+step as DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output.
+`value` is device-timed with inputs resident in HBM; `e2e` goes
 through the public Python API with the per-step inputs -- every view's camera and fp32 [3,H,W]
 ground-truth image, what the reference moves per step at train.py:377 -- copied from pinned host
 memory, an L1 loss against that image (train.py:384) and the loss scalar read back, inside the timed region.  `--impl reference` times the CPU restatement of the reference
@@ -24,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "fwd+bwd frames/sec @1M Gaussians 1080p"
 UNIT = "frames/s"
@@ -73,7 +76,13 @@ def parse():
     ap.add_argument("--grad-allreduce", default="auto", choices=["auto", "nvls", "nccl"],
                     help="N > 1: sum the gradients with the library's in-switch kernel (GradArena), with NCCL, or "
                          "(auto) time both and keep the faster")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the resident step returned in its last timed step (images, radii and parameter "
+                         "gradients at a fixed, seeded sample of pixels and Gaussians) as DIR/<name>.npy, float32")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be >= 1")
+    return a
 
 
 def load_peaks():
@@ -278,6 +287,7 @@ class RasterWorkload:
         self.reduced = [self.params[k] for k in names] + ([self.extra] if fused_feat else [])   # all-reduced gradients
         self.grads = self.reduced + [self.means2D]
         self.allreduce = True
+        self.keep_step, self.kept = None, None
         self._e2e_ready = False
         # N > 1: the step's gradient buffer lives in symmetric memory and is summed by our own in-switch kernel
         self.arena = None
@@ -302,27 +312,35 @@ class RasterWorkload:
         from opengaussian_b200.rasterizer import GaussianRasterizer
         if self.fused_feat:
             color, radii, depth, alpha, feat = GaussianRasterizer(rs)(means2D=self.means2D, extra_feats=self.extra, **self.params)
-            return color, feat, depth, alpha
+            return color, feat, depth, alpha, radii
         color, radii, depth, alpha = GaussianRasterizer(rs)(means2D=self.means2D, **self.params)
-        return color, None, depth, alpha
+        return color, None, depth, alpha, radii
 
     def _grad_outputs(self, outs, Gd):
-        color, feat, depth, alpha = outs
+        color, feat, depth, alpha = outs[:4]
         C = self.C
         if feat is None:
             return (color, depth, alpha), (Gd[0:3], Gd[C:C + 1], Gd[C + 1:C + 2])
         return (color, feat, depth, alpha), (Gd[0:3], Gd[3:C], Gd[C:C + 1], Gd[C + 1:C + 2])
 
     def step(self, i):
+        """Step i renders views (i * V + v) % len(settings).  Step `keep_step` keeps every view's forward outputs in
+        `kept` (references only: no copy, nothing synchronised)."""
         from opengaussian_b200.dist import render_views_backward
         self.zero_grads()
         V = self.V
+        kept = {} if i == self.keep_step else None
 
         def view(v):
-            return self._grad_outputs(self._call(self.settings[(i * V + v) % len(self.settings)]), self.G)
+            outs = self._call(self.settings[(i * V + v) % len(self.settings)])
+            if kept is not None:
+                kept[v] = outs
+            return self._grad_outputs(outs, self.G)
 
         render_views_backward(view, list(range(V)), self.reduced, already_split=True, streams=self.S,
                               reduce=self.allreduce)
+        if kept is not None:
+            self.kept = [kept[v] for v in range(V)]
 
     # ---- end to end ----
     def _e2e_setup(self):
@@ -428,6 +446,38 @@ class RasterWorkload:
         return out
 
 
+DUMP_BYTES = 60_000_000      # --dump-outputs: at most this much in all, half for the pixel arrays, half per Gaussian
+
+
+def dump_outputs(wl, out_dir):
+    """Writes what the kept step returned to its caller as float32 DIR/<name>.npy: per view `color` [V,3,S], `feat`
+    [V,F,S] (fused feature channels only), `depth` and `alpha` [V,1,S] at S pixels, per view `radii` [V,G], and
+    `grad_<input>` [G,...] of every rasterizer input at G Gaussians.  The pixels and Gaussians are a seeded sample
+    (all of them when they fit DUMP_BYTES): a function of the workload and --views-per-step only."""
+    import numpy as np
+    torch = wl.cx.torch
+    outs = [tuple(None if t is None else t.detach() for t in o) for o in wl.kept]   # the images are autograd outputs
+    images = {nm: torch.stack([o[k] for o in outs]).flatten(2)
+              for k, nm in enumerate(("color", "feat", "depth", "alpha")) if outs[0][k] is not None}
+    inputs = dict(wl.params, means2D=wl.means2D, **({"ins_feat": wl.extra} if wl.extra is not None else {}))
+    grads = {nm: t.grad for nm, t in inputs.items() if t.grad is not None}
+    rng = np.random.default_rng(0)
+
+    def sample(n, floats_per_item):
+        m = min(n, DUMP_BYTES // 2 // (4 * floats_per_item))
+        idx = np.arange(n) if m == n else np.sort(rng.choice(n, m, replace=False))
+        return torch.from_numpy(idx).to(wl.cx.dev)
+
+    px = sample(wl.H * wl.W, sum(t.shape[0] * t.shape[1] for t in images.values()))
+    gs = sample(wl.P, len(outs) + sum(t[0].numel() for t in grads.values()))
+    arrays = {nm: t[:, :, px] for nm, t in images.items()}
+    arrays["radii"] = torch.stack([o[4] for o in outs])[:, gs]
+    arrays.update({"grad_" + nm: t[gs] for nm, t in grads.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for nm, t in arrays.items():
+        np.save(os.path.join(out_dir, nm + ".npy"), t.float().cpu().numpy())
+
+
 def raster_headline(cx, a):
     """The BASELINE metric: fwd+bwd frames/s at 1 M Gaussians, 1080p -- resident, end to end, roofline, breakdown."""
     import gc
@@ -471,11 +521,20 @@ def raster_headline(cx, a):
         for _ in range(2):
             wl.step(i)
             i += 1
+    # the timed region starts on the first camera however many settle steps the allocator took, so that its last
+    # step renders the same views in every run
+    i += -i % len(wl.settings)
+    if a.dump_outputs:
+        wl.keep_step = i + R * K - 1
     _lib.profile_enable(not a.no_profile)
     _lib.profile_read()
     times, i = cx.timed_repeats(wl.step, i, K, R)
     prof = _lib.profile_read()
     _lib.profile_enable(False)
+    if a.dump_outputs:
+        if cx.rank == 0:
+            dump_outputs(wl, a.dump_outputs)
+        wl.keep_step, wl.kept = None, None
     if a.no_profile:
         _lib.profile_enable(True)
         for _ in range(K):

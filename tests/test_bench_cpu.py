@@ -37,6 +37,53 @@ def test_reference_arm_other_ranks_exit_silently():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_sample_and_budget(tmp_path, monkeypatch):
+    """--dump-outputs: float32 files of the kept step's outputs and gradients, the same seeded sample of pixels and
+    Gaussians on every call, everything when it fits, and never more than DUMP_BYTES."""
+    import types
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    P, H, W, V = 5000, 40, 60, 3
+    g = torch.Generator().manual_seed(0)
+    params = {k: torch.zeros(P, *s) for k, s in (("means3D", (3,)), ("opacities", (1,)), ("shs", (16, 3)),
+                                                  ("scales", (3,)), ("rotations", (4,)))}
+    for t in params.values():
+        t.grad = torch.randn(t.shape, generator=g)
+    means2D = torch.zeros(P, 3)
+    means2D.grad = torch.randn(P, 3, generator=g)
+
+    def out(*shape):            # what the rasterizer returns: a non-leaf tensor attached to the autograd graph
+        return torch.randn(*shape, generator=g).requires_grad_(True) * 1.0
+
+    kept = [(out(3, H, W), None, out(1, H, W), out(1, H, W), torch.randint(0, 9, (P,), generator=g, dtype=torch.int32))
+            for _ in range(V)]
+    wl = types.SimpleNamespace(cx=types.SimpleNamespace(torch=torch, dev=torch.device("cpu")), kept=kept, params=params,
+                               means2D=means2D, extra=None, P=P, H=H, W=W)
+
+    def load(d):
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+
+    bench.dump_outputs(wl, str(tmp_path / "all"))
+    full = load(tmp_path / "all")
+    assert sorted(full) == ["alpha", "color", "depth", "grad_means2D", "grad_means3D", "grad_opacities", "grad_rotations",
+                            "grad_scales", "grad_shs", "radii"]
+    assert all(a.dtype == np.float32 for a in full.values())
+    assert np.array_equal(full["color"], torch.stack([k[0] for k in kept]).flatten(2).detach().numpy())
+    assert np.array_equal(full["radii"], torch.stack([k[4] for k in kept]).float().numpy())
+    assert np.array_equal(full["grad_shs"], params["shs"].grad.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 200_000)
+    for d in ("a", "b"):
+        bench.dump_outputs(wl, str(tmp_path / d))
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    assert sum(x.nbytes for x in a.values()) <= 200_000
+    assert a["color"].shape[:2] == (V, 3) and 0 < a["color"].shape[2] < H * W
+    assert a["grad_shs"].shape[1:] == (16, 3) and 0 < a["grad_shs"].shape[0] < P
+    assert np.isin(a["grad_shs"].reshape(-1), full["grad_shs"].reshape(-1)).all()
+
+
 def test_algorithmic_bytes_worked_example():
     """SURVEY.md section 8d's worked example: P = P_vis = 1 M, N = 8 M, 1080p, C = 3, degree 3, 45 key bits."""
     sys.path.insert(0, ROOT)
