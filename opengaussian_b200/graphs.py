@@ -16,8 +16,15 @@ parameters' CURRENT VALUES and tensors that stay alive at the same address (came
 its Python side effects happen only on the eager and the capturing visit.  Parameters are read in place, so optimizer
 steps are seen; a parameter that is REPLACED by a new tensor (or any change the ``guard`` reports, e.g. the geometry's
 version counters) drops the graphs and starts over.  Gradients are written, not accumulated: after the call
-``p.grad`` is this view's gradient (the graph's own buffer, valid until the same view is replayed again);
-``step(view, accumulate=True)`` adds it to an existing ``.grad`` instead (the 2nd..Vth view of a multi-view step).
+``p.grad`` is this view's gradient in a tensor of its own, as after an eager backward; ``step(view, accumulate=True)``
+adds it to an existing ``.grad`` instead (the 2nd..Vth view of a multi-view step, in any order, or every view after
+``optimizer.zero_grad(set_to_none=False)``).  The returned loss is a tensor of its own as well.  A replay's outputs
+are copied out of the graph before the call returns (one read and one write of each gradient: 48 MB of traffic at
+1 M Gaussians x 6 channels), so no ``.grad`` and no loss the caller holds is ever a graph's buffer -- which a later
+replay of that graph, or of another graph whose intermediates share its memory, would overwrite.  That is also why
+every view's graph can share one memory pool: the graphs never run concurrently and nothing they write outlives the
+call, so the step keeps one set of intermediates instead of one per camera.  Camera matrices, like the parameters, are read in place: a camera edited in place needs ``reset()`` (or a
+``guard`` that reports it).
 Anything that cannot be captured -- a view whose geometry is not resident (cache disabled or over budget), trainable
 geometry (the forward then has to read the frame's duplicate count back) -- runs eagerly, every time, with the same
 results."""
@@ -85,7 +92,7 @@ class GraphedViewStep:
     def _capture(self, view, sig):
         dev = self.params[0].device
         if self._pool is None:
-            self._pool = torch.cuda.graph_pool_handle()   # one pool for every view's graph: they never run concurrently
+            self._pool = torch.cuda.graph_pool_handle()   # one pool for every view's graph (see the module docstring)
         for p in self.params:
             p.grad = None
         g = _Graph()
@@ -146,8 +153,11 @@ class GraphedViewStep:
         g.graph.replay()
         self.replays += 1
         for p, gr in zip(self.params, g.grads):
-            if accumulate and p.grad is not None and gr is not None and p.grad is not gr:
+            if gr is None:
+                if not accumulate:
+                    p.grad = None
+            elif accumulate and p.grad is not None:
                 p.grad.add_(gr)
             else:
-                p.grad = gr
-        return g.loss
+                p.grad = gr.clone()
+        return g.loss.clone()

@@ -93,6 +93,38 @@ def _sig(t):
     return None if t is None else (t.data_ptr(), t._version, tuple(t.shape), tuple(t.stride()))
 
 
+_CAM_COPIES = collections.OrderedDict()   # _sig(source) + dtype -> (contiguous fp32 copy, source), least recently used first
+_CAM_COPIES_MAX = 4096                     # three matrices per camera at most; a copy costs one 512-byte block
+
+
+def camera_inputs(viewmatrix, projmatrix, campos):
+    """The camera part of a forward: ``(key, (viewmatrix, projmatrix, campos))`` -- the key taken from the CALLER's
+    tensors (storage, version counter, shape, stride: the rule the geometry follows), the tensors as the C ABI needs them
+    (contiguous float32).  The reference builds ``world_view_transform`` and the projection matrix transposed
+    (scene/cameras.py:71-73), i.e. non-contiguous: their copies are made once per source tensor and reused while the
+    source is unchanged, so the key, and the address a captured graph reads, repeat from one step to the next.  An
+    in-place edit of the source (or of its base) bumps its version: new key, fresh copy."""
+    key = (_sig(viewmatrix), _sig(projmatrix), _sig(campos))
+    out = []
+    for t, sig in zip((viewmatrix, projmatrix, campos), key):
+        if t is None or (t.dtype == torch.float32 and t.is_contiguous()):
+            out.append(t)
+            continue
+        sig = sig + (t.dtype,)
+        hit = _CAM_COPIES.get(sig)
+        if hit is not None:
+            _CAM_COPIES.move_to_end(sig)
+            out.append(hit[0])
+            continue
+        c = _f32c(t)
+        if not (c.is_cuda and torch.cuda.is_current_stream_capturing()):   # a copy made inside a capture is the graph's
+            _CAM_COPIES[sig] = (c, t)                                        # own memory: never handed out again
+            while len(_CAM_COPIES) > _CAM_COPIES_MAX:
+                _CAM_COPIES.popitem(last=False)
+        out.append(c)
+    return key, tuple(out)
+
+
 def pin_for_capture(device, *tensors):
     """While graphs.GraphedViewStep captures on `device`, remembers `tensors` (library-internal cached buffers the
     captured kernels read) for as long as the graph lives; a no-op otherwise."""
@@ -121,10 +153,10 @@ class ViewCache:
     fill an entry at once; forwards on activated tensors only when the same tensors arrive twice in a row
     (`second_sighting`) -- the getters, the Stage-2 rescale draw and the cluster filters build new tensors per call.
 
-    Validity is decided from what torch guarantees: an entry is keyed by the camera tensors and matched against the
-    geometry tensors' storage address, shape and VERSION COUNTER (bumped by every in-place op, shared by detach()
-    and views -- so the per-iteration `.detach()` of train.py:431-436 still hits, an optimizer step or a densification
-    misses).  The entry holds references to those tensors, so an address cannot be recycled while it is alive.
+    Validity is decided from what torch guarantees: an entry is keyed by the caller's camera tensors (camera_inputs;
+    the reference's transposed matrices included) and matched against the geometry tensors' storage address, shape and
+    VERSION COUNTER (bumped by every in-place op, shared by detach() and views -- so the per-iteration `.detach()` of
+    train.py:431-436 still hits, an optimizer step or a densification misses).  The entry holds references to those tensors, so an address cannot be recycled while it is alive.
     NOT seen: writes through `tensor.data` or raw pointers -- call `view_cache.clear()` after such edits, or set
     `view_cache.enabled = False` (env OGS_VIEW_CACHE=0; per call: `pipe.view_cache = False` in render()).  The `radii`
     a cache hit returns alias the entry's copy: read-only, as every caller in the reference treats them."""
@@ -173,9 +205,14 @@ class ViewCache:
                     evictions=self.evictions, max_bytes=self.max_bytes)
 
     @staticmethod
-    def keys(rs, means3D, opacities, sh, sh_rest, colors_precomp, scales, rotations, cov3D, act_flags, n_feat_act):
+    def keys(rs, means3D, opacities, sh, sh_rest, colors_precomp, scales, rotations, cov3D, act_flags, n_feat_act,
+             cam_key=None):
+        """(camera key, geometry key) of a forward; ``cam_key`` is camera_inputs()'s key of the caller's camera tensors
+        (default: taken from ``rs``)."""
         dev = means3D.device
-        cam = (dev.type, dev.index, _sig(rs.viewmatrix), _sig(rs.projmatrix), _sig(rs.campos), int(rs.image_height),
+        if cam_key is None:
+            cam_key = (_sig(rs.viewmatrix), _sig(rs.projmatrix), _sig(rs.campos))
+        cam = (dev.type, dev.index) + cam_key + (int(rs.image_height),
                int(rs.image_width), float(rs.tanfovx), float(rs.tanfovy), float(rs.scale_modifier),
                int(rs.sh_degree) if sh is not None else -1, bool(int(act_flags) & ~_lib.ACT_EXTRA_UNIT_HALF))
         geom = (_sig(means3D), _sig(opacities), _sig(sh), _sig(sh_rest), colors_precomp is not None, _sig(scales),
@@ -398,7 +435,9 @@ class _RasterizeGaussians(torch.autograd.Function):
                 _BG_FULL[dev.index] = hit
             bg_full = hit[1]
             pin_for_capture(dev, bg_full)
-        rs = rs._replace(viewmatrix=_f32c(rs.viewmatrix), projmatrix=_f32c(rs.projmatrix), campos=_f32c(rs.campos))
+        cam_src = (rs.viewmatrix, rs.projmatrix, rs.campos)
+        cam_sig, cam = camera_inputs(*cam_src)
+        rs = rs._replace(viewmatrix=cam[0], projmatrix=cam[1], campos=cam[2])
 
         color_all = torch.empty(3 + n_extra, H, W, dtype=torch.float32, device=dev)
         depth = torch.empty(1, H, W, dtype=torch.float32, device=dev)
@@ -418,11 +457,10 @@ class _RasterizeGaussians(torch.autograd.Function):
         if frozen:
             n_feat_act = n_extra if (act_flags & _lib.ACT_EXTRA_UNIT_HALF) else 0
             cam_key, geom_key = ViewCache.keys(rs, means3D, opacities, sh, sh_rest, colors_precomp, scales, rotations,
-                                               cov3Ds_precomp, act_flags, n_feat_act)
+                                               cov3Ds_precomp, act_flags, n_feat_act, cam_key=cam_sig)
             entry = view_cache.lookup(cam_key, geom_key)
             if entry is None:
-                keep = (rs.viewmatrix, rs.projmatrix, rs.campos, means3D, opacities, sh, sh_rest, scales, rotations,
-                        cov3Ds_precomp)
+                keep = cam_src + cam + (means3D, opacities, sh, sh_rest, scales, rotations, cov3Ds_precomp)
                 admit = bool(act_flags & ~_lib.ACT_EXTRA_UNIT_HALF) or \
                     view_cache.second_sighting(dev.index, (cam_key, geom_key), keep)
         if entry is None and torch.cuda.is_current_stream_capturing():
@@ -430,7 +468,7 @@ class _RasterizeGaussians(torch.autograd.Function):
                                 "rasterizer.view_cache (frozen geometry, one eager visit first): a fresh forward reads "
                                 "the frame's duplicate count back to the host")
         if entry is not None:
-            pin_for_capture(dev, entry.geom, entry.binning, entry.radii)   # an evicted entry must not free what a graph reads
+            pin_for_capture(dev, entry.geom, entry.binning, entry.radii, *cam)   # an evicted entry must not free what a graph reads
             radii = entry.radii.detach()     # a fresh tensor object over the first call's radii (this Function's own output)
             ro = _lib.RasterOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha), None)
             with torch.cuda.device(dev):

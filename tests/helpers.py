@@ -38,3 +38,38 @@ def grad_violations(got, want, rtol=1e-3):
     tol = rtol * np.abs(want) + rtol * rms + 1e-30
     ratio = np.abs(got - want) / tol
     return float((ratio > 1.0).mean()), float(ratio.max())
+
+
+def separation_loss_fp64(mean, iteration, rows=slice(None)):
+    """train.py:123-155 (separation_loss) restated with the loss in float64, differentiable w.r.t. `mean` by autograd.
+    The rank weights are computed as the reference computes them (`sorted_indices.float()`: float32), the ranks by a
+    STABLE argsort, i.e. ties by column -- the CUDA kernel's rule; the reference's unstable argsort may order exact ties
+    either way, which changes neither the value nor, for identical rows, the total gradient.  `rows` restricts the sum
+    to those rows of the [N, N] matrix (each row's weights depend on that row only), so that a large N can be
+    evaluated and differentiated a block of rows at a time; the slices' sums add up to the loss."""
+    m = mean.double()
+    N = m.shape[0]
+    r = torch.arange(N)[rows]
+    inv = 1.0 / ((m[r, None, :] - m[None, :, :]).pow(2).sum(2) + 1)
+    inv = inv.masked_fill(r[:, None] == torch.arange(N)[None, :], 0)
+    ranks = inv.detach().argsort(dim=1, stable=True).argsort(dim=1)
+    w = (ranks.float() / (N - 1)) * (1.0 - 0.1) + 0.1
+    if iteration is not None and iteration > 35000:
+        w[w < 0.9] = 0.1
+    return (inv * w.double()).sum() / (N * (N - 1))
+
+
+def min_rank_gap(mean, rows=slice(None)):
+    """Smallest relative gap between two DISTINCT inverse distances 1 / (|m_i - m_j|^2 + 1) within a row of `mean`
+    (float64): above ~1e-6 no float32 rounding can reorder them, so the float32 kernel and a float64 reference rank
+    every row the same way."""
+    m = mean.double()
+    N = m.shape[0]
+    r = torch.arange(N)[rows]
+    inv = 1.0 / ((m[r, None, :] - m[None, :, :]).pow(2).sum(2) + 1)
+    inv = inv.masked_fill(r[:, None] == torch.arange(N)[None, :], 0)
+    s = inv.sort(dim=1).values
+    lo, hi = s[:, :-1], s[:, 1:]
+    gap = (hi - lo) / hi.clamp(min=1e-300)
+    gap = gap[hi != lo]
+    return float(gap.min()) if gap.numel() else float("inf")

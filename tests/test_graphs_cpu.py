@@ -95,3 +95,56 @@ def test_accumulate_adds_into_existing_grad():
         st(5.0, accumulate=True)
         assert torch.equal(w.grad, first + 5.0), rep
     assert st.stats()["graphs"] == 2
+
+
+def test_accumulate_in_any_order_across_eager_capture_and_replay():
+    """A, B(acc), A(acc): a replayed view that finds its own earlier output in .grad must still add to it."""
+    w = torch.tensor([1.0, -1.0], requires_grad=True)
+    st = _Step(lambda v: (w * v).sum(), [w])
+    for rep in range(4):                               # eager, capture + replay, replay, replay
+        st(1.0)
+        st(5.0, accumulate=True)
+        st(1.0, accumulate=True)
+        assert torch.equal(w.grad, torch.full((2,), 7.0)), (rep, w.grad)
+    assert st.stats()["graphs"] == 2 and st.stats()["replays"] >= 6
+
+
+def test_zero_grad_then_accumulate_every_view_in_changing_orders():
+    """optimizer.zero_grad() (both forms) and then step(v, accumulate=True) for every view, in a new order each step --
+    from the start, and after single-view steps (accumulate=False) have visited and captured every view."""
+    w = torch.tensor([1.0, 2.0, -1.0], requires_grad=True)
+    views = (1.0, 2.0, 3.0, 4.0)
+    orders = [(0, 1, 2, 3), (3, 2, 1, 0), (1, 3, 0, 2), (2, 0, 3, 1), (0, 2, 1, 3), (3, 1, 2, 0)]
+    for set_to_none in (False, True):
+        for single_view_first in (False, True):
+            w.grad = None
+            st = _Step(lambda v: (w * w).sum() * v, [w])
+            opt = torch.optim.SGD([w], lr=0.0)
+            if single_view_first:
+                for v in views + views:
+                    st(v)
+            for k, order in enumerate(orders):             # eager, capture, then replays
+                opt.zero_grad(set_to_none=set_to_none)
+                for i in order:
+                    st(views[i], accumulate=True)
+                assert torch.equal(w.grad, 2.0 * w.detach() * sum(views)), (set_to_none, single_view_first, k, w.grad)
+            assert st.stats()["graphs"] == 4
+
+
+def test_returned_loss_and_grad_outlive_later_replays():
+    """A loss (or a .grad) the caller keeps is not overwritten by later steps, of the same view or another one."""
+    w = torch.tensor([1.0, 2.0], requires_grad=True)
+    st = _Step(lambda v: (w * w).sum() * v, [w])
+    for _ in range(2):                                 # eager, capture: the graphs exist from here on
+        st(1.0)
+        st(2.0)
+    kept = []
+    for scale in (1.0, 2.0, 3.0):
+        with torch.no_grad():
+            w.copy_(torch.tensor([1.0, 2.0]) * scale)
+        for v in (1.0, 2.0):
+            loss = st(v)
+            kept.append((loss, float(loss), w.grad, w.grad.clone()))
+    assert st.stats()["replays"] >= 7
+    for loss, value, grad, grad_value in kept:
+        assert float(loss) == value and torch.equal(grad, grad_value)

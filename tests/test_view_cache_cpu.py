@@ -5,7 +5,7 @@ import types
 
 import torch
 
-from opengaussian_b200.rasterizer import GaussianRasterizationSettings, ViewCache, _sig, _ViewEntry
+from opengaussian_b200.rasterizer import GaussianRasterizationSettings, ViewCache, _sig, _ViewEntry, camera_inputs
 
 
 def _rs(view, proj, campos, sh_degree=3):
@@ -93,3 +93,62 @@ def test_activated_tensors_are_admitted_on_their_second_sighting_only():
     g = _geo()
     assert _keys(_rs(view, proj, pos), g, act=7)[0] != _keys(_rs(view, proj, pos), g, act=0)[0]
     assert _keys(_rs(view, proj, pos), g, act=7)[0] == _keys(_rs(view, proj, pos), g, act=7 | 8)[0]
+
+
+def _reference_camera(seed=0):
+    """Camera tensors as scene/cameras.py:71-73 builds them: transposed (non-contiguous) view and projection, their
+    product, the centre row of the inverse."""
+    g = torch.Generator().manual_seed(seed)
+    w2v = torch.eye(4)
+    w2v[:3, :3] = torch.linalg.qr(torch.randn(3, 3, generator=g))[0]
+    w2v[:3, 3] = torch.randn(3, generator=g)
+    view = torch.tensor(w2v.numpy()).transpose(0, 1)
+    proj = torch.rand(4, 4, generator=g).transpose(0, 1)
+    full = view.unsqueeze(0).bmm(proj.unsqueeze(0)).squeeze(0)
+    return view, full, view.inverse()[3, :3]
+
+
+def test_reference_camera_key_repeats_and_its_copy_is_reused():
+    view, full, centre = _reference_camera()
+    assert not view.is_contiguous() and not centre.is_contiguous()     # inverse() returns a column-major matrix
+    key, (v, p, c) = camera_inputs(view, full, centre)
+    assert v.is_contiguous() and v.dtype == torch.float32 and torch.equal(v, view)
+    assert c.is_contiguous() and torch.equal(c, centre)
+    assert p is full                                   # already what the C ABI takes: no copy
+    for _ in range(3):
+        key2, (v2, p2, c2) = camera_inputs(view, full, centre)
+        assert key2 == key and v2 is v and p2 is p and c2 is c
+    assert camera_inputs(view.detach(), full, centre)[0] == key   # another tensor object over the same contents
+    # the key is the one ViewCache.keys takes from the caller's settings, not from the copy
+    g = _geo()
+    assert _keys(_rs(view, full, centre), g)[0] == ViewCache.keys(
+        _rs(v, p, c), g.means3D, g.opacities, g.sh, g.sh_rest, None, g.scales, g.rotations, None, 7, 6, cam_key=key)[0]
+    assert _keys(_rs(v, p, c), g)[0] != _keys(_rs(view, full, centre), g)[0]
+    # a float64 camera: one float32 copy, reused
+    d = view.double()
+    k64, (v64, _, _) = camera_inputs(d, full, centre)
+    assert v64.dtype == torch.float32 and camera_inputs(d, full, centre)[1][0] is v64 and k64 != key
+
+
+def test_in_place_camera_edit_gives_a_new_key_and_a_fresh_copy():
+    view, full, centre = _reference_camera(1)
+    key, (v, _, _) = camera_inputs(view, full, centre)
+    before = v.clone()
+    view.mul_(2.0)                                      # through the transposed tensor
+    key2, (v2, _, _) = camera_inputs(view, full, centre)
+    assert key2 != key and v2 is not v and torch.equal(v2, view) and torch.equal(v, before)
+    view._base.add_(1.0)                                 # through its base: the version counter is shared
+    key3, (v3, _, _) = camera_inputs(view, full, centre)
+    assert key3 not in (key, key2) and torch.equal(v3, view)
+    full.sub_(0.5)                                      # a contiguous matrix is keyed the same way
+    key4, (_, p4, _) = camera_inputs(view, full, centre)
+    assert key4 != key3 and p4 is full and camera_inputs(view, full, centre)[0] == key4
+
+
+def test_equal_values_in_a_new_camera_tensor_are_a_new_key():
+    view, full, centre = _reference_camera(2)
+    key, (v, _, _) = camera_inputs(view, full, centre)
+    twin = view._base.clone().transpose(0, 1)            # same values, new storage (a re-created Camera)
+    key2, (v2, _, _) = camera_inputs(twin, full, centre)
+    assert key2 != key and v2 is not v and torch.equal(v2, v)
+    assert camera_inputs(view, full, centre)[0] == key and camera_inputs(view, full, centre)[1][0] is v
