@@ -26,9 +26,7 @@
  *   ogs_kmeans_assign            scene/kmeans_quantize.py:38-55 (get_dist) + :181-182,:200-201,
  *                                :223-224,:237-238 (argmin) fused with :82-87,:183-187,:202-205
  *                                (one-hot centroid sums and counts)
- *   ogs_kmeans_finalize          scene/kmeans_quantize.py:208-214 (centres = sums / counts, reset)
  *   ogs_kmeans_gather_st         scene/kmeans_quantize.py:273-275 (gather centres, straight-through)
- *   ogs_kmeans_count             scene/kmeans_quantize.py:89-144 (equalize_cluster_size member counts)
  *   ogs_kmeans_assign_segmented, ogs_kmeans_finalize_fixed
  *                                scene/kmeans_quantize.py:196-214,233-238 (leaf mode) for all coarse clusters at once
  *   ogs_multimem_allreduce_f32   no reference counterpart: the view-parallel step's gradient all-reduce, reduced inside
@@ -58,7 +56,7 @@
 extern "C" {
 #endif
 
-#define OGS_ABI_VERSION 6
+#define OGS_ABI_VERSION 7
 #define OGS_TILE 16
 #define OGS_MAX_CHANNELS 16 /* 3 colour channels + n_extra <= OGS_MAX_CHANNELS */
 
@@ -229,17 +227,10 @@ int ogs_kmeans_assign(int64_t N, const float* a, int32_t Da, const float* b, int
                       int64_t selected, int64_t id_offset, int64_t* ids_out, float* sums,
                       float* counts, void* stream);
 
-/* centers_out[j, :] = sums[j, :] / (counts[j] + eps_count)  for j in [0, k). */
-int ogs_kmeans_finalize(int32_t k, int32_t D, const float* sums, const float* counts,
-                        float eps_count, float* centers_out, void* stream);
-
 /* out[i, :] = feat[i, :] - feat[i, :] + centers[ids[i], :Dout]  evaluated as the reference does
  * (x - x + c in fp32), i.e. the forward value of the straight-through quantised feature. */
 int ogs_kmeans_gather_st(int64_t N, const float* feat, int32_t Dout, const float* centers,
                          int32_t Dc, const int64_t* ids, float* out, void* stream);
-
-/* Per-cluster member counts: counts_out int64 [k] (zeroed by the call). */
-int ogs_kmeans_count(int64_t N, const int64_t* ids, int32_t k, int64_t* counts_out, void* stream);
 
 /* ---- fine level of the two-level codebook, ALL coarse clusters in one launch ----
  * Replaces k1 calls of the reference's leaf mode (scene/kmeans_quantize.py:196-206 assign + :82-87,:202-205

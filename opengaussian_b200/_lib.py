@@ -5,6 +5,8 @@ There is NO fallback: if the shared library is missing or a call fails this modu
 import ctypes as C
 import os
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("OGS_LIB_PATH") or os.path.join(_HERE, "csrc", "libogs_b200.so")   # env: developer A/B builds
 
@@ -81,9 +83,7 @@ EXPORTS = {
     "ogs_raster_export": (C.c_int, [C.POINTER(RasterInputs), C.POINTER(RasterState)] + [_fp] * 10 + [C.c_void_p]),
     "ogs_kmeans_assign": (C.c_int, [C.c_int64, _fp, C.c_int32, _fp, C.c_int32, C.c_float, _fp, C.c_int32, _fp,
                                     C.c_int64, C.c_int64, _fp, _fp, _fp, C.c_void_p]),
-    "ogs_kmeans_finalize": (C.c_int, [C.c_int32, C.c_int32, _fp, _fp, C.c_float, _fp, C.c_void_p]),
     "ogs_kmeans_gather_st": (C.c_int, [C.c_int64, _fp, C.c_int32, _fp, C.c_int32, _fp, _fp, C.c_void_p]),
-    "ogs_kmeans_count": (C.c_int, [C.c_int64, _fp, C.c_int32, _fp, C.c_void_p]),
     "ogs_kmeans_assign_segmented": (C.c_int, [C.c_int64, _fp, C.c_int32, _fp, _fp, _fp, C.c_int32, C.c_int32, _fp, _fp,
                                               C.c_int32, C.c_void_p]),
     "ogs_kmeans_finalize_fixed": (C.c_int, [C.c_int32, C.c_int32, _fp, C.c_int32, C.c_float, _fp, _fp, C.c_void_p]),
@@ -133,7 +133,7 @@ def lib() -> C.CDLL:
             fn = getattr(L, name)
             fn.restype = res
             fn.argtypes = args
-        if L.ogs_abi_version() != 6:
+        if L.ogs_abi_version() != 7:
             raise OgsError("libogs_b200.so ABI version mismatch")
         _LIB = L
     return _LIB
@@ -145,6 +145,15 @@ def check(rc: int, what: str):
         if rc == -2:
             raise Exception(msg)          # same exception type/message as the reference Python layer
         raise OgsError(f"{what} failed (rc={rc}): {msg}")
+
+
+def launch(name: str, device, *args) -> None:
+    """Calls the C-ABI entry point `name` with `args` followed by the current stream of `device`, with `device` the
+    current CUDA device for the duration of the call (the library keys its per-device state on cudaGetDevice, and CUDA
+    refuses a launch into another device's stream); raises as check() does on a non-zero return."""
+    with torch.cuda.device(device):
+        rc = getattr(lib(), name)(*args, C.c_void_p(torch.cuda.current_stream(device).cuda_stream))
+    check(rc, name)
 
 
 PROFILE_FAMILIES = ("preprocess_fwd", "depth_sort_scan", "emit", "tile_sort", "tile_ranges", "blend_fwd",

@@ -565,15 +565,6 @@ int ogs_kmeans_assign(int64_t N, const float* a, int32_t Da, const float* b, int
                                 counts, (cudaStream_t)stream_);
 }
 
-int ogs_kmeans_finalize(int32_t k, int32_t D, const float* sums, const float* counts, float eps_count,
-                        float* centers_out, void* stream_) {
-    if (k < 0 || D < 1 || !sums || !counts || !centers_out) { set_error("kmeans_finalize: bad arguments"); return -1; }
-    int rc = launch_kmeans_finalize(k, D, sums, counts, eps_count, centers_out, (cudaStream_t)stream_);
-    if (rc) return rc;
-    OGS_KERNEL_CHECK("kmeans_finalize", 0, (cudaStream_t)stream_);
-    return 0;
-}
-
 int ogs_kmeans_gather_st(int64_t N, const float* feat, int32_t Dout, const float* centers, int32_t Dc,
                          const int64_t* ids, float* out, void* stream_) {
     if (N < 0 || Dout < 1 || Dc < Dout || (N > 0 && (!feat || !centers || !ids || !out))) {
@@ -583,14 +574,6 @@ int ogs_kmeans_gather_st(int64_t N, const float* feat, int32_t Dout, const float
     int rc = launch_kmeans_gather_st(N, feat, Dout, centers, Dc, ids, out, (cudaStream_t)stream_);
     if (rc) return rc;
     OGS_KERNEL_CHECK("kmeans_gather_st", 0, (cudaStream_t)stream_);
-    return 0;
-}
-
-int ogs_kmeans_count(int64_t N, const int64_t* ids, int32_t k, int64_t* counts_out, void* stream_) {
-    if (N < 0 || k < 0 || !counts_out || (N > 0 && !ids)) { set_error("kmeans_count: bad arguments"); return -1; }
-    int rc = launch_kmeans_count(N, ids, k, counts_out, (cudaStream_t)stream_);
-    if (rc) return rc;
-    OGS_KERNEL_CHECK("kmeans_count", 0, (cudaStream_t)stream_);
     return 0;
 }
 

@@ -292,10 +292,8 @@ __device__ __forceinline__ bool ogs_rect_hit_s(const float4 sa, const float2 sb,
 int launch_kmeans_assign(int64_t N, const float* a, int Da, const float* b, int Db, float scale_b,
                          const float* centers, int k, const int64_t* select_ids, int64_t selected, int64_t id_offset,
                          int64_t* ids_out, float* sums, float* counts, cudaStream_t s);
-int launch_kmeans_finalize(int k, int D, const float* sums, const float* counts, float eps, float* out, cudaStream_t s);
 int launch_kmeans_gather_st(int64_t N, const float* feat, int Dout, const float* centers, int Dc, const int64_t* ids,
                             float* out, cudaStream_t s);
-int launch_kmeans_count(int64_t N, const int64_t* ids, int k, int64_t* counts, cudaStream_t s);
 size_t kmeans_lloyd_workspace_bytes(int k, int D);
 size_t kmeans_seg_lloyd_workspace_bytes(int k1, int k2, int D);
 int launch_kmeans_lloyd_pass(int64_t N, const float* a, int Da, const float* b, int Db, float scale_b, float* centers, int k,

@@ -460,20 +460,6 @@ int launch_kmeans_lloyd_pass(int64_t N, const float* a, int Da, const float* b, 
     return -5;
 }
 
-__global__ void kmeans_finalize_kernel(int k, int D, const float* __restrict__ sums, const float* __restrict__ counts,
-                                       float eps, float* __restrict__ out) {
-    const int e = blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= k * D) return;
-    const int j = e / D;
-    out[e] = __fdiv_rn(sums[e], __fadd_rn(counts[j], eps));
-}
-
-int launch_kmeans_finalize(int k, int D, const float* sums, const float* counts, float eps, float* out, cudaStream_t s) {
-    if (k * D <= 0) return 0;
-    kmeans_finalize_kernel<<<(k * D + 127) / 128, 128, 0, s>>>(k, D, sums, counts, eps, out);
-    return 0;
-}
-
 __global__ void kmeans_gather_st_kernel(int64_t N, const float* __restrict__ feat, int Dout,
                                         const float* __restrict__ centers, int Dc, const int64_t* __restrict__ ids,
                                         float* __restrict__ out) {
@@ -490,31 +476,6 @@ int launch_kmeans_gather_st(int64_t N, const float* feat, int Dout, const float*
     const int64_t tot = N * Dout;
     if (tot <= 0) return 0;
     kmeans_gather_st_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(N, feat, Dout, centers, Dc, ids, out);
-    return 0;
-}
-
-__global__ void kmeans_count_kernel(int64_t N, const int64_t* __restrict__ ids, int k, unsigned long long* __restrict__ counts) {
-    extern __shared__ unsigned int s_cnt[];
-    for (int e = threadIdx.x; e < k; e += blockDim.x) s_cnt[e] = 0;
-    __syncthreads();
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t id = ids[i];
-        if (id >= 0 && id < k) atomicAdd(&s_cnt[id], 1u);
-    }
-    __syncthreads();
-    for (int e = threadIdx.x; e < k; e += blockDim.x)
-        if (s_cnt[e]) atomicAdd(&counts[e], (unsigned long long)s_cnt[e]);
-}
-
-int launch_kmeans_count(int64_t N, const int64_t* ids, int k, int64_t* counts, cudaStream_t s) {
-    if (k <= 0) return 0;
-    cudaError_t e = cudaMemsetAsync(counts, 0, (size_t)k * 8, s);
-    if (e != cudaSuccess) return cuda_fail(e, "memset counts");
-    if (N <= 0) return 0;
-    if ((size_t)k * 4 > 48 * 1024) { set_error("kmeans_count: k=%d too large", k); return -5; }
-    int64_t want = (N + 255) / 256;
-    int grid = (int)(want < OGS_NUM_SMS * 8 ? want : OGS_NUM_SMS * 8);
-    kmeans_count_kernel<<<grid, 256, (size_t)k * 4, s>>>(N, ids, k, (unsigned long long*)counts);
     return 0;
 }
 

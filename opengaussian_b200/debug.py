@@ -11,7 +11,6 @@ from .rasterizer import GaussianRasterizationSettings, _Alloc, _f32c, _fill_inpu
 
 def forward_with_state(rs: GaussianRasterizationSettings, means3D, opacities, shs=None, colors_precomp=None,
                        scales=None, rotations=None, cov3D_precomp=None, extra=None, export=True):
-    L = _lib.lib()
     dev = means3D.device
     means3D, opacities, shs, colors_precomp = _f32c(means3D), _f32c(opacities), _f32c(shs), _f32c(colors_precomp)
     scales, rotations, cov3D_precomp, extra = _f32c(scales), _f32c(rotations), _f32c(cov3D_precomp), _f32c(extra)
@@ -30,9 +29,7 @@ def forward_with_state(rs: GaussianRasterizationSettings, means3D, opacities, sh
     ro = _lib.RasterOutputs(_lib.ptr(color), _lib.ptr(depth), _lib.ptr(alpha), _lib.ptr(radii))
     st = _lib.RasterState()
     alloc = _Alloc(dev)
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    _lib.check(L.ogs_raster_forward(C.byref(ri), C.byref(ro), alloc.fn, alloc.user, C.byref(st), C.c_void_p(stream)),
-               "ogs_raster_forward")
+    _lib.launch("ogs_raster_forward", dev, C.byref(ri), C.byref(ro), alloc.fn, alloc.user, C.byref(st))
     N = int(st.num_rendered)
     out = dict(color=color, depth=depth, alpha=alpha, radii=radii, N=N, _bufs=alloc.bufs, _state=st, _inputs=ri,
                _keep=(means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, bg_full, rs))
@@ -48,9 +45,8 @@ def forward_with_state(rs: GaussianRasterizationSettings, means3D, opacities, sh
         tt = torch.zeros(P, dtype=torch.int32, device=dev)
         fT = torch.zeros(H, W, device=dev)
         nc = torch.zeros(H, W, dtype=torch.int32, device=dev)
-        _lib.check(L.ogs_raster_export(C.byref(ri), C.byref(st), _lib.ptr(keys), _lib.ptr(plist), _lib.ptr(ranges),
-                                       _lib.ptr(xy), _lib.ptr(dep), _lib.ptr(co), _lib.ptr(rgb), _lib.ptr(tt),
-                                       _lib.ptr(fT), _lib.ptr(nc), C.c_void_p(stream)), "ogs_raster_export")
+        _lib.launch("ogs_raster_export", dev, C.byref(ri), C.byref(st), _lib.ptr(keys), _lib.ptr(plist), _lib.ptr(ranges),
+                    _lib.ptr(xy), _lib.ptr(dep), _lib.ptr(co), _lib.ptr(rgb), _lib.ptr(tt), _lib.ptr(fT), _lib.ptr(nc))
         out.update(keys=keys[:N], point_list=plist[:N], ranges=ranges, xy=xy, geom_depth=dep, conic_opacity=co,
                    rgb=rgb, tiles_touched=tt, final_T=fT, n_contrib=nc)
     return out

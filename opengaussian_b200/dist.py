@@ -177,19 +177,12 @@ class GradArena:
     def all_reduce(self, n_floats: int, barriers: bool = True):
         """In-place sum over the ranks of the first n_floats of the arena, enqueued on the current stream.
         (barriers=False is a timing aid only: the result is then unordered against the other ranks' writes.)"""
-        import ctypes as C
         n = (int(n_floats) + 3) // 4 * 4
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        if not barriers:
-            with torch.cuda.device(self.device):
-                rc = self._lib.lib().ogs_multimem_allreduce_f32(C.c_void_p(self.mc), n, self.rank, self.world, stream)
-            self._lib.check(rc, "ogs_multimem_allreduce_f32")
-            return
-        self.hdl.barrier(channel=0)                 # every rank's gradients are written
-        with torch.cuda.device(self.device):
-            rc = self._lib.lib().ogs_multimem_allreduce_f32(C.c_void_p(self.mc), n, self.rank, self.world, stream)
-        self._lib.check(rc, "ogs_multimem_allreduce_f32")
-        self.hdl.barrier(channel=1)                 # every slice has been stored everywhere
+        if barriers:
+            self.hdl.barrier(channel=0)             # every rank's gradients are written
+        self._lib.launch("ogs_multimem_allreduce_f32", self.device, self.mc, n, self.rank, self.world)
+        if barriers:
+            self.hdl.barrier(channel=1)             # every slice has been stored everywhere
 
     def close(self):
         from .rasterizer import set_grad_arena
@@ -267,11 +260,8 @@ class PeerReducer:
             return t
         if not t.is_contiguous() or t.dtype not in (torch.float32, torch.int64):
             raise self._lib.OgsError("PeerReducer.all_reduce needs a contiguous float32 or int64 tensor")
-        L = self._lib.lib()
-        stream = self._C.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
-        with torch.cuda.device(t.device):
-            rc = L.ogs_peer_allreduce(self.comm, t.data_ptr(), t.numel(), 0 if t.dtype == torch.float32 else 1, stream)
-        self._lib.check(rc, "ogs_peer_allreduce")
+        self._lib.launch("ogs_peer_allreduce", t.device, self.comm, t.data_ptr(), t.numel(),
+                         0 if t.dtype == torch.float32 else 1)
         return t
 
     def check(self):

@@ -17,8 +17,6 @@ The padded index lists built by ``equalize_cluster_size`` (:89-144: ``cluster_id
 max_cnt, excl_clusters, excl_cluster_ids``) only feed that discarded computation; they are
 materialised lazily on first access.
 """
-import ctypes as C
-
 import torch
 
 from . import _lib
@@ -26,15 +24,10 @@ from . import _lib
 CHUNK = 10000  # reference chunk size (:178); only its count matters (the eps added to counts)
 
 
-def _stream(dev):
-    return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-
-
 def kmeans_assign(a, b, scale_b, centers, select_ids=None, selected=-1, id_offset=0, ids_out=None,
                   sums=None, counts=None):
     """One fused assign (+ optional centroid sums/counts accumulation) pass through the C ABI.
     a [N,Da] (+ b [N,Db] * scale_b) vs centers [k, Da+Db]; returns ids (int64 [N])."""
-    L = _lib.lib()
     a = a.detach()
     if a.dtype != torch.float32 or not a.is_contiguous():
         a = a.float().contiguous()
@@ -50,11 +43,8 @@ def kmeans_assign(a, b, scale_b, centers, select_ids=None, selected=-1, id_offse
         raise _lib.OgsError("k-means kernels need CUDA tensors (there is no CPU fallback)")
     if ids_out is None:
         ids_out = torch.empty(N, dtype=torch.int64, device=a.device)
-    with torch.cuda.device(a.device):
-        rc = L.ogs_kmeans_assign(N, _lib.ptr(a), Da, _lib.ptr(b), Db, float(scale_b), _lib.ptr(centers), k,
-                                 _lib.ptr(select_ids), int(selected), int(id_offset), _lib.ptr(ids_out),
-                                 _lib.ptr(sums), _lib.ptr(counts), _stream(a.device))
-    _lib.check(rc, "ogs_kmeans_assign")
+    _lib.launch("ogs_kmeans_assign", a.device, N, _lib.ptr(a), Da, _lib.ptr(b), Db, float(scale_b), _lib.ptr(centers), k,
+                _lib.ptr(select_ids), int(selected), int(id_offset), _lib.ptr(ids_out), _lib.ptr(sums), _lib.ptr(counts))
     return ids_out
 
 
@@ -71,7 +61,6 @@ def kmeans_assign_segmented(a, coarse_ids, seg_centers, seg_k, k2, ids_out=None,
     """Fine level for ALL coarse clusters in one launch (C ABI ogs_kmeans_assign_segmented): point i competes among
     rows [c*k2, c*k2 + seg_k[c]) of seg_centers, c = coarse_ids[i]; ids_out[i] = c*k2 + argmin.  acc (int64
     [k1*k2*(D+1)], added to) receives the exact fixed-point centroid sums and counts."""
-    L = _lib.lib()
     a = a.detach()
     if a.dtype != torch.float32 or not a.is_contiguous():
         a = a.float().contiguous()
@@ -88,10 +77,8 @@ def kmeans_assign_segmented(a, coarse_ids, seg_centers, seg_k, k2, ids_out=None,
         ids_out = torch.full((N,), k1 * k2, dtype=torch.int64, device=a.device)
     if acc is not None and (acc.dtype != torch.int64 or acc.numel() < k1 * k2 * (D + 1) or not acc.is_contiguous()):
         raise _lib.OgsError("acc must be a contiguous int64 tensor of k1*k2*(D+1) elements")
-    with torch.cuda.device(a.device):
-        rc = L.ogs_kmeans_assign_segmented(N, _lib.ptr(a), D, _lib.ptr(coarse_ids), _lib.ptr(seg_centers), _lib.ptr(seg_k),
-                                           k1, int(k2), _lib.ptr(ids_out), _lib.ptr(acc), int(fix_bits), _stream(a.device))
-    _lib.check(rc, "ogs_kmeans_assign_segmented")
+    _lib.launch("ogs_kmeans_assign_segmented", a.device, N, _lib.ptr(a), D, _lib.ptr(coarse_ids), _lib.ptr(seg_centers),
+                _lib.ptr(seg_k), k1, int(k2), _lib.ptr(ids_out), _lib.ptr(acc), int(fix_bits))
     return ids_out
 
 
@@ -109,26 +96,20 @@ def lloyd_pass(a, b, scale_b, centers, counts_state, eps_add, ids_out, ws: Lloyd
     """One Lloyd iteration in one launch (C ABI ogs_kmeans_lloyd_pass): `centers` [k_out, D] is updated in place from
     its first k rows; counts_state [k_out] carries the reference's count bookkeeping; comm = PeerReducer.comm when the
     points are sharded over GPUs."""
-    L = _lib.lib()
     k_out = centers.shape[0]
     k = k_out if k is None else k
-    with torch.cuda.device(a.device):
-        rc = L.ogs_kmeans_lloyd_pass(a.shape[0], _lib.ptr(a), a.shape[1], _lib.ptr(b), 0 if b is None else b.shape[1],
-                                     float(scale_b), _lib.ptr(centers), k, k_out, _lib.ptr(select_ids), int(selected),
-                                     int(id_offset), _lib.ptr(ids_out), _lib.ptr(counts_state), float(eps_add), comm,
-                                     _lib.ptr(ws.buf), _stream(a.device))
-    _lib.check(rc, "ogs_kmeans_lloyd_pass")
+    _lib.launch("ogs_kmeans_lloyd_pass", a.device, a.shape[0], _lib.ptr(a), a.shape[1], _lib.ptr(b),
+                0 if b is None else b.shape[1], float(scale_b), _lib.ptr(centers), k, k_out, _lib.ptr(select_ids),
+                int(selected), int(id_offset), _lib.ptr(ids_out), _lib.ptr(counts_state), float(eps_add), comm,
+                _lib.ptr(ws.buf))
 
 
 def lloyd_pass_segmented(a, coarse_ids, seg_centers, seg_k, k2, counts_state, ids_out, fix_bits, ws: LloydWorkspace,
                          comm=None, eps_add=1e-6):
     """One Lloyd pass of every coarse cluster's fine level in one launch (C ABI ogs_kmeans_lloyd_pass_segmented)."""
-    L = _lib.lib()
-    with torch.cuda.device(a.device):
-        rc = L.ogs_kmeans_lloyd_pass_segmented(a.shape[0], _lib.ptr(a), a.shape[1], _lib.ptr(coarse_ids), _lib.ptr(seg_centers),
-                                               _lib.ptr(seg_k), seg_k.numel(), int(k2), _lib.ptr(ids_out), int(fix_bits),
-                                               _lib.ptr(counts_state), float(eps_add), comm, _lib.ptr(ws.buf), _stream(a.device))
-    _lib.check(rc, "ogs_kmeans_lloyd_pass_segmented")
+    _lib.launch("ogs_kmeans_lloyd_pass_segmented", a.device, a.shape[0], _lib.ptr(a), a.shape[1], _lib.ptr(coarse_ids),
+                _lib.ptr(seg_centers), _lib.ptr(seg_k), seg_k.numel(), int(k2), _lib.ptr(ids_out), int(fix_bits),
+                _lib.ptr(counts_state), float(eps_add), comm, _lib.ptr(ws.buf))
 
 
 class _GatherStraightThrough(torch.autograd.Function):
@@ -136,14 +117,11 @@ class _GatherStraightThrough(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, feat, centers, ids):
-        L = _lib.lib()
         f = feat.detach().float().contiguous()
         c = centers.detach().float().contiguous()
         out = torch.empty_like(f)
-        with torch.cuda.device(f.device):
-            rc = L.ogs_kmeans_gather_st(f.shape[0], _lib.ptr(f), f.shape[1], _lib.ptr(c), c.shape[1],
-                                        _lib.ptr(ids), _lib.ptr(out), _stream(f.device))
-        _lib.check(rc, "ogs_kmeans_gather_st")
+        _lib.launch("ogs_kmeans_gather_st", f.device, f.shape[0], _lib.ptr(f), f.shape[1], _lib.ptr(c), c.shape[1],
+                    _lib.ptr(ids), _lib.ptr(out))
         return out
 
     @staticmethod
@@ -301,22 +279,16 @@ class Quantize_kMeans():
         if not dist_on or comm is not None:
             # ONE launch per Lloyd iteration (C ABI ogs_kmeans_lloyd_pass): assign + centroid sums + [all-reduce over
             # NVLink peer memory by the kernel's last CTA] + the reference's centre update, in place on `cur`
-            L = _lib.lib()
             if mode == "root":
-                cur, k_in, k_out, eps_add = centers.clone(), k, k, n_eps * 1e-6
+                cur, k_in, eps_add = centers.clone(), k, n_eps * 1e-6
             else:
-                cur, k_in, k_out, eps_add = self.leaf_centers[start_id:start_id + k2], n_sub, k2, 1e-6
-            ws = torch.zeros((L.ogs_kmeans_lloyd_workspace_bytes(k_in, D) + 3) // 4, dtype=torch.int32, device=dev)
-            counts_state = torch.full((k_out,), 1e-6, dtype=torch.float32, device=dev)
+                cur, k_in, eps_add = self.leaf_centers[start_id:start_id + k2], n_sub, 1e-6
+            ws = LloydWorkspace(dev, k=k_in, D=D)
+            counts_state = torch.full((cur.shape[0],), 1e-6, dtype=torch.float32, device=dev)
             a_c = a if (a.dtype == torch.float32 and a.is_contiguous()) else a.float().contiguous()
             b_c = None if b is None else (b if (b.dtype == torch.float32 and b.is_contiguous()) else b.float().contiguous())
             for _ in range(self.num_kmeans_iters):
-                with torch.cuda.device(dev):
-                    rc = L.ogs_kmeans_lloyd_pass(N, _lib.ptr(a_c), a_c.shape[1], _lib.ptr(b_c), 0 if b_c is None else b_c.shape[1],
-                                                 float(scale_b), _lib.ptr(cur), k_in, k_out, _lib.ptr(select), int(selected),
-                                                 int(id_offset), _lib.ptr(ids), _lib.ptr(counts_state), float(eps_add), comm,
-                                                 _lib.ptr(ws), _stream(dev))
-                _lib.check(rc, "ogs_kmeans_lloyd_pass")
+                lloyd_pass(a_c, b_c, scale_b, cur, counts_state, eps_add, ids, ws, comm, k_in, select, selected, id_offset)
             if mode == "root":
                 centers = cur
         else:
@@ -396,7 +368,6 @@ class Quantize_kMeans():
             stats = torch.cat([mx, nn])
         max_abs, n_glob = (float(v) for v in stats.tolist())
         fix = fixed_point_bits(int(n_glob), max_abs)
-        L = _lib.lib()
         counts_state = torch.full((rows,), 1e-6, dtype=torch.float32, device=dev)
         ids = self.leaf_cls_ids
         comm = self.reducer.comm if (self.distributed and self.reducer is not None) else None
@@ -404,23 +375,17 @@ class Quantize_kMeans():
         if not self.distributed or comm is not None:
             # ONE launch per Lloyd pass: segmented assign + exact sums + [integer all-reduce over NVLink peer memory by the
             # kernel's last CTA] + centre update of every block, in place on leaf_centers
-            ws = torch.zeros((L.ogs_kmeans_lloyd_segmented_workspace_bytes(k1, k2, D) + 3) // 4, dtype=torch.int32, device=dev)
+            ws = LloydWorkspace(dev, D=D, k1=k1, k2=k2)
             for _ in range(self.num_kmeans_iters):
-                with torch.cuda.device(dev):
-                    rc = L.ogs_kmeans_lloyd_pass_segmented(N, _lib.ptr(a), D, _lib.ptr(coarse), _lib.ptr(self.leaf_centers),
-                                                           _lib.ptr(seg_k), k1, k2, _lib.ptr(ids), fix, _lib.ptr(counts_state),
-                                                           1e-6, comm, _lib.ptr(ws), _stream(dev))
-                _lib.check(rc, "ogs_kmeans_lloyd_pass_segmented")
+                lloyd_pass_segmented(a, coarse, self.leaf_centers, seg_k, k2, counts_state, ids, fix, ws, comm)
         else:
             acc = torch.zeros(rows * (D + 1), dtype=torch.int64, device=dev)
             for _ in range(self.num_kmeans_iters):
                 acc.zero_()
                 kmeans_assign_segmented(a, coarse, self.leaf_centers, seg_k, k2, ids, acc, fix)
                 self._all_reduce(acc)
-                with torch.cuda.device(dev):
-                    rc = L.ogs_kmeans_finalize_fixed(rows, D, _lib.ptr(acc), fix, 1e-6, _lib.ptr(counts_state),
-                                                     _lib.ptr(self.leaf_centers), _stream(dev))
-                _lib.check(rc, "ogs_kmeans_finalize_fixed")
+                _lib.launch("ogs_kmeans_finalize_fixed", dev, rows, D, _lib.ptr(acc), fix, 1e-6, _lib.ptr(counts_state),
+                            _lib.ptr(self.leaf_centers))
         kmeans_assign_segmented(a, self.cls_ids, self.leaf_centers, seg_k, k2, ids, None, fix)
         self.leaf_cls_ids = ids
         self.nn_index = ids

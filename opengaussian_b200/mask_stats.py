@@ -13,15 +13,9 @@ The reference expands ``feat_map [C,H,W]`` and ``gt_masks [M,H,W]`` to ``[M,C,H,
 Both functions are differentiable (custom autograd, gradients to ``feat_map``, ``image_mask`` and the
 mask means), because ``train.py:450-456`` back-propagates through them.
 """
-import ctypes as C
-
 import torch
 
 from . import _lib
-
-
-def _stream(dev):
-    return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
 
 ID_MAP_MIN_MASKS = 16     # below this the M mask bytes per pixel are as cheap as building the id map
@@ -49,10 +43,7 @@ class _MaskSet:
         elif ID_MAP_MIN_MASKS <= M <= 32767 and HW > 0:
             self.ids = torch.empty(HW, dtype=torch.int16, device=dev)
             self.overlap = torch.empty(1, dtype=torch.int32, device=dev)
-            with torch.cuda.device(dev):
-                rc = _lib.lib().ogs_mask_id_map(M, HW, _lib.ptr(self.bytes), _lib.ptr(self.ids), _lib.ptr(self.overlap),
-                                                _stream(dev))
-            _lib.check(rc, "ogs_mask_id_map")
+            _lib.launch("ogs_mask_id_map", dev, M, HW, _lib.ptr(self.bytes), _lib.ptr(self.ids), _lib.ptr(self.overlap))
 
 
 # The mask set of the LAST gt_masks tensor seen: mask_feature_mean and cohesion_loss of one training step receive the
@@ -101,8 +92,8 @@ class _MaskMean(torch.autograd.Function):
         dev = feat.device
         sums = torch.empty(M, Cn, device=dev)
         counts = torch.empty(M, device=dev)
-        _lib.check(_lib.lib().ogs_mask_mean_forward(M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ms), _lib.ptr(img),
-                                                   _lib.ptr(sums), _lib.ptr(counts), _stream(dev)), "ogs_mask_mean_forward")
+        _lib.launch("ogs_mask_mean_forward", dev, M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ms), _lib.ptr(img),
+                    _lib.ptr(sums), _lib.ptr(counts))
         cnt = counts.clamp(min=1)
         mean = sums / cnt[:, None]
         ctx.save_for_backward(feat, img if img is not None else torch.empty(0, device=dev), counts, mean)
@@ -124,9 +115,8 @@ class _MaskMean(torch.autograd.Function):
         K = torch.where(counts > 1, (G * mean).sum(1), torch.zeros_like(counts)).contiguous()
         dfeat = torch.empty_like(feat)
         dimg = torch.empty(HW, device=dev) if img is not None else None
-        _lib.check(_lib.lib().ogs_mask_mean_backward(M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ctx.ms), _lib.ptr(img), _lib.ptr(G),
-                                                    _lib.ptr(K), _lib.ptr(dfeat), _lib.ptr(dimg), _stream(dev)),
-                   "ogs_mask_mean_backward")
+        _lib.launch("ogs_mask_mean_backward", dev, M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ctx.ms), _lib.ptr(img), _lib.ptr(G),
+                    _lib.ptr(K), _lib.ptr(dfeat), _lib.ptr(dimg))
         g_img = None
         if dimg is not None and ctx.needs_input_grad[2]:
             g_img = dimg.view(1, feat.shape[1], feat.shape[2]).sum_to_size(ctx.img_shape)
@@ -144,8 +134,8 @@ def mask_feature_mean(feat_map, gt_masks, image_mask=None, return_var=False):
     feat, ms, img, M, Cn, HW = _prep(feat_map, gt_masks, image_mask)
     sq = torch.empty(M, Cn, device=feat.device)
     mean_d = mean.detach().contiguous()
-    _lib.check(_lib.lib().ogs_mask_var_forward(M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ms), _lib.ptr(img), _lib.ptr(mean_d),
-                                              _lib.ptr(sq), _stream(feat.device)), "ogs_mask_var_forward")
+    _lib.launch("ogs_mask_var_forward", feat.device, M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ms), _lib.ptr(img),
+                _lib.ptr(mean_d), _lib.ptr(sq))
     cnt = counts.clamp(min=1)
     variance = (sq / cnt[:, None]).mean(dim=1)
     return mean, variance, cnt
@@ -159,8 +149,8 @@ class _Cohesion(torch.autograd.Function):
         mean = feat_mean_stack.detach().float().contiguous()
         dsum = torch.empty(M, device=dev)
         npix = torch.empty(M, device=dev)
-        _lib.check(_lib.lib().ogs_cohesion_forward(M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ms), _lib.ptr(mean), _lib.ptr(dsum),
-                                                  _lib.ptr(npix), _stream(dev)), "ogs_cohesion_forward")
+        _lib.launch("ogs_cohesion_forward", dev, M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ms), _lib.ptr(mean), _lib.ptr(dsum),
+                    _lib.ptr(npix))
         ctx.save_for_backward(feat, mean, npix)
         ctx.ms = ms
         ctx.shape = feat_map.shape
@@ -175,8 +165,8 @@ class _Cohesion(torch.autograd.Function):
         coef = (g.float() / (max(M, 1) * npix.clamp(min=1))).contiguous()
         dfeat = torch.empty_like(feat)
         dmean = torch.empty(M, Cn, device=dev)
-        _lib.check(_lib.lib().ogs_cohesion_backward(M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ctx.ms), _lib.ptr(mean), _lib.ptr(coef),
-                                                   _lib.ptr(dfeat), _lib.ptr(dmean), _stream(dev)), "ogs_cohesion_backward")
+        _lib.launch("ogs_cohesion_backward", dev, M, Cn, HW, _lib.ptr(feat), *_mask_ptrs(ctx.ms), _lib.ptr(mean),
+                    _lib.ptr(coef), _lib.ptr(dfeat), _lib.ptr(dmean))
         return dfeat.view(ctx.shape), None, dmean
 
 
@@ -197,10 +187,8 @@ class _Separation(torch.autograd.Function):
         buf = torch.empty(N * N + N + 1 + N * Cn, dtype=torch.float32, device=dev)
         loss = buf[N * N + N:N * N + N + 1]
         dmean = buf[N * N + N + 1:].view(N, Cn)
-        with torch.cuda.device(dev):
-            rc = _lib.lib().ogs_separation_loss(N, Cn, _lib.ptr(m), int(bool(small_weights)), _lib.ptr(buf), _lib.ptr(loss),
-                                                _lib.ptr(dmean), _stream(dev))
-        _lib.check(rc, "ogs_separation_loss")
+        _lib.launch("ogs_separation_loss", dev, N, Cn, _lib.ptr(m), int(bool(small_weights)), _lib.ptr(buf), _lib.ptr(loss),
+                    _lib.ptr(dmean))
         ctx.save_for_backward(dmean)
         return loss.reshape(())
 
@@ -241,8 +229,8 @@ def pair_mask_feature_mean(feat_map, masks):
         sums = torch.empty(1, Cn, device=feat.device)
         counts = torch.empty(1, device=feat.device)
         w = masks[i].detach().float().contiguous().view(HW)     # the reference multiplies by masks.float()
-        _lib.check(_lib.lib().ogs_mask_mean_forward(1, Cn, HW, _lib.ptr(feat), *_mask_ptrs(mk), _lib.ptr(w), _lib.ptr(sums),
-                                                   _lib.ptr(counts), _stream(feat.device)), "ogs_mask_mean_forward")
+        _lib.launch("ogs_mask_mean_forward", feat.device, 1, Cn, HW, _lib.ptr(feat), *_mask_ptrs(mk), _lib.ptr(w),
+                    _lib.ptr(sums), _lib.ptr(counts))
         outs.append(sums[0] / (counts[0] + 1e-6))
     return torch.stack(outs) if outs else feat_map.new_zeros(0, feat_map.shape[1])
 
@@ -273,10 +261,8 @@ def get_SAM_mask_and_feat(gt_sam_mask, level=3, filter_th=50, original_mask_feat
     invalid_pix = torch.empty(H, W, dtype=torch.bool, device=dev)
     ids = torch.empty(HW, dtype=torch.int16, device=dev)
     mask_bool = torch.empty(num, H, W, dtype=torch.bool, device=dev)
-    with torch.cuda.device(dev):
-        rc = _lib.lib().ogs_sam_masks(num, HW, _lib.ptr(level_ids), offset, _lib.ptr(mask_id), _lib.ptr(invalid_pix),
-                                      _lib.ptr(ids), _lib.ptr(mask_bool), _stream(dev))
-    _lib.check(rc, "ogs_sam_masks")
+    _lib.launch("ogs_sam_masks", dev, num, HW, _lib.ptr(level_ids), offset, _lib.ptr(mask_id), _lib.ptr(invalid_pix),
+                _lib.ptr(ids), _lib.ptr(mask_bool))
     register_mask_ids(mask_bool, ids)
     if original_mask_feat is not None:
         max_ind = int(gt_sam_mask[level].max()) + 1
@@ -307,8 +293,8 @@ def mask_pair_counts(masks1, masks2):
     if n + m > 0:
         nbytes = int(_lib.lib().ogs_mask_iou_scratch_bytes(n, m, HW))
         scratch = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
-        _lib.check(_lib.lib().ogs_mask_pair_counts(n, m, HW, _lib.ptr(a), _lib.ptr(b), _lib.ptr(scratch), _lib.ptr(inter),
-                                                  _lib.ptr(counts), _stream(dev)), "ogs_mask_pair_counts")
+        _lib.launch("ogs_mask_pair_counts", dev, n, m, HW, _lib.ptr(a), _lib.ptr(b), _lib.ptr(scratch), _lib.ptr(inter),
+                    _lib.ptr(counts))
     return inter, counts[:n], counts[n:]
 
 

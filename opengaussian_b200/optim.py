@@ -76,8 +76,5 @@ class FusedAdam(torch.optim.Adam):
                 a.n = p.numel()
                 a.step_size, a.bias_correction2_sqrt, a.beta1, a.beta2, a.eps = step_size, bc2s, beta1, beta2, eps
                 a.one_minus_beta1, a.one_minus_beta2 = 1 - beta1, 1 - beta2
-            with torch.cuda.device(dev):
-                stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-                _lib.check(_lib.lib().ogs_adam_step(len(items), C.cast(arr, C.c_void_p), float(grad_scale), stream),
-                           "ogs_adam_step")
+            _lib.launch("ogs_adam_step", dev, len(items), C.cast(arr, C.c_void_p), float(grad_scale))
         return loss

@@ -448,7 +448,6 @@ class _RasterizeGaussians(torch.autograd.Function):
                           extra, n_extra, sh_rest, act_flags)
         st = _lib.RasterState()
         alloc = _Alloc(dev)
-        stream = torch.cuda.current_stream(dev).cuda_stream
         # Frozen geometry (OpenGaussian stages 1-3, train.py:431-436): reuse the camera's records and tile lists
         frozen = view_cache.enabled and P > 0 and not rs.debug and not any(
             t is not None and t.requires_grad for t in (means3D, sh, opacities, scales, rotations, cov3Ds_precomp, sh_rest))
@@ -471,18 +470,14 @@ class _RasterizeGaussians(torch.autograd.Function):
             pin_for_capture(dev, entry.geom, entry.binning, entry.radii, *cam)   # an evicted entry must not free what a graph reads
             radii = entry.radii.detach()     # a fresh tensor object over the first call's radii (this Function's own output)
             ro = _lib.RasterOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha), None)
-            with torch.cuda.device(dev):
-                rc = L.ogs_raster_forward_cached(C.byref(ri), C.byref(ro), alloc.fn, alloc.user, C.byref(entry.state),
-                                                 C.byref(st), C.c_void_p(stream))
-            _lib.check(rc, "ogs_raster_forward_cached")
+            _lib.launch("ogs_raster_forward_cached", dev, C.byref(ri), C.byref(ro), alloc.fn, alloc.user,
+                        C.byref(entry.state), C.byref(st))
             alloc.bufs["geom"], alloc.bufs["binning"] = entry.geom, entry.binning
         else:
             if admit:
                 ri.defer_capacity_check = 0      # the entry needs this frame's duplicate count now
             ro = _lib.RasterOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha), _lib.ptr(radii))
-            with torch.cuda.device(dev):
-                rc = L.ogs_raster_forward(C.byref(ri), C.byref(ro), alloc.fn, alloc.user, C.byref(st), C.c_void_p(stream))
-            _lib.check(rc, "ogs_raster_forward")
+            _lib.launch("ogs_raster_forward", dev, C.byref(ri), C.byref(ro), alloc.fn, alloc.user, C.byref(st))
             if admit and int(st.num_rendered) >= 0:
                 gb, bb = C.c_int64(0), C.c_int64(0)
                 _lib.check(L.ogs_raster_cached_bytes(C.byref(ri), st.num_rendered, C.byref(gb), C.byref(bb)),
@@ -632,10 +627,7 @@ class _RasterizeGaussians(torch.autograd.Function):
         go = _lib.RasterGradsOut(_lib.ptr(g_means3D), _lib.ptr(g_means2D), _lib.ptr(g_opac), _lib.ptr(g_sh),
                                  _lib.ptr(g_colors), _lib.ptr(g_scales), _lib.ptr(g_rot), _lib.ptr(g_cov),
                                  _lib.ptr(g_extra), _lib.ptr(g_sh_rest), _lib.ptr(scratch), accumulate, 0)
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        with torch.cuda.device(dev):
-            rc = L.ogs_raster_backward(C.byref(ri), C.byref(ctx.state), C.byref(gi), C.byref(go), C.c_void_p(stream))
-        _lib.check(rc, "ogs_raster_backward")
+        _lib.launch("ogs_raster_backward", dev, C.byref(ri), C.byref(ctx.state), C.byref(gi), C.byref(go))
         if accumulate:       # already added into the leaves' .grad (means2D unless it was fused too)
             return (None, None if (accumulate & 2) else g_means2D) + (None,) * 11
         if g_extra is not None and n_extra != ctx.n_extra_user:
@@ -658,15 +650,11 @@ class GaussianRasterizer(nn.Module):
 
     def markVisible(self, positions: torch.Tensor) -> torch.Tensor:
         """Near-plane frustum test (upstream markVisible): bool [P]."""
-        L = _lib.lib()
         with torch.no_grad():
             pos = _f32c(positions)
             view = _f32c(self.raster_settings.viewmatrix)
             out = torch.empty(pos.shape[0], dtype=torch.uint8, device=pos.device)
-            stream = torch.cuda.current_stream(pos.device).cuda_stream
-            with torch.cuda.device(pos.device):
-                rc = L.ogs_mark_visible(pos.shape[0], _lib.ptr(pos), _lib.ptr(view), _lib.ptr(out), C.c_void_p(stream))
-            _lib.check(rc, "ogs_mark_visible")
+            _lib.launch("ogs_mark_visible", pos.device, pos.shape[0], _lib.ptr(pos), _lib.ptr(view), _lib.ptr(out))
         return out.bool()
 
     def forward_raw(self, means3D, means2D, opacity_logits, features_dc, features_rest, log_scales, raw_rotations,

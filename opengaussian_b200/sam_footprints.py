@@ -131,10 +131,9 @@ def batched_splat_ids(camera, gaussians, gaussian_ids, sam_mask, scaling_modifie
                                    color=WHITE_SH_COLOR, viewmatrix=view.data_ptr(), projmatrix=proj.data_ptr(),
                                    sam_ids=sam.data_ptr(), empty_id=empty_id, reserved_=0)
         overflow = C.c_int32(0)
-        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _lib.check(_lib.lib().ogs_splat_footprint_votes(C.byref(inp), *(_lib.ptr(out[k]) for k in
-                                                       ("dominant_id", "dominant_weight", "footprint_pixels", "q_max", "radii")),
-                                                       C.byref(overflow), stream), "ogs_splat_footprint_votes")
+        _lib.launch("ogs_splat_footprint_votes", dev, C.byref(inp),
+                    *(_lib.ptr(out[k]) for k in ("dominant_id", "dominant_weight", "footprint_pixels", "q_max", "radii")),
+                    C.byref(overflow))
         if overflow.value:
             for j in torch.nonzero(out["dominant_weight"] < 0).flatten().tolist():
                 did, wm, _ = get_splat_id_and_weights(camera, gaussians, int(ids[j]), sam_mask)

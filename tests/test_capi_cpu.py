@@ -28,8 +28,8 @@ def test_header_symbols_exported(lib):
         assert hasattr(lib, n), n
 
 
-def test_abi_version_and_sass_target(lib):
-    assert lib.ogs_abi_version() == 6
+def test_abi_version_7_and_sass_target(lib):
+    assert lib.ogs_abi_version() == 7
     import subprocess
     from opengaussian_b200 import _lib
     out = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
