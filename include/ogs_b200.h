@@ -20,6 +20,11 @@
  *       Raw-parameter mode (act_flags / shs_rest) additionally folds the GaussianModel getters of
  *       scene/gaussian_model.py:122-169 and the (normalize(ins_feat)+1)/2 of
  *       gaussian_renderer/__init__.py:127 into the same kernels (SURVEY.md 8a9).
+ *   ogs_raster_forward_subsets   the per-subset rasterizer forwards of the coarse-cluster and leaf loops of
+ *                                gaussian_renderer/__init__.py:174-236,245-356 (one per cluster or leaf, each
+ *                                with its own gather, preprocess, sorts and blend), for all subsets of a view
+ *                                in one call: one preprocess and binning, then a stable per-tile partition by
+ *                                subset and one blend over (tiles x subsets).  Forward only.
  *   ogs_mark_visible             upstream GaussianRasterizer.markVisible (mark_visible symbol)
  *   ogs_raster_export            debug view of the geometry records and the sorted (tile|depth) keys
  *                                (upstream geomState / binningState)
@@ -203,6 +208,25 @@ int ogs_raster_capacity_check(void);
 int64_t ogs_raster_capacity_hint(int64_t new_hint);
 
 size_t ogs_raster_backward_scratch_floats(int32_t P, int32_t n_extra);
+
+/* ---- all subsets of a view in one call (render()'s no-grad cluster / leaf passes) ----
+ * subset int32 [P]: slot in [0, S) or -1 (not rendered; any value outside [0, S) is treated as -1).  Every slot's
+ * images equal, bit for bit, an ogs_raster_forward of the rows with subset == slot (in increasing index order):
+ * a pass over a subset sorts its rows stably by depth, then stably by tile, so its tile lists are the frame's lists
+ * restricted to the subset, in the same order.  The call runs one preprocess and one binning over the Gaussians
+ * that belong to a slot, partitions each tile's list stably by slot and blends all (tile, slot) pairs in one launch.
+ * Inputs as for ogs_raster_forward, activated (act_flags == 0).  Forward only: no state, no radii.
+ * Reads the frame's duplicate count synchronously (one host wait per call) and leaves the running capacity
+ * estimate of ogs_raster_capacity_hint untouched.  Temporaries come from `alloc` (tags "geom", "binning") and the
+ * stream-ordered pool.  1 <= S <= OGS_MAX_SUBSETS (the partition kernel keeps S counters in shared memory). */
+#define OGS_MAX_SUBSETS 4096
+typedef struct ogs_subset_outputs {
+    float* color;   /* [S, 3 + n_extra, H, W] planar, background composited as in ogs_raster_forward */
+    float* depth;   /* [S, H, W] or NULL */
+    float* alpha;   /* [S, H, W] 1 - T_final */
+} ogs_subset_outputs;
+int ogs_raster_forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, int32_t S,
+                               const ogs_subset_outputs* out, ogs_alloc_fn alloc, void* alloc_user, void* stream);
 
 int ogs_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, uint8_t* present,
                      void* stream);

@@ -34,6 +34,13 @@ class RasterOutputs(C.Structure):
     _fields_ = [("color", _fp), ("depth", _fp), ("alpha", _fp), ("radii", _fp)]
 
 
+class SubsetOutputs(C.Structure):
+    _fields_ = [("color", _fp), ("depth", _fp), ("alpha", _fp)]
+
+
+MAX_SUBSETS = 4096     # OGS_MAX_SUBSETS
+
+
 class RasterState(C.Structure):
     _fields_ = [("geom", _fp), ("binning", _fp), ("image", _fp), ("num_rendered", C.c_int64),
                 ("geom_bytes", C.c_int64), ("binning_bytes", C.c_int64), ("image_bytes", C.c_int64), ("feat", _fp)]
@@ -75,6 +82,8 @@ EXPORTS = {
                                       C.POINTER(RasterGradsOut), C.c_void_p]),
     "ogs_raster_forward_cached": (C.c_int, [C.POINTER(RasterInputs), C.POINTER(RasterOutputs), ALLOC_FN, C.c_void_p,
                                             C.POINTER(RasterState), C.POINTER(RasterState), C.c_void_p]),
+    "ogs_raster_forward_subsets": (C.c_int, [C.POINTER(RasterInputs), _fp, C.c_int32, C.POINTER(SubsetOutputs), ALLOC_FN,
+                                             C.c_void_p, C.c_void_p]),
     "ogs_raster_cached_bytes": (C.c_int, [C.POINTER(RasterInputs), C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "ogs_raster_capacity_check": (C.c_int, []),
     "ogs_raster_capacity_hint": (C.c_int64, [C.c_int64]),

@@ -33,6 +33,7 @@ UNITS = {
     "mask_iou.cu": [],
     "adam.cu": [],
     "footprint.cu": [],
+    "subsets.cu": [],
     "capi.cu": [],
 }
 

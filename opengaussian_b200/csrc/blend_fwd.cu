@@ -21,6 +21,9 @@
 // ogs_stage -- the exponent comes out in the log2 domain, one MUFU.EX2 per pixel) followed by
 // their C colours + depth; per group of 32 staged Gaussians lane l tests Gaussian l against the
 // warp's block (ogs_rect_hit_s) and only the ballot survivors are blended.
+// SUBSETS = true (ogs_raster_forward_subsets): blockIdx.z is a subset; its tile lists start at
+// ranges + z * tiles and its images at z * C * H * W (colour) and z * H * W (depth, alpha; depth may be
+// NULL).  No final_T / n_contrib: that path has no backward.
 #include "common.cuh"
 #include <stdlib.h>
 
@@ -28,7 +31,7 @@ namespace ogs {
 
 #define BATCH 256
 
-template <int C, int PAIRS>
+template <int C, int PAIRS, bool SUBSETS>
 __global__ void __launch_bounds__(128 / PAIRS) blend_fwd_kernel(BlendFwdArgs a) {
     constexpr int THREADS = 128 / PAIRS;      // 4 / PAIRS warps
     constexpr int NPX = 2 * PAIRS;            // pixels per lane
@@ -45,7 +48,9 @@ __global__ void __launch_bounds__(128 / PAIRS) blend_fwd_kernel(BlendFwdArgs a) 
     const float pxf = (float)px;
     const float bx0 = (float)bxi, by0 = (float)byi;
 
-    const uint2 range = a.ranges[tile];
+    const uint2* ranges = a.ranges;
+    if constexpr (SUBSETS) ranges += (size_t)blockIdx.z * gx * gridDim.y;
+    const uint2 range = ranges[tile];
     int todo = (int)(range.y - range.x);
     const int rounds = (todo + BATCH - 1) / BATCH;
 
@@ -143,13 +148,22 @@ __global__ void __launch_bounds__(128 / PAIRS) blend_fwd_kernel(BlendFwdArgs a) 
         if (px < a.W && py < a.H) {
             const size_t pix = (size_t)py * a.W + px;
             const float T = fabsf((k & 1) ? T2[p].y : T2[p].x);
-            a.final_T[pix] = T;
-            a.n_contrib[pix] = last[k];
+            if constexpr (SUBSETS) {
+                const size_t z = blockIdx.z;
 #pragma unroll
-            for (int c = 0; c < C; c++)
-                a.out_color[c * HW + pix] = ((k & 1) ? acc[p][c].y : acc[p][c].x) + T * __ldg(a.bg + c);
-            a.out_depth[pix] = (k & 1) ? acc[p][C].y : acc[p][C].x;
-            a.out_alpha[pix] = 1.0f - T;
+                for (int c = 0; c < C; c++)
+                    a.out_color[(z * C + c) * HW + pix] = ((k & 1) ? acc[p][c].y : acc[p][c].x) + T * __ldg(a.bg + c);
+                if (a.out_depth) a.out_depth[z * HW + pix] = (k & 1) ? acc[p][C].y : acc[p][C].x;
+                a.out_alpha[z * HW + pix] = 1.0f - T;
+            } else {
+                a.final_T[pix] = T;
+                a.n_contrib[pix] = last[k];
+#pragma unroll
+                for (int c = 0; c < C; c++)
+                    a.out_color[c * HW + pix] = ((k & 1) ? acc[p][c].y : acc[p][c].x) + T * __ldg(a.bg + c);
+                a.out_depth[pix] = (k & 1) ? acc[p][C].y : acc[p][C].x;
+                a.out_alpha[pix] = 1.0f - T;
+            }
         }
     }
 }
@@ -158,8 +172,14 @@ template <int C>
 static int launch_c(const BlendFwdArgs& a, cudaStream_t s) {
     dim3 grid((a.W + 15) / 16, (a.H + 15) / 16);
     static const int pairs = getenv("OGS_FWD_PAIRS") ? atoi(getenv("OGS_FWD_PAIRS")) : OGS_FWD_PAIRS;  // tuning knob
-    if (pairs == 2) blend_fwd_kernel<C, 2><<<grid, 64, 0, s>>>(a);
-    else blend_fwd_kernel<C, 1><<<grid, 128, 0, s>>>(a);
+    if (pairs == 2) blend_fwd_kernel<C, 2, false><<<grid, 64, 0, s>>>(a);
+    else blend_fwd_kernel<C, 1, false><<<grid, 128, 0, s>>>(a);
+    return 0;
+}
+
+template <int C>
+static int launch_subsets_c(const BlendFwdArgs& a, int S, cudaStream_t s) {
+    blend_fwd_kernel<C, OGS_FWD_PAIRS, true><<<dim3((a.W + 15) / 16, (a.H + 15) / 16, S), 128 / OGS_FWD_PAIRS, 0, s>>>(a);
     return 0;
 }
 
@@ -171,6 +191,19 @@ int launch_blend_forward(const BlendFwdArgs& a, cudaStream_t s) {
         case 9: return launch_c<9>(a, s);
         case 12: return launch_c<12>(a, s);
         case 16: return launch_c<16>(a, s);
+    }
+    set_error("blend forward: unsupported channel count %d (supported: 3,4,6,9,12,16)", a.C);
+    return -4;
+}
+
+int launch_blend_forward_subsets(const BlendFwdArgs& a, int S, cudaStream_t s) {
+    switch (a.C) {
+        case 3: return launch_subsets_c<3>(a, S, s);
+        case 4: return launch_subsets_c<4>(a, S, s);
+        case 6: return launch_subsets_c<6>(a, S, s);
+        case 9: return launch_subsets_c<9>(a, S, s);
+        case 12: return launch_subsets_c<12>(a, S, s);
+        case 16: return launch_subsets_c<16>(a, S, s);
     }
     set_error("blend forward: unsupported channel count %d (supported: 3,4,6,9,12,16)", a.C);
     return -4;

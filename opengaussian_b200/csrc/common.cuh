@@ -185,6 +185,13 @@ struct BlendFwdArgs {
     float *out_color, *out_depth, *out_alpha, *final_T; uint32_t* n_contrib;
 };
 int launch_blend_forward(const BlendFwdArgs& a, cudaStream_t s);
+// S subsets: a.ranges = [S][tiles] segment bounds, outputs [S][C][H][W] / [S][H][W]; final_T, n_contrib unused
+int launch_blend_forward_subsets(const BlendFwdArgs& a, int S, cudaStream_t s);
+
+// subsets (subsets.cu): culled depth key for Gaussians outside [0, S); stable per-tile partition by subset
+int launch_subset_exclude(int P, int S, const int32_t* subset, uint32_t* depth_keys, cudaStream_t s);
+int launch_subset_partition(int tiles, int S, const uint2* ranges, const uint32_t* point_list, const int32_t* subset,
+                            uint32_t* out_list, uint2* sub_ranges, cudaStream_t s);
 
 struct BlendBwdArgs {
     int P, W, H, C;

@@ -694,3 +694,62 @@ class GaussianRasterizer(nn.Module):
         if extra_feats is None:
             return color, radii, depth, alpha
         return color, radii, depth, alpha, feat
+
+    def forward_subsets(self, means3D, opacities, subset, num_subsets, shs=None, colors_precomp=None, scales=None,
+                        rotations=None, cov3D_precomp=None, extra_feats=None, extra_bg=None):
+        """Renders ``num_subsets`` disjoint subsets of the Gaussians in one call (C ABI ogs_raster_forward_subsets):
+        ``subset [P]`` holds each Gaussian's slot in ``[0, num_subsets)`` or -1 (not rendered).  Slot k's images equal,
+        bit for bit, ``forward()`` on the rows with ``subset == k``.  Activated inputs as for ``forward()``; forward
+        only (no backward, no radii) and outside the view cache.  Returns ``(color [S,3,H,W], depth [S,1,H,W],
+        alpha [S,1,H,W], feats [S,F,H,W] or None)``."""
+        rs = self.raster_settings
+        if means3D.shape[0] > 0:
+            shs, colors_precomp = _none_if_empty(shs), _none_if_empty(colors_precomp)
+            scales, rotations, cov3D_precomp = _none_if_empty(scales), _none_if_empty(rotations), _none_if_empty(cov3D_precomp)
+        if (shs is None and colors_precomp is None) or (shs is not None and colors_precomp is not None):
+            raise Exception('Please provide excatly one of either SHs or precomputed colors!')
+        if ((scales is None or rotations is None) and cov3D_precomp is None) or \
+                ((scales is not None or rotations is not None) and cov3D_precomp is not None):
+            raise Exception('Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!')
+        inputs = (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra_feats)
+        if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs):
+            raise _lib.OgsError("forward_subsets has no backward: call it under torch.no_grad() or with inputs that "
+                                "do not require grad")
+        dev = means3D.device
+        if dev.type != "cuda":
+            raise _lib.OgsError("GaussianRasterizer needs CUDA tensors (there is no CPU fallback)")
+        means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra = (_f32c(t) for t in inputs)
+        P = means3D.shape[0]
+        S = int(num_subsets)
+        if tuple(subset.shape) != (P,):
+            raise _lib.OgsError(f"subset must have shape [{P}], got {tuple(subset.shape)}")
+        subset = subset.to(device=dev, dtype=torch.int32).contiguous()
+        H, W = int(rs.image_height), int(rs.image_width)
+        n_extra_user = 0 if extra is None else int(extra.shape[1])
+        n_extra = n_extra_user
+        if n_extra_user:
+            c_tot = next((c for c in _SUPPORTED_C if c >= 3 + n_extra_user), None)
+            if c_tot is None:
+                raise _lib.OgsError(f"extra_feats: at most {_SUPPORTED_C[-1] - 3} channels are supported")
+            if c_tot != 3 + n_extra_user:   # pad with zero channels up to a compiled width
+                extra = torch.cat([extra, extra.new_zeros(P, c_tot - 3 - n_extra_user)], 1).contiguous()
+                n_extra = c_tot - 3
+        bg = _f32c(rs.bg).reshape(-1)
+        if n_extra:
+            eb = bg.new_zeros(0) if extra_bg is None else _f32c(extra_bg).reshape(-1).to(dev)
+            bg = torch.cat([bg, eb, bg.new_zeros(n_extra - eb.numel())])
+        _, cam = camera_inputs(rs.viewmatrix, rs.projmatrix, rs.campos)
+        rs = rs._replace(viewmatrix=cam[0], projmatrix=cam[1], campos=cam[2])
+
+        color_all = torch.empty(max(S, 0), 3 + n_extra, H, W, dtype=torch.float32, device=dev)
+        depth = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
+        alpha = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
+        ri = _fill_inputs(rs, bg, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra,
+                          n_extra)
+        ri.defer_capacity_check = 0
+        alloc = _Alloc(dev)
+        so = _lib.SubsetOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha))
+        _lib.launch("ogs_raster_forward_subsets", dev, C.byref(ri), _lib.ptr(subset), S, C.byref(so), alloc.fn,
+                    alloc.user)
+        feats = color_all[:, 3:3 + n_extra_user] if n_extra_user else None
+        return color_all[:, :3], depth, alpha, feats

@@ -17,6 +17,7 @@ The feature channels get the same background as the reference gives them (bg_col
 each 3-channel group, because the reference reuses one rasterizer for all passes).  The CPU RNG
 draws (`torch.rand(1)` at :121,124) are reproduced so that training stays in lock-step.
 ``fused=False`` falls back to the reference's literal pass structure (used by the parity test).
+Cluster / leaf passes that need no gradient: all subsets of the call in ONE rasterizer call (_render_slots).
 """
 import math
 
@@ -95,6 +96,175 @@ def _feat_pass(rasterizer, bg3, means3D, means2D, opacity, scales, rotations, co
     img, _, _, alpha = rasterizer(means3D=means3D, means2D=means2D, shs=None, colors_precomp=feat,
                                   opacities=opacity, scales=scales, rotations=rotations, cov3D_precomp=cov3D_precomp)
     return img, alpha
+
+
+# ---- the coarse-cluster and leaf passes of render(): a planning step and a render step ----
+# The planners decide, in the reference's loop order, which clusters / leaves reach the rasterizer and with which rows;
+# their filters are disjoint, so they are handed on as ONE int32 slot map `subset` ([P]: slot k or -1, the filter of
+# slot k is subset == k).  The render step then runs either one rasterizer call for all slots
+# (GaussianRasterizer.forward_subsets: no-grad passes) or the reference's one pass per slot (passes whose outputs need
+# a gradient, and fused=False).
+
+SUBSET_BATCH_BYTES = 4 << 30    # output bytes of one forward_subsets call, S * (C + 2) * H * W * 4; more slots are split
+
+
+def _slot_map(ids, base, slots):
+    """int32 [P]: the position of ids[i] in `slots` where base[i] holds, else -1."""
+    subset = torch.full(ids.shape, -1, dtype=torch.int32, device=ids.device)
+    if slots:
+        n = max(slots) + 1
+        lut = torch.full((n,), -1, dtype=torch.int32, device=ids.device)
+        lut[torch.tensor(slots, dtype=torch.long, device=ids.device)] = torch.arange(
+            len(slots), dtype=torch.int32, device=ids.device)
+        ok = base & (ids >= 0) & (ids < n)
+        subset = torch.where(ok, lut[ids.clamp(0, n - 1).long()], subset)
+    return subset
+
+
+def _post_process(filter_idx, means3D):
+    """The reference's per-leaf outlier removal (:315-322): keeps the points whose mean distance to their sqrt(n) nearest
+    neighbours is below mean + std."""
+    filter_idx = filter_idx.clone()
+    nearest_k_distance = _knn_mean_dists(means3D[filter_idx].detach(), int(filter_idx.sum() ** 0.5))
+    mean_d, std_d = nearest_k_distance.mean(), nearest_k_distance.std()
+    mask = nearest_k_distance.mean(dim=-1) < mean_d + std_d
+    mask = mask.squeeze()
+    filter_idx[filter_idx != 0] = mask
+    return filter_idx
+
+
+def _plan_clusters(cluster_idx, num_cluster, viewed_pts, scale_filter, better_vis, selected_root_id, cluster_occur_cam):
+    """Coarse clusters of the loop :173-236 that reach the rasterizer, in loop order -> (cluster ids, slot map).  Filter of
+    cluster idx: cluster_idx == idx, visible, and with better_vis all scales < 0.5 and at least 100 such points (the
+    counts of all clusters come from one bincount).  The silhouette test (:222) is the render step's."""
+    cand = []
+    for idx in range(num_cluster):
+        if not better_vis and idx != selected_root_id:
+            continue
+        if cluster_occur_cam is not None and cluster_occur_cam[idx] == False:  # noqa: E712
+            continue
+        cand.append(idx)
+    base = viewed_pts & scale_filter if better_vis else viewed_pts
+    if better_vis and cand:
+        counts = torch.bincount(cluster_idx[base & (cluster_idx >= 0)], minlength=num_cluster).tolist()
+        cand = [idx for idx in cand if counts[idx] >= 100]
+    return cand, _slot_map(cluster_idx, base, cand)
+
+
+def _plan_leaves(leaf_cluster_idx, lerf_range, selected_leaf_id, pre_mask, viewed_pts, scale_filter, better_vis,
+                 post_process, means3D):
+    """Leaves of the loop :245-356 that reach the rasterizer, in loop order -> (leaf ids = occured_leaf_id, slot map).
+    Filter of leaf idx: leaf_cluster_idx == idx (with selected_leaf_id: any of those leaves), & pre_mask, visible; with
+    better_vis all scales < 0.1 and at least 100 points; then post_process's outlier removal; then at least 10 points.
+    With selected_leaf_id every iteration has the same filter and the loop stops after the first pass: at most one
+    slot.  Without post_process the counts of all leaves come from one bincount."""
+    base = viewed_pts if pre_mask is None else pre_mask & viewed_pts
+    if better_vis:
+        base = base & scale_filter
+    if selected_leaf_id is not None:
+        filt = (leaf_cluster_idx.unsqueeze(1) == selected_leaf_id).any(dim=1) & base
+        if not lerf_range or (better_vis and filt.sum() < 100):
+            return [], _slot_map(leaf_cluster_idx, filt, [])
+        if post_process:
+            filt = _post_process(filt, means3D)
+        if filt.sum() < 10:
+            return [], _slot_map(leaf_cluster_idx, filt, [])
+        return [lerf_range[0]], torch.where(filt, 0, -1).to(torch.int32)
+    if not lerf_range:
+        return [], _slot_map(leaf_cluster_idx, base, [])
+    counts = torch.bincount(leaf_cluster_idx[base & (leaf_cluster_idx >= 0)], minlength=max(lerf_range) + 1).tolist()
+    count = lambda idx: counts[idx] if 0 <= idx < len(counts) else 0          # noqa: E731
+    cand = [idx for idx in lerf_range if not (better_vis and count(idx) < 100)]
+    if not post_process:
+        cand = [idx for idx in cand if count(idx) >= 10]
+        return cand, _slot_map(leaf_cluster_idx, base, cand)
+    subset = _slot_map(leaf_cluster_idx, base, cand)
+    kept = []
+    for k, idx in enumerate(cand):
+        filt = subset == k
+        post = _post_process(filt, means3D)
+        subset = torch.where(filt & ~post, -1, subset).to(torch.int32)
+        if post.sum() >= 10:
+            kept.append(k)
+    lut = torch.full((len(cand) + 1,), -1, dtype=torch.int32, device=subset.device)     # renumber the kept slots
+    lut[torch.tensor(kept, dtype=torch.long, device=subset.device)] = torch.arange(len(kept), dtype=torch.int32,
+                                                                                  device=subset.device)
+    subset = torch.where(subset >= 0, lut[subset.long()], subset)
+    return [cand[k] for k in kept], subset
+
+
+def _use_batched(fused, *inputs):
+    """One forward_subsets call for all slots unless a gradient must reach an input (it has no backward) or the caller
+    asked for the reference's literal passes (fused=False)."""
+    return fused and not (torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs))
+
+
+def _render_slots(rasterizer, bg3, ids, subset, means3D, means2D, opacity, scales, rotations, cov3D_precomp, feat, shs,
+                  fused, keep_min_alpha=None):
+    """The images of the planned slots -> (images, silhouettes), lists in slot order, each entry as _feat_pass returns it.
+    keep_min_alpha: keep only the slots whose silhouette exceeds it somewhere (the coarse loop's test, :222), and
+    remove the others from `ids` in place."""
+    imgs, sils = [], []
+    if _use_batched(fused, means3D, opacity, scales, rotations, cov3D_precomp, feat, shs):
+        keep_ids = []
+        for a, b, img, sil in _render_slots_batched(rasterizer, bg3, len(ids), subset, means3D, opacity, scales,
+                                                    rotations, cov3D_precomp, feat, shs):
+            if keep_min_alpha is not None:
+                keep = (sil.amax(dim=(1, 2, 3)) > keep_min_alpha).tolist()       # one host read per launch
+                sel = [k for k in range(b - a) if keep[k]]
+                keep_ids += [ids[a + k] for k in sel]
+                if len(sel) != b - a:
+                    sel_t = torch.tensor(sel, dtype=torch.long, device=img.device)
+                    img, sil = img.index_select(0, sel_t), sil.index_select(0, sel_t)
+            imgs += list(img.unbind(0))
+            sils += list(sil.unbind(0))
+        if keep_min_alpha is not None:
+            ids[:] = keep_ids
+        return imgs, sils
+
+    def filt(t, idx):
+        return None if t is None else t[idx]
+
+    keep_ids = []
+    for k, idx in enumerate(ids):
+        filter_idx = subset == k
+        img, sil = _feat_pass(rasterizer, bg3, means3D[filter_idx], means2D[filter_idx], opacity[filter_idx],
+                              scales[filter_idx], rotations[filter_idx], filt(cov3D_precomp, filter_idx),
+                              feat[filter_idx], shs=filt(shs, filter_idx), fused=fused)
+        if keep_min_alpha is not None and not sil.max() > keep_min_alpha:
+            continue
+        keep_ids.append(idx)
+        imgs.append(img)
+        sils.append(sil)
+    ids[:] = keep_ids
+    return imgs, sils
+
+
+def _render_slots_batched(rasterizer, bg3, S, subset, means3D, opacity, scales, rotations, cov3D_precomp, feat, shs):
+    """forward_subsets over slots [a, b) per launch, each launch's outputs within SUBSET_BATCH_BYTES: yields
+    (a, b, images [b-a,F,H,W], silhouettes [b-a,1,H,W]) with the channel layout of _feat_pass."""
+    rs = rasterizer.raster_settings
+    H, W = int(rs.image_height), int(rs.image_width)
+    if shs is not None:
+        nb, kw = 0, dict(shs=shs)
+    elif feat.shape[-1] > 3:
+        nb = feat.shape[-1] - 3
+        kw = dict(colors_precomp=feat[:, :3], extra_feats=feat[:, 3:], extra_bg=torch.cat([bg3] * ((nb + 2) // 3))[:nb])
+    else:
+        nb, kw = 0, dict(colors_precomp=feat)
+    per_launch = max(1, SUBSET_BATCH_BYTES // ((3 + nb + 2) * H * W * 4))
+    for a in range(0, S, per_launch):
+        b = min(S, a + per_launch)
+        sub = subset if (a == 0 and b == S) else torch.where((subset >= a) & (subset < b), subset - a, -1)
+        color, _, alpha, extra = rasterizer.forward_subsets(means3D, opacity, sub, b - a, scales=scales,
+                                                            rotations=rotations, cov3D_precomp=cov3D_precomp, **kw)
+        if shs is not None:
+            img = torch.cat((color, color), dim=1)
+        elif extra is not None:
+            img = torch.cat((color, extra), dim=1)
+        else:
+            img = color.contiguous()
+        yield a, b, img, alpha
 
 
 def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
@@ -241,9 +411,6 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
                     means3D=means3D, means2D=means2D, shs=shs, colors_precomp=colors_precomp, opacities=opacity,
                     scales=sc(scales), rotations=rotations, cov3D_precomp=cov3D_precomp)
 
-    def filt(t, idx):
-        return None if t is None else t[idx]
-
     # ---- [Stage 2.2] coarse cluster-level feature maps (:173-236) ----
     viewed_pts = radii > 0
     if cluster_idx is not None:
@@ -253,28 +420,14 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
         cluster_occur = None
     if render_cluster and cluster_idx is not None and viewed_pts.sum() != 0:
         ins_feat = (pc.get_ins_feat(origin=origin_feat) + 1) / 2
-        rendered_clusters = []
-        rendered_cluster_silhouettes = []
         scale_filter = (scales < 0.5).all(dim=1)
-        for idx in range(num_cluster):
-            if not better_vis and idx != selected_root_id:
-                continue
-            if viewpoint_camera.bClusterOccur is not None and viewpoint_camera.bClusterOccur[idx] == False:  # noqa: E712
-                continue
-            filter_idx = cluster_idx == idx
-            filter_idx = filter_idx & viewed_pts
-            if better_vis:
-                filter_idx = filter_idx & scale_filter
-                if filter_idx.sum() < 100:
-                    continue
-            rendered_cluster, cluster_silhouette = _feat_pass(
-                rasterizer, bg3, means3D[filter_idx], means2D[filter_idx], opacity[filter_idx],
-                sc(scales[filter_idx]), rotations[filter_idx], filt(cov3D_precomp, filter_idx), ins_feat[filter_idx],
-                fused=fused)
-            if cluster_silhouette.max() > 0.8:
-                cluster_occur[idx] = True
-                rendered_clusters.append(rendered_cluster)
-                rendered_cluster_silhouettes.append(cluster_silhouette)
+        ids, subset = _plan_clusters(cluster_idx, int(num_cluster), viewed_pts, scale_filter, better_vis,
+                                     selected_root_id, viewpoint_camera.bClusterOccur)
+        rendered_clusters, rendered_cluster_silhouettes = _render_slots(
+            rasterizer, bg3, ids, subset, means3D, means2D, opacity, sc(scales), rotations, cov3D_precomp, ins_feat,
+            None, fused, keep_min_alpha=0.8)
+        for idx in ids:
+            cluster_occur[idx] = True
         if len(rendered_cluster_silhouettes) != 0:
             rendered_cluster_silhouettes = torch.vstack(rendered_cluster_silhouettes)
     else:
@@ -284,9 +437,6 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
     if leaf_cluster_idx is not None and leaf_cluster_idx.numel() > 0:
         ins_feat = (pc.get_ins_feat(origin=origin_feat) + 1) / 2
         scale_filter = (scales < 0.1).all(dim=1)
-        rendered_leaf_clusters = []
-        rendered_leaf_cluster_silhouettes = []
-        occured_leaf_id = []
         if selected_leaf_id is None:
             if selected_root_id is not None:
                 start_leaf = selected_root_id * leaf_num
@@ -297,40 +447,13 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
             lerf_range = range(start_leaf, end_leaf)
         else:
             lerf_range = selected_leaf_id.tolist()
-        for _, leaf_idx in enumerate(lerf_range):
-            if viewpoint_camera.bClusterOccur is not None and \
-                    viewpoint_camera.bClusterOccur[selected_root_id] == False:  # noqa: E712
-                continue
-            if selected_leaf_id is None:
-                filter_idx = leaf_cluster_idx == leaf_idx
-            else:
-                filter_idx = (leaf_cluster_idx.unsqueeze(1) == selected_leaf_id).any(dim=1)
-            if pre_mask is not None:
-                filter_idx = filter_idx & pre_mask
-            filter_idx = filter_idx & viewed_pts
-            if better_vis:
-                filter_idx = filter_idx & scale_filter
-                if filter_idx.sum() < 100:
-                    continue
-            max_time = 5
-            if post_process and max_time > 0:
-                nearest_k_distance = _knn_mean_dists(means3D[filter_idx].detach(), int(filter_idx.sum() ** 0.5))
-                mean_d, std_d = nearest_k_distance.mean(), nearest_k_distance.std()
-                mask = nearest_k_distance.mean(dim=-1) < mean_d + std_d
-                mask = mask.squeeze()
-                filter_idx[filter_idx != 0] = mask
-                max_time -= 1
-            if filter_idx.sum() < 10:
-                continue
-            occured_leaf_id.append(leaf_idx)
-            leaf_img, leaf_sil = _feat_pass(
-                rasterizer, bg3, means3D[filter_idx], means2D[filter_idx], opacity[filter_idx], scales[filter_idx],
-                rotations[filter_idx], filt(cov3D_precomp, filter_idx), ins_feat[filter_idx],
-                shs=shs[filter_idx] if seg_rgb else None, fused=fused)
-            rendered_leaf_clusters.append(leaf_img)
-            rendered_leaf_cluster_silhouettes.append(leaf_sil)
-            if selected_leaf_id is not None and len(rendered_leaf_clusters) > 0:
-                break
+        skip_all = len(lerf_range) > 0 and viewpoint_camera.bClusterOccur is not None and \
+            bool(viewpoint_camera.bClusterOccur[selected_root_id] == False)  # noqa: E712
+        occured_leaf_id, subset = _plan_leaves(leaf_cluster_idx, [] if skip_all else list(lerf_range), selected_leaf_id,
+                                               pre_mask, viewed_pts, scale_filter, better_vis, post_process, means3D)
+        rendered_leaf_clusters, rendered_leaf_cluster_silhouettes = _render_slots(
+            rasterizer, bg3, occured_leaf_id, subset, means3D, means2D, opacity, scales, rotations, cov3D_precomp,
+            ins_feat, shs if seg_rgb else None, fused)
         if len(rendered_leaf_cluster_silhouettes) != 0:
             rendered_leaf_cluster_silhouettes = torch.vstack(rendered_leaf_cluster_silhouettes)
     else:
