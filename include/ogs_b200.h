@@ -24,7 +24,11 @@
  *                                gaussian_renderer/__init__.py:174-236,245-356 (one per cluster or leaf, each
  *                                with its own gather, preprocess, sorts and blend), for all subsets of a view
  *                                in one call: one preprocess and binning, then a stable per-tile partition by
- *                                subset and one blend over (tiles x subsets).  Forward only.
+ *                                subset and one blend over (tiles x subsets).
+ *   ogs_raster_forward_subsets_state / ogs_raster_backward_subsets
+ *                                the same with the reference's backward through those passes (the gradient-carrying
+ *                                cluster pass of train.py:475-489): a forward that keeps its state and one blend
+ *                                backward over (tiles x subsets).
  *   ogs_mark_visible             upstream GaussianRasterizer.markVisible (mark_visible symbol)
  *   ogs_raster_export            debug view of the geometry records and the sorted (tile|depth) keys
  *                                (upstream geomState / binningState)
@@ -209,13 +213,14 @@ int64_t ogs_raster_capacity_hint(int64_t new_hint);
 
 size_t ogs_raster_backward_scratch_floats(int32_t P, int32_t n_extra);
 
-/* ---- all subsets of a view in one call (render()'s no-grad cluster / leaf passes) ----
+/* ---- all subsets of a view in one call (render()'s cluster / leaf passes) ----
  * subset int32 [P]: slot in [0, S) or -1 (not rendered; any value outside [0, S) is treated as -1).  Every slot's
  * images equal, bit for bit, an ogs_raster_forward of the rows with subset == slot (in increasing index order):
  * a pass over a subset sorts its rows stably by depth, then stably by tile, so its tile lists are the frame's lists
  * restricted to the subset, in the same order.  The call runs one preprocess and one binning over the Gaussians
  * that belong to a slot, partitions each tile's list stably by slot and blends all (tile, slot) pairs in one launch.
- * Inputs as for ogs_raster_forward, activated (act_flags == 0).  Forward only: no state, no radii.
+ * Inputs as for ogs_raster_forward, activated (act_flags == 0).  No radii; ogs_raster_forward_subsets keeps no state
+ * (forward only), ogs_raster_forward_subsets_state below does.
  * Reads the frame's duplicate count synchronously (one host wait per call) and leaves the running capacity
  * estimate of ogs_raster_capacity_hint untouched.  Temporaries come from `alloc` (tags "geom", "binning") and the
  * stream-ordered pool.  1 <= S <= OGS_MAX_SUBSETS (the partition kernel keeps S counters in shared memory). */
@@ -227,6 +232,20 @@ typedef struct ogs_subset_outputs {
 } ogs_subset_outputs;
 int ogs_raster_forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, int32_t S,
                                const ogs_subset_outputs* out, ogs_alloc_fn alloc, void* alloc_user, void* stream);
+/* ogs_raster_forward_subsets that also fills `state` for ogs_raster_backward_subsets: the same images, bit for bit, plus
+ * an "image" buffer from `alloc` (final_T float[S][H][W], then n_contrib uint32[S][H][W]: S * H * W * 8 bytes) that
+ * stays alive with "geom" and "binning" (which holds the frame's and the partitioned tile lists) until the backward
+ * has run.  state->num_rendered = N of the frame. */
+int ogs_raster_forward_subsets_state(const ogs_raster_inputs* in, const int32_t* subset, int32_t S,
+                                     const ogs_subset_outputs* out, ogs_alloc_fn alloc, void* alloc_user,
+                                     ogs_raster_state* state, void* stream);
+/* Backward of ogs_raster_forward_subsets_state (same inputs, same S).  gin holds every slot's image gradients:
+ * dL_dcolor [S, 3 + n_extra, H, W], or with dL_dfeat set [S, 3, H, W] or NULL; dL_dfeat [S, n_extra, H, W];
+ * dL_ddepth, dL_dalpha [S, H, W] or NULL.  gout as for ogs_raster_backward, per Gaussian: the subsets are disjoint, so
+ * each Gaussian's gradient is that of its own slot's images, and Gaussians of no slot get zero.  accumulate must be 0.
+ * A state whose buffer sizes do not match P, S, W and H (a state of another call) is an argument error. */
+int ogs_raster_backward_subsets(const ogs_raster_inputs* in, int32_t S, const ogs_raster_state* state,
+                                const ogs_raster_grads_in* gin, const ogs_raster_grads_out* gout, void* stream);
 
 int ogs_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, uint8_t* present,
                      void* stream);

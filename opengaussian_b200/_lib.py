@@ -84,6 +84,10 @@ EXPORTS = {
                                             C.POINTER(RasterState), C.POINTER(RasterState), C.c_void_p]),
     "ogs_raster_forward_subsets": (C.c_int, [C.POINTER(RasterInputs), _fp, C.c_int32, C.POINTER(SubsetOutputs), ALLOC_FN,
                                              C.c_void_p, C.c_void_p]),
+    "ogs_raster_forward_subsets_state": (C.c_int, [C.POINTER(RasterInputs), _fp, C.c_int32, C.POINTER(SubsetOutputs),
+                                                   ALLOC_FN, C.c_void_p, C.POINTER(RasterState), C.c_void_p]),
+    "ogs_raster_backward_subsets": (C.c_int, [C.POINTER(RasterInputs), C.c_int32, C.POINTER(RasterState),
+                                              C.POINTER(RasterGradsIn), C.POINTER(RasterGradsOut), C.c_void_p]),
     "ogs_raster_cached_bytes": (C.c_int, [C.POINTER(RasterInputs), C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "ogs_raster_capacity_check": (C.c_int, []),
     "ogs_raster_capacity_hint": (C.c_int64, [C.c_int64]),

@@ -24,6 +24,10 @@
 //    summed and ONE red.global.add per value per (tile, Gaussian) is issued, skipping zeros;
 //  * GEOM=false specialisation (OpenGaussian stages 1-2 detach geometry, train.py:431-436): only
 //    w = alpha T and dL/dc are evaluated.
+// SUBSETS = true (ogs_raster_backward_subsets): blockIdx.z is a subset; its tile lists start at ranges + z * tiles
+// (the partitioned lists of ogs_raster_forward_subsets_state), its final_T / n_contrib and depth / alpha gradients at
+// z * H * W, its colour gradients at z * (3 or C) * H * W and its feature gradients at z * (C - 3) * H * W.  The
+// subsets are disjoint, so a Gaussian's accumulator row only receives its own subset's contributions.
 #include "common.cuh"
 #include <stdlib.h>
 
@@ -95,7 +99,7 @@ constexpr int bwd_min_blocks(int C, int pairs, bool geom = true) { return (pairs
 // loss -- so their pixel gradients are not loaded, their weighted sums not formed and not reduced across the lanes
 // (6 of 9 values: a third of the FFMA2s and of the reduction of every evaluated entry).  The accumulator rows keep
 // their C columns (preprocess_bwd reads them by column); columns [0, C0) stay zero.
-template <int C, bool GEOM, int PAIRS, int C0 = 0>
+template <int C, bool GEOM, int PAIRS, int C0 = 0, bool SUBSETS = false>
 __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEOM || C0 == 0)) blend_bwd_kernel(BlendBwdArgs a) {
     static_assert(C0 == 0 || !GEOM, "the geometry gradients need every channel");
     constexpr int BWD_THREADS = 128 / PAIRS, BWD_WARPS = 4 / PAIRS, NPX = 2 * PAIRS;
@@ -120,7 +124,9 @@ __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEO
     const float pxf = (float)px;
     const float bx0 = (float)bxi, by0 = (float)byi;
     const size_t HW = (size_t)a.H * a.W;
-    const uint2 range = a.ranges[tile];
+    const size_t z = SUBSETS ? blockIdx.z : 0;                       // 0 folds every offset below away
+    const size_t zc = SUBSETS ? z * (a.dL_dfeat ? 3 : C) * HW : 0;  // colour planes per subset: 3 with dL_dfeat, else C
+    const uint2 range = a.ranges[tile + z * gx * gridDim.y];
 
     // per-lane state of the pixel pairs (.x: row y + 8 p, .y: row y + 8 p + 4)
     float2 T2[PAIRS], S2[PAIRS], gd2[PAIRS], ga2[PAIRS], tfbg2[PAIRS], npy[PAIRS];
@@ -136,19 +142,19 @@ __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEO
             const int py = y0 + 4 * k;
             const bool inside = px < a.W && py < a.H;
             const size_t pix = (size_t)py * a.W + px;
-            last[2 * p + k] = inside ? (int)a.n_contrib[pix] : 0;
-            Tf[k] = inside ? a.final_T[pix] : 0.f;
+            last[2 * p + k] = inside ? (int)a.n_contrib[z * HW + pix] : 0;
+            Tf[k] = inside ? a.final_T[z * HW + pix] : 0.f;
 #pragma unroll
             for (int cc = 0; cc < CG; cc++) {
                 const int c = C0 + cc;
-                const float* plane = (a.dL_dfeat && c >= 3) ? a.dL_dfeat + (size_t)(c - 3) * HW
-                                                            : (a.dL_dcolor ? a.dL_dcolor + (size_t)c * HW : nullptr);
+                const float* plane = (a.dL_dfeat && c >= 3) ? a.dL_dfeat + (z * (C - 3) + (size_t)(c - 3)) * HW
+                                                            : (a.dL_dcolor ? a.dL_dcolor + zc + (size_t)c * HW : nullptr);
                 gv[k][cc] = (inside && plane) ? __ldg(plane + pix) : 0.f;
                 if constexpr (GEOM) bgd[k] = fmaf(__ldg(a.bg + c), gv[k][cc], bgd[k]);
             }
             if constexpr (GEOM) {
-                gdv[k] = (inside && a.dL_ddepth) ? __ldg(a.dL_ddepth + pix) : 0.f;
-                gav[k] = (inside && a.dL_dalpha) ? __ldg(a.dL_dalpha + pix) : 0.f;
+                gdv[k] = (inside && a.dL_ddepth) ? __ldg(a.dL_ddepth + z * HW + pix) : 0.f;
+                gav[k] = (inside && a.dL_dalpha) ? __ldg(a.dL_dalpha + z * HW + pix) : 0.f;
             }
         }
         npy[p] = make_float2(-(float)y0, -(float)(y0 + 4));
@@ -313,47 +319,52 @@ __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEO
     }
 }
 
-template <int C, bool GEOM, int C0 = 0>
-static int launch_cg(const BlendBwdArgs& a, cudaStream_t s) {
+template <int C, bool GEOM, int C0, bool SUBSETS>
+static int launch_cg(const BlendBwdArgs& a, int S, cudaStream_t s) {
     constexpr int V = GEOM ? C + 7 : C;
     // two pairs per lane pay off while the pixel state fits the register file comfortably (measured: C <= 9)
     static const int env_pairs = getenv("OGS_BWD_PAIRS") ? atoi(getenv("OGS_BWD_PAIRS")) : 0;  // tuning knob
     const int pairs = env_pairs ? env_pairs : (C <= 9 ? 2 : 1);
-    dim3 grid((a.W + 15) / 16, (a.H + 15) / 16);
+    dim3 grid((a.W + 15) / 16, (a.H + 15) / 16, S);
     const size_t smem = (size_t)2 * (4 / (pairs == 2 ? 2 : 1)) * BB * V * sizeof(float);
     static PerDeviceOnce attr_done[2];
     if (smem > 24 * 1024 && attr_done[pairs == 2].todo()) {   // static + dynamic shared memory may pass the 48 KB default
-        if (pairs == 2) OGS_CUDA(cudaFuncSetAttribute(blend_bwd_kernel<C, GEOM, 2, C0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-        else OGS_CUDA(cudaFuncSetAttribute(blend_bwd_kernel<C, GEOM, 1, C0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+        if (pairs == 2) OGS_CUDA(cudaFuncSetAttribute(blend_bwd_kernel<C, GEOM, 2, C0, SUBSETS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+        else OGS_CUDA(cudaFuncSetAttribute(blend_bwd_kernel<C, GEOM, 1, C0, SUBSETS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
         attr_done[pairs == 2].done();
     }
-    if (pairs == 2) blend_bwd_kernel<C, GEOM, 2, C0><<<grid, 64, smem, s>>>(a);
-    else blend_bwd_kernel<C, GEOM, 1, C0><<<grid, 128, smem, s>>>(a);
+    if (pairs == 2) blend_bwd_kernel<C, GEOM, 2, C0, SUBSETS><<<grid, 64, smem, s>>>(a);
+    else blend_bwd_kernel<C, GEOM, 1, C0, SUBSETS><<<grid, 128, smem, s>>>(a);
     return 0;
 }
 
-template <int C>
-static int launch_c(const BlendBwdArgs& a, cudaStream_t s) {
-    if (a.geom) return launch_cg<C, true>(a, s);
+template <int C, bool SUBSETS>
+static int launch_c(const BlendBwdArgs& a, int S, cudaStream_t s) {
+    if (a.geom) return launch_cg<C, true, 0, SUBSETS>(a, S, s);
     if constexpr (C > 3) {
-        if (!a.dL_dcolor && a.dL_dfeat) return launch_cg<C, false, 3>(a, s);   // only the feature channels carry a gradient
+        if (!a.dL_dcolor && a.dL_dfeat) return launch_cg<C, false, 3, SUBSETS>(a, S, s);   // only the feature channels carry a gradient
     }
-    return launch_cg<C, false>(a, s);
+    return launch_cg<C, false, 0, SUBSETS>(a, S, s);
 }
 
-int launch_blend_backward(const BlendBwdArgs& a, cudaStream_t s) {
+template <bool SUBSETS>
+static int launch_any(const BlendBwdArgs& a, int S, cudaStream_t s) {
     cudaError_t e = cudaMemsetAsync(a.acc, 0, (size_t)a.P * a.stride * sizeof(float), s);
     if (e != cudaSuccess) return cuda_fail(e, "memset acc");
     switch (a.C) {
-        case 3: return launch_c<3>(a, s);
-        case 4: return launch_c<4>(a, s);
-        case 6: return launch_c<6>(a, s);
-        case 9: return launch_c<9>(a, s);
-        case 12: return launch_c<12>(a, s);
-        case 16: return launch_c<16>(a, s);
+        case 3: return launch_c<3, SUBSETS>(a, S, s);
+        case 4: return launch_c<4, SUBSETS>(a, S, s);
+        case 6: return launch_c<6, SUBSETS>(a, S, s);
+        case 9: return launch_c<9, SUBSETS>(a, S, s);
+        case 12: return launch_c<12, SUBSETS>(a, S, s);
+        case 16: return launch_c<16, SUBSETS>(a, S, s);
     }
     set_error("blend backward: unsupported channel count %d", a.C);
     return -4;
 }
+
+int launch_blend_backward(const BlendBwdArgs& a, cudaStream_t s) { return launch_any<false>(a, 1, s); }
+
+int launch_blend_backward_subsets(const BlendBwdArgs& a, int S, cudaStream_t s) { return launch_any<true>(a, S, s); }
 
 }  // namespace ogs

@@ -23,7 +23,8 @@
 // warp's block (ogs_rect_hit_s) and only the ballot survivors are blended.
 // SUBSETS = true (ogs_raster_forward_subsets): blockIdx.z is a subset; its tile lists start at
 // ranges + z * tiles and its images at z * C * H * W (colour) and z * H * W (depth, alpha; depth may be
-// NULL).  No final_T / n_contrib: that path has no backward.
+// NULL).  final_T / n_contrib (ogs_raster_forward_subsets_state) go to z * H * W + pixel when set, n_contrib
+// counted inside the slot's own tile segment; NULL (ogs_raster_forward_subsets) writes no state.
 #include "common.cuh"
 #include <stdlib.h>
 
@@ -155,6 +156,10 @@ __global__ void __launch_bounds__(128 / PAIRS) blend_fwd_kernel(BlendFwdArgs a) 
                     a.out_color[(z * C + c) * HW + pix] = ((k & 1) ? acc[p][c].y : acc[p][c].x) + T * __ldg(a.bg + c);
                 if (a.out_depth) a.out_depth[z * HW + pix] = (k & 1) ? acc[p][C].y : acc[p][C].x;
                 a.out_alpha[z * HW + pix] = 1.0f - T;
+                if (a.final_T) {
+                    a.final_T[z * HW + pix] = T;
+                    a.n_contrib[z * HW + pix] = last[k];
+                }
             } else {
                 a.final_T[pix] = T;
                 a.n_contrib[pix] = last[k];

@@ -159,6 +159,170 @@ static int validate_inputs(const ogs_raster_inputs* in) {
     return 0;
 }
 
+// The buffers of a subset pass (ogs_raster_forward_subsets_state) that its backward reads back: the binning buffer holds
+// the frame's lists and ranges (BinLayout), then the lists partitioned by subset and the [S][tiles] segment bounds; the
+// image buffer holds final_T and n_contrib of every subset, [S][H][W] each.
+struct SubsetBinLayout {
+    BinLayout frame;
+    size_t seg_list, sub_ranges, total;
+    static SubsetBinLayout make(int64_t N, int tiles, int S) {
+        SubsetBinLayout l;
+        l.frame = BinLayout::make(N, tiles);
+        l.seg_list = l.frame.total;
+        l.sub_ranges = align_up(l.seg_list + (size_t)(N > 0 ? N : 1) * 4, 256);
+        l.total = l.sub_ranges + (size_t)S * tiles * sizeof(uint2);
+        return l;
+    }
+};
+
+static ImgLayout subset_img_layout(int W, int H, int S) {
+    const size_t n = (size_t)S * W * H;
+    ImgLayout l;
+    l.final_T = 0;
+    l.n_contrib = align_up(n * 4, 256);
+    l.total = align_up(l.n_contrib + n * 4, 256);
+    return l;
+}
+
+// The parameter gradients from the blend's per-Gaussian accumulators (shared by the frame and subset backwards).
+static int preprocess_backward(const ogs_raster_inputs* in, const GeomPtrs& g, const ogs_raster_grads_out* go,
+                               float* acc, int stride, int geom, cudaStream_t s) {
+    PreprocessBwdArgs pa;
+    pa.P = in->P; pa.D = in->sh_degree; pa.M = in->M; pa.C = 3 + in->n_extra; pa.W = in->W; pa.H = in->H;
+    pa.act_flags = in->act_flags; pa.shs_rest = in->shs_rest; pa.extra = in->extra; pa.opacities = in->opacities;
+    pa.dL_dshs_rest = go->dL_dshs_rest; pa.accumulate = go->accumulate;
+    pa.means3D = in->means3D; pa.scales = in->scales; pa.rotations = in->rotations;
+    pa.cov3D_precomp = in->cov3D_precomp; pa.shs = in->shs;
+    pa.scale_modifier = in->scale_modifier; pa.tanfovx = in->tanfovx; pa.tanfovy = in->tanfovy;
+    pa.view = in->viewmatrix; pa.proj = in->projmatrix; pa.campos = in->campos;
+    pa.g = g; pa.acc = acc; pa.stride = stride; pa.geom = geom;
+    pa.dL_dmeans3D = go->dL_dmeans3D; pa.dL_dmeans2D = go->dL_dmeans2D; pa.dL_dopacities = go->dL_dopacities;
+    pa.dL_dshs = go->dL_dshs; pa.dL_dcolors_precomp = go->dL_dcolors_precomp; pa.dL_dscales = go->dL_dscales;
+    pa.dL_drotations = go->dL_drotations; pa.dL_dcov3D = go->dL_dcov3D; pa.dL_dextra = go->dL_dextra;
+    prof_begin(PF_PREPROCESS_BWD, s);
+    const int rc = launch_preprocess_backward(pa, s);
+    prof_end(PF_PREPROCESS_BWD, s);
+    if (rc) return rc;
+    OGS_KERNEL_CHECK("preprocess_backward", in->debug, s);
+    return 0;
+}
+
+static int forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, int32_t S, const ogs_subset_outputs* out,
+                           ogs_alloc_fn alloc, void* alloc_user, ogs_raster_state* st, cudaStream_t s) {
+    int rc = validate_inputs(in);
+    if (rc) return rc;
+    if (in->P > 0 && !subset) { set_error("forward_subsets: subset is NULL"); return -1; }
+    if (S < 1 || S > OGS_MAX_SUBSETS) { set_error("forward_subsets: S=%d out of range [1, %d]", S, OGS_MAX_SUBSETS); return -1; }
+    if (in->act_flags != 0) { set_error("forward_subsets: needs activated inputs (act_flags == 0)"); return -1; }
+    if (!out || !out->color || !out->alpha || !alloc) { set_error("forward_subsets: outputs/alloc must be set"); return -1; }
+    if ((rc = ensure_pool())) return rc;
+    const int P = in->P, W = in->W, H = in->H, C = 3 + in->n_extra;
+    const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
+    const bool has_sh = in->shs != nullptr;
+    const GeomLayout gl = GeomLayout::make(P, has_sh, 0);
+    void* geom = alloc(alloc_user, gl.total, "geom");
+    if (!geom) { set_error("allocation callback returned NULL"); return -6; }
+    const GeomPtrs g = GeomPtrs::from(geom, gl);
+    const ImgLayout il = subset_img_layout(W, H, S);
+    void* image = nullptr;
+    if (st) {
+        image = alloc(alloc_user, il.total, "image");
+        if (!image) { set_error("allocation callback returned NULL"); return -6; }
+    }
+
+    int64_t N = 0;
+    AsyncScratch scratch1(s);
+    BinScratch sc;
+    memset(&sc, 0, sizeof sc);
+    if (P > 0) {
+        const size_t pw = align_up((size_t)(P + 2) * 4, 256);
+        sc.cub_temp_bytes = align_up(depth_sort_temp_bytes(P), 256);
+        OGS_CUDA(scratch1.alloc(pw * 6 + sc.cub_temp_bytes));
+        char* s1 = (char*)scratch1.p;
+        sc.dkeys_in = (uint32_t*)(s1);
+        sc.dvals_in = (uint32_t*)(s1 + pw);
+        sc.dkeys_out = (uint32_t*)(s1 + 2 * pw);
+        sc.dvals_out = (uint32_t*)(s1 + 3 * pw);
+        sc.offsets = (uint32_t*)(s1 + 4 * pw);
+        int32_t* radii = (int32_t*)(s1 + 5 * pw);
+        sc.cub_temp = s1 + 6 * pw;
+
+        PreprocessArgs pa;
+        pa.P = P; pa.D = in->sh_degree; pa.M = in->M; pa.W = W; pa.H = H;
+        pa.act_flags = 0; pa.n_extra = in->n_extra; pa.shs_rest = in->shs_rest; pa.extra = in->extra;
+        pa.means3D = in->means3D; pa.scales = in->scales; pa.rotations = in->rotations;
+        pa.cov3D_precomp = in->cov3D_precomp; pa.opacities = in->opacities; pa.shs = in->shs;
+        pa.scale_modifier = in->scale_modifier; pa.tanfovx = in->tanfovx; pa.tanfovy = in->tanfovy;
+        pa.view = in->viewmatrix; pa.proj = in->projmatrix; pa.campos = in->campos;
+        pa.radii = radii; pa.g = g; pa.depth_keys = sc.dkeys_in; pa.depth_vals = sc.dvals_in;
+        prof_begin(PF_PREPROCESS_FWD, s);
+        rc = launch_preprocess_forward(pa, s);
+        if (!rc) rc = launch_subset_exclude(P, S, subset, sc.dkeys_in, s);     // rows of no slot: the culled key
+        prof_end(PF_PREPROCESS_FWD, s);
+        if (rc) return rc;
+        OGS_KERNEL_CHECK("preprocess_forward (subsets)", in->debug, s);
+        prof_begin(PF_DEPTH_SORT_SCAN, s);
+        rc = depth_sort_and_scan(P, g, sc, s, in->debug);
+        prof_end(PF_DEPTH_SORT_SCAN, s);
+        if (rc) return rc;
+        uint32_t* h = pinned_scalar(forward_ctx());     // the synchronous-check words: free between calls of this thread
+        if (!h) { set_error("cudaMallocHost failed"); return 2; }
+        OGS_CUDA(cudaMemcpyAsync(h, sc.offsets + P, 8, cudaMemcpyDeviceToHost, s));
+        OGS_CUDA(cudaStreamSynchronize(s));
+        if (h[1]) { set_error("more than 2^32 - 1 (Gaussian, tile) duplicates in one frame: 32-bit offsets overflow"); return -7; }
+        N = (int64_t)h[0];
+    }
+
+    // binning: the frame's lists and ranges, then the partitioned lists and the [S][tiles] segment bounds
+    const SubsetBinLayout bl = SubsetBinLayout::make(N, tiles, S);
+    char* binning = (char*)alloc(alloc_user, bl.total, "binning");
+    if (!binning) { set_error("allocation callback returned NULL"); return -6; }
+    uint32_t* point_list = (uint32_t*)(binning + bl.frame.point_list);
+    uint2* ranges = (uint2*)(binning + bl.frame.ranges);
+    uint32_t* seg_list = (uint32_t*)(binning + bl.seg_list);
+    uint2* sub_ranges = (uint2*)(binning + bl.sub_ranges);
+    if (N > 0) {
+        AsyncScratch scratch2(s);
+        const size_t k2 = align_up((size_t)N * 2, 256), v4 = align_up((size_t)N * 4, 256);
+        const size_t tb = align_up(tile_sort_temp_bytes(N), 256);
+        OGS_CUDA(scratch2.alloc(2 * k2 + v4 + tb));
+        char* s2 = (char*)scratch2.p;
+        sc.cub_temp = s2 + 2 * k2 + v4;
+        sc.cub_temp_bytes = tb;
+        rc = emit_sort_ranges(P, W, H, sc.offsets + P, N, g, sc, (uint16_t*)s2, (uint32_t*)(s2 + 2 * k2),
+                              (uint16_t*)(s2 + k2), point_list, ranges, s, in->debug);
+        if (rc) return rc;
+        prof_begin(PF_RANGES, s);
+        rc = launch_subset_partition(tiles, S, ranges, point_list, subset, seg_list, sub_ranges, s);
+        prof_end(PF_RANGES, s);
+        if (rc) return rc;
+        OGS_KERNEL_CHECK("subset_partition", in->debug, s);
+    } else {
+        OGS_CUDA(cudaMemsetAsync(sub_ranges, 0, (size_t)S * tiles * sizeof(uint2), s));
+    }
+
+    BlendFwdArgs ba;
+    ba.W = W; ba.H = H; ba.C = C;
+    ba.ranges = sub_ranges; ba.point_list = seg_list; ba.rec0 = g.rec0; ba.rec1 = g.rec1;
+    ba.base = has_sh ? g.rgb : in->colors_precomp;
+    ba.extra = in->extra; ba.bg = in->bg;
+    ba.out_color = out->color; ba.out_depth = out->depth; ba.out_alpha = out->alpha;
+    ba.final_T = image ? (float*)((char*)image + il.final_T) : nullptr;
+    ba.n_contrib = image ? (uint32_t*)((char*)image + il.n_contrib) : nullptr;
+    prof_begin(PF_BLEND_FWD, s);
+    rc = launch_blend_forward_subsets(ba, S, s);
+    prof_end(PF_BLEND_FWD, s);
+    if (rc) return rc;
+    OGS_KERNEL_CHECK("blend_forward_subsets", in->debug, s);
+    if (st) {
+        memset(st, 0, sizeof *st);
+        st->geom = geom; st->binning = binning; st->image = image;
+        st->num_rendered = N;
+        st->geom_bytes = (int64_t)gl.total; st->binning_bytes = (int64_t)bl.total; st->image_bytes = (int64_t)il.total;
+    }
+    return 0;
+}
+
 }  // namespace ogs
 
 using namespace ogs;
@@ -361,108 +525,63 @@ int ogs_raster_forward(const ogs_raster_inputs* in, const ogs_raster_outputs* ou
 
 int ogs_raster_forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, int32_t S, const ogs_subset_outputs* out,
                                ogs_alloc_fn alloc, void* alloc_user, void* stream_) {
+    return forward_subsets(in, subset, S, out, alloc, alloc_user, nullptr, (cudaStream_t)stream_);
+}
+
+int ogs_raster_forward_subsets_state(const ogs_raster_inputs* in, const int32_t* subset, int32_t S,
+                                     const ogs_subset_outputs* out, ogs_alloc_fn alloc, void* alloc_user,
+                                     ogs_raster_state* st, void* stream_) {
+    if (!st) { set_error("forward_subsets_state: state is NULL"); return -1; }
+    return forward_subsets(in, subset, S, out, alloc, alloc_user, st, (cudaStream_t)stream_);
+}
+
+int ogs_raster_backward_subsets(const ogs_raster_inputs* in, int32_t S, const ogs_raster_state* st,
+                                const ogs_raster_grads_in* gin, const ogs_raster_grads_out* go, void* stream_) {
     int rc = validate_inputs(in);
     if (rc) return rc;
-    if (in->P > 0 && !subset) { set_error("forward_subsets: subset is NULL"); return -1; }
-    if (S < 1 || S > OGS_MAX_SUBSETS) { set_error("forward_subsets: S=%d out of range [1, %d]", S, OGS_MAX_SUBSETS); return -1; }
-    if (in->act_flags != 0) { set_error("forward_subsets: needs activated inputs (act_flags == 0)"); return -1; }
-    if (!out || !out->color || !out->alpha || !alloc) { set_error("forward_subsets: outputs/alloc must be set"); return -1; }
-    cudaStream_t s = (cudaStream_t)stream_;
-    if ((rc = ensure_pool())) return rc;
+    if (S < 1 || S > OGS_MAX_SUBSETS) { set_error("backward_subsets: S=%d out of range [1, %d]", S, OGS_MAX_SUBSETS); return -1; }
+    if (in->act_flags != 0) { set_error("backward_subsets: needs activated inputs (act_flags == 0)"); return -1; }
+    if (!st || !gin || !go || (!gin->dL_dcolor && !gin->dL_dfeat) || !go->scratch) { set_error("state/grads/scratch must be set"); return -1; }
+    if (gin->dL_dfeat && in->n_extra <= 0) { set_error("dL_dfeat needs n_extra > 0"); return -1; }
+    if (go->accumulate) { set_error("backward_subsets: accumulate is not supported"); return -1; }
+    if (go->dL_dshs_rest && !go->dL_dshs) { set_error("dL_dshs_rest needs dL_dshs"); return -1; }
     const int P = in->P, W = in->W, H = in->H, C = 3 + in->n_extra;
     const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
     const bool has_sh = in->shs != nullptr;
     const GeomLayout gl = GeomLayout::make(P, has_sh, 0);
-    void* geom = alloc(alloc_user, gl.total, "geom");
-    if (!geom) { set_error("allocation callback returned NULL"); return -6; }
-    const GeomPtrs g = GeomPtrs::from(geom, gl);
-
-    int64_t N = 0;
-    AsyncScratch scratch1(s);
-    BinScratch sc;
-    memset(&sc, 0, sizeof sc);
-    if (P > 0) {
-        const size_t pw = align_up((size_t)(P + 2) * 4, 256);
-        sc.cub_temp_bytes = align_up(depth_sort_temp_bytes(P), 256);
-        OGS_CUDA(scratch1.alloc(pw * 6 + sc.cub_temp_bytes));
-        char* s1 = (char*)scratch1.p;
-        sc.dkeys_in = (uint32_t*)(s1);
-        sc.dvals_in = (uint32_t*)(s1 + pw);
-        sc.dkeys_out = (uint32_t*)(s1 + 2 * pw);
-        sc.dvals_out = (uint32_t*)(s1 + 3 * pw);
-        sc.offsets = (uint32_t*)(s1 + 4 * pw);
-        int32_t* radii = (int32_t*)(s1 + 5 * pw);
-        sc.cub_temp = s1 + 6 * pw;
-
-        PreprocessArgs pa;
-        pa.P = P; pa.D = in->sh_degree; pa.M = in->M; pa.W = W; pa.H = H;
-        pa.act_flags = 0; pa.n_extra = in->n_extra; pa.shs_rest = in->shs_rest; pa.extra = in->extra;
-        pa.means3D = in->means3D; pa.scales = in->scales; pa.rotations = in->rotations;
-        pa.cov3D_precomp = in->cov3D_precomp; pa.opacities = in->opacities; pa.shs = in->shs;
-        pa.scale_modifier = in->scale_modifier; pa.tanfovx = in->tanfovx; pa.tanfovy = in->tanfovy;
-        pa.view = in->viewmatrix; pa.proj = in->projmatrix; pa.campos = in->campos;
-        pa.radii = radii; pa.g = g; pa.depth_keys = sc.dkeys_in; pa.depth_vals = sc.dvals_in;
-        prof_begin(PF_PREPROCESS_FWD, s);
-        rc = launch_preprocess_forward(pa, s);
-        if (!rc) rc = launch_subset_exclude(P, S, subset, sc.dkeys_in, s);     // rows of no slot: the culled key
-        prof_end(PF_PREPROCESS_FWD, s);
-        if (rc) return rc;
-        OGS_KERNEL_CHECK("preprocess_forward (subsets)", in->debug, s);
-        prof_begin(PF_DEPTH_SORT_SCAN, s);
-        rc = depth_sort_and_scan(P, g, sc, s, in->debug);
-        prof_end(PF_DEPTH_SORT_SCAN, s);
-        if (rc) return rc;
-        uint32_t* h = pinned_scalar(forward_ctx());     // the synchronous-check words: free between calls of this thread
-        if (!h) { set_error("cudaMallocHost failed"); return 2; }
-        OGS_CUDA(cudaMemcpyAsync(h, sc.offsets + P, 8, cudaMemcpyDeviceToHost, s));
-        OGS_CUDA(cudaStreamSynchronize(s));
-        if (h[1]) { set_error("more than 2^32 - 1 (Gaussian, tile) duplicates in one frame: 32-bit offsets overflow"); return -7; }
-        N = (int64_t)h[0];
+    const ImgLayout il = subset_img_layout(W, H, S);
+    if (!st->geom || !st->binning || !st->image || st->num_rendered < 0 || st->geom_bytes != (int64_t)gl.total ||
+        st->image_bytes != (int64_t)il.total ||
+        st->binning_bytes != (int64_t)SubsetBinLayout::make(st->num_rendered, tiles, S).total) {
+        set_error("backward_subsets: state does not belong to a forward_subsets_state of these sizes (P=%d, S=%d, %dx%d)",
+                  P, S, W, H);
+        return -1;
     }
-
-    // binning: the frame's lists and ranges, then the partitioned lists and the [S][tiles] segment bounds
-    const BinLayout bl = BinLayout::make(N, tiles);
-    const size_t seg_list_off = bl.total;
-    const size_t sub_ranges_off = align_up(seg_list_off + (size_t)(N > 0 ? N : 1) * 4, 256);
-    char* binning = (char*)alloc(alloc_user, sub_ranges_off + (size_t)S * tiles * sizeof(uint2), "binning");
-    if (!binning) { set_error("allocation callback returned NULL"); return -6; }
-    uint32_t* point_list = (uint32_t*)(binning + bl.point_list);
-    uint2* ranges = (uint2*)(binning + bl.ranges);
-    uint32_t* seg_list = (uint32_t*)(binning + seg_list_off);
-    uint2* sub_ranges = (uint2*)(binning + sub_ranges_off);
-    if (N > 0) {
-        AsyncScratch scratch2(s);
-        const size_t k2 = align_up((size_t)N * 2, 256), v4 = align_up((size_t)N * 4, 256);
-        const size_t tb = align_up(tile_sort_temp_bytes(N), 256);
-        OGS_CUDA(scratch2.alloc(2 * k2 + v4 + tb));
-        char* s2 = (char*)scratch2.p;
-        sc.cub_temp = s2 + 2 * k2 + v4;
-        sc.cub_temp_bytes = tb;
-        rc = emit_sort_ranges(P, W, H, sc.offsets + P, N, g, sc, (uint16_t*)s2, (uint32_t*)(s2 + 2 * k2),
-                              (uint16_t*)(s2 + k2), point_list, ranges, s, in->debug);
-        if (rc) return rc;
-        prof_begin(PF_RANGES, s);
-        rc = launch_subset_partition(tiles, S, ranges, point_list, subset, seg_list, sub_ranges, s);
-        prof_end(PF_RANGES, s);
-        if (rc) return rc;
-        OGS_KERNEL_CHECK("subset_partition", in->debug, s);
-    } else {
-        OGS_CUDA(cudaMemsetAsync(sub_ranges, 0, (size_t)S * tiles * sizeof(uint2), s));
-    }
-
-    BlendFwdArgs ba;
-    ba.W = W; ba.H = H; ba.C = C;
-    ba.ranges = sub_ranges; ba.point_list = seg_list; ba.rec0 = g.rec0; ba.rec1 = g.rec1;
+    if (P == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream_;
+    const SubsetBinLayout bl = SubsetBinLayout::make(st->num_rendered, tiles, S);
+    const GeomPtrs g = GeomPtrs::from(st->geom, gl);
+    const int geom = (go->dL_dmeans3D || go->dL_dmeans2D || go->dL_dopacities || go->dL_dshs || go->dL_dshs_rest ||
+                      go->dL_dscales || go->dL_drotations || go->dL_dcov3D) ? 1 : 0;
+    BlendBwdArgs ba;
+    ba.P = P; ba.W = W; ba.H = H; ba.C = C;
+    ba.ranges = (const uint2*)((char*)st->binning + bl.sub_ranges);
+    ba.point_list = (const uint32_t*)((char*)st->binning + bl.seg_list);
+    ba.rec0 = g.rec0; ba.rec1 = g.rec1;
     ba.base = has_sh ? g.rgb : in->colors_precomp;
     ba.extra = in->extra; ba.bg = in->bg;
-    ba.out_color = out->color; ba.out_depth = out->depth; ba.out_alpha = out->alpha;
-    ba.final_T = nullptr; ba.n_contrib = nullptr;
-    prof_begin(PF_BLEND_FWD, s);
-    rc = launch_blend_forward_subsets(ba, S, s);
-    prof_end(PF_BLEND_FWD, s);
+    ba.final_T = (const float*)((char*)st->image + il.final_T);
+    ba.n_contrib = (const uint32_t*)((char*)st->image + il.n_contrib);
+    ba.dL_dcolor = gin->dL_dcolor; ba.dL_ddepth = gin->dL_ddepth; ba.dL_dalpha = gin->dL_dalpha; ba.dL_dfeat = gin->dL_dfeat;
+    ba.geom = geom;
+    ba.acc = (float*)go->scratch;
+    ba.stride = blend_bwd_stride(C, geom);
+    prof_begin(PF_BLEND_BWD, s);
+    rc = launch_blend_backward_subsets(ba, S, s);
+    prof_end(PF_BLEND_BWD, s);
     if (rc) return rc;
-    OGS_KERNEL_CHECK("blend_forward_subsets", in->debug, s);
-    return 0;
+    OGS_KERNEL_CHECK("blend_backward_subsets", in->debug, s);
+    return preprocess_backward(in, g, go, ba.acc, ba.stride, geom, s);
 }
 
 int ogs_raster_cached_bytes(const ogs_raster_inputs* in, int64_t num_rendered, int64_t* geom_bytes, int64_t* binning_bytes) {
@@ -600,25 +719,7 @@ int ogs_raster_backward(const ogs_raster_inputs* in, const ogs_raster_state* st,
     prof_end(PF_BLEND_BWD, s);
     if (rc) return rc;
     OGS_KERNEL_CHECK("blend_backward", in->debug, s);
-
-    PreprocessBwdArgs pa;
-    pa.P = P; pa.D = in->sh_degree; pa.M = in->M; pa.C = C; pa.W = W; pa.H = H;
-    pa.act_flags = in->act_flags; pa.shs_rest = in->shs_rest; pa.extra = in->extra; pa.opacities = in->opacities;
-    pa.dL_dshs_rest = go->dL_dshs_rest; pa.accumulate = go->accumulate;
-    pa.means3D = in->means3D; pa.scales = in->scales; pa.rotations = in->rotations;
-    pa.cov3D_precomp = in->cov3D_precomp; pa.shs = in->shs;
-    pa.scale_modifier = in->scale_modifier; pa.tanfovx = in->tanfovx; pa.tanfovy = in->tanfovy;
-    pa.view = in->viewmatrix; pa.proj = in->projmatrix; pa.campos = in->campos;
-    pa.g = g; pa.acc = ba.acc; pa.stride = ba.stride; pa.geom = geom;
-    pa.dL_dmeans3D = go->dL_dmeans3D; pa.dL_dmeans2D = go->dL_dmeans2D; pa.dL_dopacities = go->dL_dopacities;
-    pa.dL_dshs = go->dL_dshs; pa.dL_dcolors_precomp = go->dL_dcolors_precomp; pa.dL_dscales = go->dL_dscales;
-    pa.dL_drotations = go->dL_drotations; pa.dL_dcov3D = go->dL_dcov3D; pa.dL_dextra = go->dL_dextra;
-    prof_begin(PF_PREPROCESS_BWD, s);
-    rc = launch_preprocess_backward(pa, s);
-    prof_end(PF_PREPROCESS_BWD, s);
-    if (rc) return rc;
-    OGS_KERNEL_CHECK("preprocess_backward", in->debug, s);
-    return 0;
+    return preprocess_backward(in, g, go, ba.acc, ba.stride, geom, s);
 }
 
 int ogs_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, uint8_t* present, void* stream_) {

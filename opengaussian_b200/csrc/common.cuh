@@ -185,7 +185,8 @@ struct BlendFwdArgs {
     float *out_color, *out_depth, *out_alpha, *final_T; uint32_t* n_contrib;
 };
 int launch_blend_forward(const BlendFwdArgs& a, cudaStream_t s);
-// S subsets: a.ranges = [S][tiles] segment bounds, outputs [S][C][H][W] / [S][H][W]; final_T, n_contrib unused
+// S subsets: a.ranges = [S][tiles] segment bounds, outputs [S][C][H][W] / [S][H][W]; final_T, n_contrib [S][H][W]
+// or both NULL
 int launch_blend_forward_subsets(const BlendFwdArgs& a, int S, cudaStream_t s);
 
 // subsets (subsets.cu): culled depth key for Gaussians outside [0, S); stable per-tile partition by subset
@@ -211,6 +212,9 @@ struct BlendBwdArgs {
 // preprocess_bwd turns them into dL_dmean2D / dL_dconic (linear in the moments, per-Gaussian factors).
 int blend_bwd_stride(int C, int geom);
 int launch_blend_backward(const BlendBwdArgs& a, cudaStream_t s);
+// S disjoint subsets (ogs_raster_backward_subsets): a.ranges = [S][tiles] segment bounds into a.point_list, final_T /
+// n_contrib / dL_ddepth / dL_dalpha [S][H][W], dL_dcolor [S][3 or C][H][W], dL_dfeat [S][C-3][H][W]
+int launch_blend_backward_subsets(const BlendBwdArgs& a, int S, cudaStream_t s);
 
 struct PreprocessBwdArgs {
     int P, D, M, C, W, H;

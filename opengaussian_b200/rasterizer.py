@@ -19,6 +19,7 @@ from typing import NamedTuple, Optional
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 
@@ -637,6 +638,112 @@ class _RasterizeGaussians(torch.autograd.Function):
         return g_means3D, g_means2D, g_sh, g_colors, g_opac, g_scales, g_rot, g_cov, g_extra, None, None, g_sh_rest, None
 
 
+def _subset_prepare(rs, means3D, opacities, subset, num_subsets, shs, colors_precomp, scales, rotations, cov3D_precomp,
+                    extra, extra_bg):
+    """The C-ABI arguments of a subset call: (S, int32 subset, F as given, F padded to a compiled width, the padded extra
+    channels, [bg | extra_bg | 0], settings with the camera as the C ABI needs it, inputs struct)."""
+    dev = means3D.device
+    P = means3D.shape[0]
+    S = int(num_subsets)
+    if tuple(subset.shape) != (P,):
+        raise _lib.OgsError(f"subset must have shape [{P}], got {tuple(subset.shape)}")
+    subset = subset.to(device=dev, dtype=torch.int32).contiguous()
+    n_extra_user = 0 if extra is None else int(extra.shape[1])
+    n_extra = n_extra_user
+    if n_extra_user:
+        c_tot = next((c for c in _SUPPORTED_C if c >= 3 + n_extra_user), None)
+        if c_tot is None:
+            raise _lib.OgsError(f"extra_feats: at most {_SUPPORTED_C[-1] - 3} channels are supported")
+        if c_tot != 3 + n_extra_user:   # pad with zero channels up to a compiled width
+            extra = torch.cat([extra, extra.new_zeros(P, c_tot - 3 - n_extra_user)], 1).contiguous()
+            n_extra = c_tot - 3
+    bg = _f32c(rs.bg).reshape(-1)
+    if n_extra:
+        eb = bg.new_zeros(0) if extra_bg is None else _f32c(extra_bg).reshape(-1).to(dev)
+        bg = torch.cat([bg, eb, bg.new_zeros(n_extra - eb.numel())])
+    _, cam = camera_inputs(rs.viewmatrix, rs.projmatrix, rs.campos)
+    rs = rs._replace(viewmatrix=cam[0], projmatrix=cam[1], campos=cam[2])
+    ri = _fill_inputs(rs, bg, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, n_extra)
+    ri.defer_capacity_check = 0
+    return S, subset, n_extra_user, n_extra, extra, bg, rs, ri
+
+
+def _subset_outputs(S, C, H, W, dev):
+    color_all = torch.empty(max(S, 0), C, H, W, dtype=torch.float32, device=dev)
+    depth = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
+    alpha = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
+    return color_all, depth, alpha, _lib.SubsetOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha))
+
+
+class _RasterizeSubsets(torch.autograd.Function):
+    """GaussianRasterizer.forward_subsets_grad: ogs_raster_forward_subsets_state, and ogs_raster_backward_subsets for
+    the gradients of every slot's colour, feature, depth and alpha images at once."""
+
+    @staticmethod
+    def forward(ctx, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, subset, S, rs,
+                extra_bg):
+        dev = means3D.device
+        means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra = (
+            _f32c(t) for t in (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra))
+        S, subset, n_extra_user, n_extra, extra, bg, rs, ri = _subset_prepare(
+            rs, means3D, opacities, subset, S, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, extra_bg)
+        H, W = int(rs.image_height), int(rs.image_width)
+        color_all, depth, alpha, so = _subset_outputs(S, 3 + n_extra, H, W, dev)
+        st = _lib.RasterState()
+        alloc = _Alloc(dev)
+        _lib.launch("ogs_raster_forward_subsets_state", dev, C.byref(ri), _lib.ptr(subset), S, C.byref(so), alloc.fn,
+                    alloc.user, C.byref(st))
+        ctx.set_materialize_grads(False)
+        ctx.rs, ctx.bg, ctx.state, ctx.bufs = rs, bg, st, alloc.bufs     # bufs: the state's geom/binning/image buffers
+        ctx.S, ctx.n_extra, ctx.n_extra_user = S, n_extra, n_extra_user
+        ctx.save_for_backward(means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra)
+        feat = color_all[:, 3:3 + n_extra_user] if n_extra_user else color_all.new_empty(max(S, 0), 0, H, W)
+        return color_all[:, :3], depth, alpha, feat
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_color, grad_depth, grad_alpha, grad_feat):
+        means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra = ctx.saved_tensors
+        rs, S, n_extra = ctx.rs, ctx.S, ctx.n_extra
+        dev = means3D.device
+        P = means3D.shape[0]
+        H, W = int(rs.image_height), int(rs.image_width)
+        need = ctx.needs_input_grad   # means3D, opacities, shs, colors_precomp, scales, rotations, cov3D, extra
+
+        # the padding rules of _RasterizeGaussians.backward, per slot
+        gc = _f32c(grad_color) if grad_color is not None else None
+        gf = None
+        if n_extra and grad_feat is not None and grad_feat.shape[1] > 0:
+            gf = _f32c(grad_feat)
+            if gf.shape[1] != n_extra:        # zero planes for the padding channels
+                gf = torch.cat([gf, gf.new_zeros(S, n_extra - gf.shape[1], H, W)], 1)
+        if n_extra and gf is None:
+            gf = torch.zeros(S, n_extra, H, W, dtype=torch.float32, device=dev)
+        if gc is None and gf is None:
+            gc = torch.zeros(S, 3, H, W, dtype=torch.float32, device=dev)
+        gd = _f32c(grad_depth) if grad_depth is not None else None
+        ga = _f32c(grad_alpha) if grad_alpha is not None else None
+
+        def out(flag, t, *shape):
+            return torch.empty(*(shape or t.shape), dtype=torch.float32, device=dev) if flag and t is not None else None
+
+        g_means3D, g_opac, g_sh = out(need[0], means3D), out(need[1], opacities), out(need[2], shs)
+        g_colors, g_scales, g_rot = out(need[3], colors_precomp), out(need[4], scales), out(need[5], rotations)
+        g_cov, g_extra = out(need[6], cov3D_precomp), out(need[7], extra)
+        scratch = torch.empty(_lib.lib().ogs_raster_backward_scratch_floats(P, n_extra), dtype=torch.float32,
+                              device=dev)
+        ri = _fill_inputs(rs, ctx.bg, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra,
+                          n_extra)
+        gi = _lib.RasterGradsIn(_lib.ptr(gc), _lib.ptr(gd), _lib.ptr(ga), _lib.ptr(gf))
+        go = _lib.RasterGradsOut(_lib.ptr(g_means3D), None, _lib.ptr(g_opac), _lib.ptr(g_sh), _lib.ptr(g_colors),
+                                 _lib.ptr(g_scales), _lib.ptr(g_rot), _lib.ptr(g_cov), _lib.ptr(g_extra), None,
+                                 _lib.ptr(scratch), 0, 0)
+        _lib.launch("ogs_raster_backward_subsets", dev, C.byref(ri), S, C.byref(ctx.state), C.byref(gi), C.byref(go))
+        if g_extra is not None and n_extra != ctx.n_extra_user:
+            g_extra = g_extra[:, :ctx.n_extra_user].contiguous()
+        return g_means3D, g_opac, g_sh, g_colors, g_scales, g_rot, g_cov, g_extra, None, None, None, None
+
+
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                         raster_settings, extra_feats=None, extra_bg=None, sh_rest=None, act_flags=0):
     return _RasterizeGaussians.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
@@ -695,14 +802,7 @@ class GaussianRasterizer(nn.Module):
             return color, radii, depth, alpha
         return color, radii, depth, alpha, feat
 
-    def forward_subsets(self, means3D, opacities, subset, num_subsets, shs=None, colors_precomp=None, scales=None,
-                        rotations=None, cov3D_precomp=None, extra_feats=None, extra_bg=None):
-        """Renders ``num_subsets`` disjoint subsets of the Gaussians in one call (C ABI ogs_raster_forward_subsets):
-        ``subset [P]`` holds each Gaussian's slot in ``[0, num_subsets)`` or -1 (not rendered).  Slot k's images equal,
-        bit for bit, ``forward()`` on the rows with ``subset == k``.  Activated inputs as for ``forward()``; forward
-        only (no backward, no radii) and outside the view cache.  Returns ``(color [S,3,H,W], depth [S,1,H,W],
-        alpha [S,1,H,W], feats [S,F,H,W] or None)``."""
-        rs = self.raster_settings
+    def _subset_check(self, shs, colors_precomp, scales, rotations, cov3D_precomp, means3D):
         if means3D.shape[0] > 0:
             shs, colors_precomp = _none_if_empty(shs), _none_if_empty(colors_precomp)
             scales, rotations, cov3D_precomp = _none_if_empty(scales), _none_if_empty(rotations), _none_if_empty(cov3D_precomp)
@@ -711,6 +811,18 @@ class GaussianRasterizer(nn.Module):
         if ((scales is None or rotations is None) and cov3D_precomp is None) or \
                 ((scales is not None or rotations is not None) and cov3D_precomp is not None):
             raise Exception('Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!')
+        return shs, colors_precomp, scales, rotations, cov3D_precomp
+
+    def forward_subsets(self, means3D, opacities, subset, num_subsets, shs=None, colors_precomp=None, scales=None,
+                        rotations=None, cov3D_precomp=None, extra_feats=None, extra_bg=None):
+        """Renders ``num_subsets`` disjoint subsets of the Gaussians in one call (C ABI ogs_raster_forward_subsets):
+        ``subset [P]`` holds each Gaussian's slot in ``[0, num_subsets)`` or -1 (not rendered).  Slot k's images equal,
+        bit for bit, ``forward()`` on the rows with ``subset == k``.  Activated inputs as for ``forward()``; forward
+        only (no backward, no radii: ``forward_subsets_grad`` is the differentiable form) and outside the view cache.
+        Returns ``(color [S,3,H,W], depth [S,1,H,W], alpha [S,1,H,W], feats [S,F,H,W] or None)``."""
+        rs = self.raster_settings
+        shs, colors_precomp, scales, rotations, cov3D_precomp = self._subset_check(
+            shs, colors_precomp, scales, rotations, cov3D_precomp, means3D)
         inputs = (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra_feats)
         if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs):
             raise _lib.OgsError("forward_subsets has no backward: call it under torch.no_grad() or with inputs that "
@@ -719,37 +831,31 @@ class GaussianRasterizer(nn.Module):
         if dev.type != "cuda":
             raise _lib.OgsError("GaussianRasterizer needs CUDA tensors (there is no CPU fallback)")
         means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra = (_f32c(t) for t in inputs)
-        P = means3D.shape[0]
-        S = int(num_subsets)
-        if tuple(subset.shape) != (P,):
-            raise _lib.OgsError(f"subset must have shape [{P}], got {tuple(subset.shape)}")
-        subset = subset.to(device=dev, dtype=torch.int32).contiguous()
+        S, subset, n_extra_user, n_extra, extra, bg, rs, ri = _subset_prepare(
+            rs, means3D, opacities, subset, num_subsets, shs, colors_precomp, scales, rotations, cov3D_precomp, extra,
+            extra_bg)
         H, W = int(rs.image_height), int(rs.image_width)
-        n_extra_user = 0 if extra is None else int(extra.shape[1])
-        n_extra = n_extra_user
-        if n_extra_user:
-            c_tot = next((c for c in _SUPPORTED_C if c >= 3 + n_extra_user), None)
-            if c_tot is None:
-                raise _lib.OgsError(f"extra_feats: at most {_SUPPORTED_C[-1] - 3} channels are supported")
-            if c_tot != 3 + n_extra_user:   # pad with zero channels up to a compiled width
-                extra = torch.cat([extra, extra.new_zeros(P, c_tot - 3 - n_extra_user)], 1).contiguous()
-                n_extra = c_tot - 3
-        bg = _f32c(rs.bg).reshape(-1)
-        if n_extra:
-            eb = bg.new_zeros(0) if extra_bg is None else _f32c(extra_bg).reshape(-1).to(dev)
-            bg = torch.cat([bg, eb, bg.new_zeros(n_extra - eb.numel())])
-        _, cam = camera_inputs(rs.viewmatrix, rs.projmatrix, rs.campos)
-        rs = rs._replace(viewmatrix=cam[0], projmatrix=cam[1], campos=cam[2])
-
-        color_all = torch.empty(max(S, 0), 3 + n_extra, H, W, dtype=torch.float32, device=dev)
-        depth = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
-        alpha = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
-        ri = _fill_inputs(rs, bg, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra,
-                          n_extra)
-        ri.defer_capacity_check = 0
+        color_all, depth, alpha, so = _subset_outputs(S, 3 + n_extra, H, W, dev)
         alloc = _Alloc(dev)
-        so = _lib.SubsetOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha))
         _lib.launch("ogs_raster_forward_subsets", dev, C.byref(ri), _lib.ptr(subset), S, C.byref(so), alloc.fn,
                     alloc.user)
         feats = color_all[:, 3:3 + n_extra_user] if n_extra_user else None
         return color_all[:, :3], depth, alpha, feats
+
+    def forward_subsets_grad(self, means3D, opacities, subset, num_subsets, shs=None, colors_precomp=None, scales=None,
+                             rotations=None, cov3D_precomp=None, extra_feats=None, extra_bg=None):
+        """``forward_subsets`` with a backward (C ABI ogs_raster_forward_subsets_state / ogs_raster_backward_subsets):
+        the same arguments, checks and bit-identical images, returned as autograd outputs.  Gradients of every slot's
+        colour, features, depth and alpha flow to ``means3D, opacities, shs, colors_precomp, scales, rotations,
+        cov3D_precomp, extra_feats`` in one backward; each Gaussian's gradient is that of its own slot's images (those
+        of no slot get zero), as ``forward()`` + backward on each slot's rows would give.  There is no ``means2D``
+        input, hence no screen-space gradient: a caller that needs one renders each slot with ``forward()``.  Plain
+        gradient tensors (no gradient arena, no fused accumulation), outside the view cache; no double backward."""
+        shs, colors_precomp, scales, rotations, cov3D_precomp = self._subset_check(
+            shs, colors_precomp, scales, rotations, cov3D_precomp, means3D)
+        if means3D.device.type != "cuda":
+            raise _lib.OgsError("GaussianRasterizer needs CUDA tensors (there is no CPU fallback)")
+        color, depth, alpha, feats = _RasterizeSubsets.apply(means3D, opacities, shs, colors_precomp, scales, rotations,
+                                                             cov3D_precomp, extra_feats, subset, num_subsets,
+                                                             self.raster_settings, extra_bg)
+        return color, depth, alpha, (feats if feats.shape[1] > 0 else None)

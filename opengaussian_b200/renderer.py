@@ -17,7 +17,7 @@ The feature channels get the same background as the reference gives them (bg_col
 each 3-channel group, because the reference reuses one rasterizer for all passes).  The CPU RNG
 draws (`torch.rand(1)` at :121,124) are reproduced so that training stays in lock-step.
 ``fused=False`` falls back to the reference's literal pass structure (used by the parity test).
-Cluster / leaf passes that need no gradient: all subsets of the call in ONE rasterizer call (_render_slots).
+Cluster / leaf passes: all subsets of the call in ONE rasterizer call (_render_slots), with or without a gradient.
 """
 import math
 
@@ -102,10 +102,13 @@ def _feat_pass(rasterizer, bg3, means3D, means2D, opacity, scales, rotations, co
 # The planners decide, in the reference's loop order, which clusters / leaves reach the rasterizer and with which rows;
 # their filters are disjoint, so they are handed on as ONE int32 slot map `subset` ([P]: slot k or -1, the filter of
 # slot k is subset == k).  The render step then runs either one rasterizer call for all slots
-# (GaussianRasterizer.forward_subsets: no-grad passes) or the reference's one pass per slot (passes whose outputs need
-# a gradient, and fused=False).
+# (GaussianRasterizer.forward_subsets, or forward_subsets_grad when a gradient must reach the inputs) or the reference's
+# one pass per slot (_subset_route says when).
 
-SUBSET_BATCH_BYTES = 4 << 30    # output bytes of one forward_subsets call, S * (C + 2) * H * W * 4; more slots are split
+# Output bytes of one subset call, S * ((C + 2) * 4 [+ 8 state bytes with grad]) * H * W; more slots are split.  This
+# bounds what a call returns and keeps for its backward, not peak memory: the backward of a gradient-carrying call also
+# receives upstream gradient images of the same size as the outputs the loss reads (plus zero planes for padding).
+SUBSET_BATCH_BYTES = 4 << 30
 
 
 def _slot_map(ids, base, slots):
@@ -193,22 +196,43 @@ def _plan_leaves(leaf_cluster_idx, lerf_range, selected_leaf_id, pre_mask, viewe
     return [cand[k] for k in kept], subset
 
 
-def _use_batched(fused, *inputs):
-    """One forward_subsets call for all slots unless a gradient must reach an input (it has no backward) or the caller
-    asked for the reference's literal passes (fused=False)."""
-    return fused and not (torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs))
+def _needs_grad(*inputs):
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs)
+
+
+def _subset_route(fused, batched, needs_grad, means2D_grad):
+    """How _render_slots renders its slots: "batched" (one forward_subsets call, no gradient), "batched_grad" (one
+    forward_subsets_grad call) or "loop" (the reference's one rasterizer pass per slot).  The loop stays for fused=False
+    (the reference's literal passes), for pipe.batched_subsets = False (batched=False), and when the screen-space points
+    need a gradient (trainable geometry: the loop feeds viewspace_points.grad, a subset call has no means2D input).
+    A single slot (the Stage 2.2 root pass) is batched too: the call preprocesses every Gaussian where the loop gathers
+    the slot's rows, but the loop's filter, count read and gather cost more (2.83 -> 2.47 ms per step on a B200 at
+    1 M Gaussians, DESIGN.md section 8 item 8)."""
+    if not (fused and batched):
+        return "loop"
+    if not needs_grad:
+        return "batched"
+    return "loop" if means2D_grad else "batched_grad"
+
+
+def _use_batched(fused, batched, means2D, *inputs):
+    """One subset call for all slots (forward_subsets, or forward_subsets_grad when an input needs a gradient) unless
+    _subset_route keeps the loop."""
+    return _subset_route(fused, batched, _needs_grad(*inputs), means2D.requires_grad) != "loop"
 
 
 def _render_slots(rasterizer, bg3, ids, subset, means3D, means2D, opacity, scales, rotations, cov3D_precomp, feat, shs,
-                  fused, keep_min_alpha=None):
+                  fused, keep_min_alpha=None, batched=True):
     """The images of the planned slots -> (images, silhouettes), lists in slot order, each entry as _feat_pass returns it.
     keep_min_alpha: keep only the slots whose silhouette exceeds it somewhere (the coarse loop's test, :222), and
-    remove the others from `ids` in place."""
+    remove the others from `ids` in place.  batched=False: the loop (pipe.batched_subsets)."""
     imgs, sils = [], []
-    if _use_batched(fused, means3D, opacity, scales, rotations, cov3D_precomp, feat, shs):
+    inputs = (means3D, opacity, scales, rotations, cov3D_precomp, feat, shs)
+    if _use_batched(fused, batched, means2D, *inputs):
+        grad = _needs_grad(*inputs)
         keep_ids = []
         for a, b, img, sil in _render_slots_batched(rasterizer, bg3, len(ids), subset, means3D, opacity, scales,
-                                                    rotations, cov3D_precomp, feat, shs):
+                                                    rotations, cov3D_precomp, feat, shs, grad):
             if keep_min_alpha is not None:
                 keep = (sil.amax(dim=(1, 2, 3)) > keep_min_alpha).tolist()       # one host read per launch
                 sel = [k for k in range(b - a) if keep[k]]
@@ -240,9 +264,11 @@ def _render_slots(rasterizer, bg3, ids, subset, means3D, means2D, opacity, scale
     return imgs, sils
 
 
-def _render_slots_batched(rasterizer, bg3, S, subset, means3D, opacity, scales, rotations, cov3D_precomp, feat, shs):
-    """forward_subsets over slots [a, b) per launch, each launch's outputs within SUBSET_BATCH_BYTES: yields
-    (a, b, images [b-a,F,H,W], silhouettes [b-a,1,H,W]) with the channel layout of _feat_pass."""
+def _render_slots_batched(rasterizer, bg3, S, subset, means3D, opacity, scales, rotations, cov3D_precomp, feat, shs,
+                          grad=False):
+    """forward_subsets (grad: forward_subsets_grad) over slots [a, b) per launch, each launch's outputs and state within
+    SUBSET_BATCH_BYTES: yields (a, b, images [b-a,F,H,W], silhouettes [b-a,1,H,W]) with the channel layout of
+    _feat_pass."""
     rs = rasterizer.raster_settings
     H, W = int(rs.image_height), int(rs.image_width)
     if shs is not None:
@@ -252,12 +278,13 @@ def _render_slots_batched(rasterizer, bg3, S, subset, means3D, opacity, scales, 
         kw = dict(colors_precomp=feat[:, :3], extra_feats=feat[:, 3:], extra_bg=torch.cat([bg3] * ((nb + 2) // 3))[:nb])
     else:
         nb, kw = 0, dict(colors_precomp=feat)
-    per_launch = max(1, SUBSET_BATCH_BYTES // ((3 + nb + 2) * H * W * 4))
+    per_launch = max(1, SUBSET_BATCH_BYTES // (((3 + nb + 2) * 4 + (8 if grad else 0)) * H * W))
+    call = rasterizer.forward_subsets_grad if grad else rasterizer.forward_subsets
     for a in range(0, S, per_launch):
         b = min(S, a + per_launch)
         sub = subset if (a == 0 and b == S) else torch.where((subset >= a) & (subset < b), subset - a, -1)
-        color, _, alpha, extra = rasterizer.forward_subsets(means3D, opacity, sub, b - a, scales=scales,
-                                                            rotations=rotations, cov3D_precomp=cov3D_precomp, **kw)
+        color, _, alpha, extra = call(means3D, opacity, sub, b - a, scales=scales, rotations=rotations,
+                                      cov3D_precomp=cov3D_precomp, **kw)
         if shs is not None:
             img = torch.cat((color, color), dim=1)
         elif extra is not None:
@@ -285,7 +312,9 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
            root_num=64, leaf_num=10,
            fused=True):
     """Render the scene.  Background tensor (bg_color) must be on GPU!
-    ``pipe.view_cache = False`` keeps this call out of the frozen-geometry view cache (rasterizer.ViewCache)."""
+    ``pipe.view_cache = False`` keeps this call out of the frozen-geometry view cache (rasterizer.ViewCache).
+    ``pipe.batched_subsets = False`` renders the cluster / leaf passes one rasterizer pass per subset, as the reference
+    does, instead of one subset call per pass (same images; the gradients differ only in the order of float additions)."""
     if getattr(pipe, "view_cache", True) is False and _view_cache.enabled:
         with _view_cache.disabled():
             return render(viewpoint_camera, pc, pipe, bg_color, iteration, scaling_modifier, override_color, visible_mask,
@@ -370,6 +399,7 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
     rendered_image = radii = rendered_depth = rendered_alpha = None
     rendered_ins_feat = silhouette = None
     bg3 = bg_color.reshape(-1).float()
+    batched = getattr(pipe, "batched_subsets", True)
     if use_raw:
         q = getattr(pc, "_ins_feat_q", None)
         raw_feat = pc._ins_feat if (origin_feat or q is None or len(q) == 0) else q
@@ -425,7 +455,7 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
                                      selected_root_id, viewpoint_camera.bClusterOccur)
         rendered_clusters, rendered_cluster_silhouettes = _render_slots(
             rasterizer, bg3, ids, subset, means3D, means2D, opacity, sc(scales), rotations, cov3D_precomp, ins_feat,
-            None, fused, keep_min_alpha=0.8)
+            None, fused, keep_min_alpha=0.8, batched=batched)
         for idx in ids:
             cluster_occur[idx] = True
         if len(rendered_cluster_silhouettes) != 0:
@@ -453,7 +483,7 @@ def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,
                                                pre_mask, viewed_pts, scale_filter, better_vis, post_process, means3D)
         rendered_leaf_clusters, rendered_leaf_cluster_silhouettes = _render_slots(
             rasterizer, bg3, occured_leaf_id, subset, means3D, means2D, opacity, scales, rotations, cov3D_precomp,
-            ins_feat, shs if seg_rgb else None, fused)
+            ins_feat, shs if seg_rgb else None, fused, batched=batched)
         if len(rendered_leaf_cluster_silhouettes) != 0:
             rendered_leaf_cluster_silhouettes = torch.vstack(rendered_leaf_cluster_silhouettes)
     else:
