@@ -184,6 +184,124 @@ static ImgLayout subset_img_layout(int W, int H, int S) {
     return l;
 }
 
+// The sizes of a frame and the layouts of its geometry and image buffers, derived once from the inputs.  S > 0: a
+// subset pass, whose image buffer holds every subset's planes.
+struct Frame {
+    int P, W, H, C, tiles;
+    bool has_sh;
+    int n_feat_act;        // activated extra channels kept with the geometry (raw-parameter mode), else 0
+    GeomLayout gl;
+    ImgLayout il;
+    static Frame of(const ogs_raster_inputs* in, int S = 0) {
+        Frame f;
+        f.P = in->P; f.W = in->W; f.H = in->H; f.C = 3 + in->n_extra;
+        f.tiles = ((f.W + 15) / 16) * ((f.H + 15) / 16);
+        f.has_sh = in->shs != nullptr;
+        f.n_feat_act = (in->act_flags & OGS_ACT_EXTRA_UNIT_HALF) ? in->n_extra : 0;
+        f.gl = GeomLayout::make(f.P, f.has_sh, f.n_feat_act);
+        f.il = S > 0 ? subset_img_layout(f.W, f.H, S) : ImgLayout::make(f.W, f.H);
+        return f;
+    }
+};
+
+// The scan total read back as [N, overflow flag].
+static int read_count(const uint32_t* h, int64_t& N) {
+    if (h[1]) { set_error("more than 2^32 - 1 (Gaussian, tile) duplicates in one frame: 32-bit offsets overflow"); return -7; }
+    N = (int64_t)h[0];
+    return 0;
+}
+
+// The first half of a forward: preprocess (with `subset`: then the culled depth key for the Gaussians of no subset),
+// the depth sort and the scan, whose total [N, overflow flag] ends up at sc.offsets + P.  The depth-sort scratch is
+// carved from `scratch`, which must live until the tile lists are built (sc.nvis_ptr points into it).  radii NULL:
+// one more scratch array takes them.
+static int preprocess_and_sort(const ogs_raster_inputs* in, const GeomPtrs& g, int32_t* radii, const int32_t* subset,
+                               int S, AsyncScratch& scratch, BinScratch& sc, cudaStream_t s) {
+    const int P = in->P;
+    const size_t pw = align_up((size_t)(P + 2) * 4, 256);      // offsets carries two extra words: N and the overflow flag
+    const int words = radii ? 5 : 6;
+    sc.cub_temp_bytes = align_up(depth_sort_temp_bytes(P), 256);
+    OGS_CUDA(scratch.alloc(pw * words + sc.cub_temp_bytes));
+    char* s1 = (char*)scratch.p;
+    sc.dkeys_in = (uint32_t*)(s1);
+    sc.dvals_in = (uint32_t*)(s1 + pw);
+    sc.dkeys_out = (uint32_t*)(s1 + 2 * pw);
+    sc.dvals_out = (uint32_t*)(s1 + 3 * pw);
+    sc.offsets = (uint32_t*)(s1 + 4 * pw);
+    if (!radii) radii = (int32_t*)(s1 + 5 * pw);
+    sc.cub_temp = s1 + words * pw;
+
+    PreprocessArgs pa;
+    pa.P = P; pa.D = in->sh_degree; pa.M = in->M; pa.W = in->W; pa.H = in->H;
+    pa.act_flags = in->act_flags; pa.n_extra = in->n_extra; pa.shs_rest = in->shs_rest; pa.extra = in->extra;
+    pa.means3D = in->means3D; pa.scales = in->scales; pa.rotations = in->rotations;
+    pa.cov3D_precomp = in->cov3D_precomp; pa.opacities = in->opacities; pa.shs = in->shs;
+    pa.scale_modifier = in->scale_modifier; pa.tanfovx = in->tanfovx; pa.tanfovy = in->tanfovy;
+    pa.view = in->viewmatrix; pa.proj = in->projmatrix; pa.campos = in->campos;
+    pa.radii = radii; pa.g = g; pa.depth_keys = sc.dkeys_in; pa.depth_vals = sc.dvals_in;
+    prof_begin(PF_PREPROCESS_FWD, s);
+    int rc = launch_preprocess_forward(pa, s);
+    if (!rc && subset) rc = launch_subset_exclude(P, S, subset, sc.dkeys_in, s);     // rows of no slot: the culled key
+    prof_end(PF_PREPROCESS_FWD, s);
+    if (rc) return rc;
+    OGS_KERNEL_CHECK(subset ? "preprocess_forward (subsets)" : "preprocess_forward", in->debug, s);
+    prof_begin(PF_DEPTH_SORT_SCAN, s);
+    rc = depth_sort_and_scan(P, g, sc, s, in->debug);
+    prof_end(PF_DEPTH_SORT_SCAN, s);
+    return rc;
+}
+
+// The per-tile lists of the first `cap` (Gaussian, tile) duplicates: emit, sort by tile, tile ranges.  n_ptr: the device
+// count N.
+static int build_tile_lists(const Frame& f, const uint32_t* n_ptr, int64_t cap, const GeomPtrs& g, BinScratch& sc,
+                            uint32_t* point_list, uint2* ranges, cudaStream_t s, int debug) {
+    AsyncScratch scratch(s);
+    const size_t k2 = align_up((size_t)cap * 2, 256), v4 = align_up((size_t)cap * 4, 256);
+    const size_t tb = align_up(tile_sort_temp_bytes(cap), 256);
+    OGS_CUDA(scratch.alloc(2 * k2 + v4 + tb));
+    char* s2 = (char*)scratch.p;
+    sc.cub_temp = s2 + 2 * k2 + v4;
+    sc.cub_temp_bytes = tb;
+    return emit_sort_ranges(f.P, f.W, f.H, n_ptr, cap, g, sc, (uint16_t*)s2, (uint32_t*)(s2 + 2 * k2),
+                            (uint16_t*)(s2 + k2), point_list, ranges, s, debug);
+}
+
+// feat: the activated extra channels, blended instead of in->extra in raw-parameter mode.  image NULL: no final_T /
+// n_contrib are kept.
+static BlendFwdArgs blend_fwd_args(const Frame& f, const ogs_raster_inputs* in, const GeomPtrs& g, const float* feat,
+                                   const uint2* ranges, const uint32_t* point_list, float* color, float* depth,
+                                   float* alpha, void* image) {
+    BlendFwdArgs ba;
+    ba.W = f.W; ba.H = f.H; ba.C = f.C;
+    ba.ranges = ranges; ba.point_list = point_list; ba.rec0 = g.rec0; ba.rec1 = g.rec1;
+    ba.base = f.has_sh ? g.rgb : in->colors_precomp;
+    ba.extra = f.n_feat_act ? feat : in->extra; ba.bg = in->bg;
+    ba.out_color = color; ba.out_depth = depth; ba.out_alpha = alpha;
+    ba.final_T = image ? (float*)((char*)image + f.il.final_T) : nullptr;
+    ba.n_contrib = image ? (uint32_t*)((char*)image + f.il.n_contrib) : nullptr;
+    return ba;
+}
+
+// feat as for blend_fwd_args.  ba.geom: whether any geometry gradient is wanted (else the colour / feature-only form).
+static BlendBwdArgs blend_bwd_args(const Frame& f, const ogs_raster_inputs* in, const GeomPtrs& g, const float* feat,
+                                   const uint2* ranges, const uint32_t* point_list, const void* image,
+                                   const ogs_raster_grads_in* gin, const ogs_raster_grads_out* go) {
+    BlendBwdArgs ba;
+    ba.P = f.P; ba.W = f.W; ba.H = f.H; ba.C = f.C;
+    ba.ranges = ranges; ba.point_list = point_list;
+    ba.rec0 = g.rec0; ba.rec1 = g.rec1;
+    ba.base = f.has_sh ? g.rgb : in->colors_precomp;
+    ba.extra = f.n_feat_act ? feat : in->extra; ba.bg = in->bg;
+    ba.final_T = (const float*)((const char*)image + f.il.final_T);
+    ba.n_contrib = (const uint32_t*)((const char*)image + f.il.n_contrib);
+    ba.dL_dcolor = gin->dL_dcolor; ba.dL_ddepth = gin->dL_ddepth; ba.dL_dalpha = gin->dL_dalpha; ba.dL_dfeat = gin->dL_dfeat;
+    ba.geom = (go->dL_dmeans3D || go->dL_dmeans2D || go->dL_dopacities || go->dL_dshs || go->dL_dshs_rest ||
+               go->dL_dscales || go->dL_drotations || go->dL_dcov3D) ? 1 : 0;
+    ba.acc = (float*)go->scratch;
+    ba.stride = blend_bwd_stride(f.C, ba.geom);
+    return ba;
+}
+
 // The parameter gradients from the blend's per-Gaussian accumulators (shared by the frame and subset backwards).
 static int preprocess_backward(const ogs_raster_inputs* in, const GeomPtrs& g, const ogs_raster_grads_out* go,
                                float* acc, int stride, int geom, cudaStream_t s) {
@@ -216,17 +334,13 @@ static int forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, i
     if (in->act_flags != 0) { set_error("forward_subsets: needs activated inputs (act_flags == 0)"); return -1; }
     if (!out || !out->color || !out->alpha || !alloc) { set_error("forward_subsets: outputs/alloc must be set"); return -1; }
     if ((rc = ensure_pool())) return rc;
-    const int P = in->P, W = in->W, H = in->H, C = 3 + in->n_extra;
-    const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
-    const bool has_sh = in->shs != nullptr;
-    const GeomLayout gl = GeomLayout::make(P, has_sh, 0);
-    void* geom = alloc(alloc_user, gl.total, "geom");
+    const Frame f = Frame::of(in, S);
+    void* geom = alloc(alloc_user, f.gl.total, "geom");
     if (!geom) { set_error("allocation callback returned NULL"); return -6; }
-    const GeomPtrs g = GeomPtrs::from(geom, gl);
-    const ImgLayout il = subset_img_layout(W, H, S);
+    const GeomPtrs g = GeomPtrs::from(geom, f.gl);
     void* image = nullptr;
     if (st) {
-        image = alloc(alloc_user, il.total, "image");
+        image = alloc(alloc_user, f.il.total, "image");
         if (!image) { set_error("allocation callback returned NULL"); return -6; }
     }
 
@@ -234,47 +348,17 @@ static int forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, i
     AsyncScratch scratch1(s);
     BinScratch sc;
     memset(&sc, 0, sizeof sc);
-    if (P > 0) {
-        const size_t pw = align_up((size_t)(P + 2) * 4, 256);
-        sc.cub_temp_bytes = align_up(depth_sort_temp_bytes(P), 256);
-        OGS_CUDA(scratch1.alloc(pw * 6 + sc.cub_temp_bytes));
-        char* s1 = (char*)scratch1.p;
-        sc.dkeys_in = (uint32_t*)(s1);
-        sc.dvals_in = (uint32_t*)(s1 + pw);
-        sc.dkeys_out = (uint32_t*)(s1 + 2 * pw);
-        sc.dvals_out = (uint32_t*)(s1 + 3 * pw);
-        sc.offsets = (uint32_t*)(s1 + 4 * pw);
-        int32_t* radii = (int32_t*)(s1 + 5 * pw);
-        sc.cub_temp = s1 + 6 * pw;
-
-        PreprocessArgs pa;
-        pa.P = P; pa.D = in->sh_degree; pa.M = in->M; pa.W = W; pa.H = H;
-        pa.act_flags = 0; pa.n_extra = in->n_extra; pa.shs_rest = in->shs_rest; pa.extra = in->extra;
-        pa.means3D = in->means3D; pa.scales = in->scales; pa.rotations = in->rotations;
-        pa.cov3D_precomp = in->cov3D_precomp; pa.opacities = in->opacities; pa.shs = in->shs;
-        pa.scale_modifier = in->scale_modifier; pa.tanfovx = in->tanfovx; pa.tanfovy = in->tanfovy;
-        pa.view = in->viewmatrix; pa.proj = in->projmatrix; pa.campos = in->campos;
-        pa.radii = radii; pa.g = g; pa.depth_keys = sc.dkeys_in; pa.depth_vals = sc.dvals_in;
-        prof_begin(PF_PREPROCESS_FWD, s);
-        rc = launch_preprocess_forward(pa, s);
-        if (!rc) rc = launch_subset_exclude(P, S, subset, sc.dkeys_in, s);     // rows of no slot: the culled key
-        prof_end(PF_PREPROCESS_FWD, s);
-        if (rc) return rc;
-        OGS_KERNEL_CHECK("preprocess_forward (subsets)", in->debug, s);
-        prof_begin(PF_DEPTH_SORT_SCAN, s);
-        rc = depth_sort_and_scan(P, g, sc, s, in->debug);
-        prof_end(PF_DEPTH_SORT_SCAN, s);
-        if (rc) return rc;
+    if (f.P > 0) {
+        if ((rc = preprocess_and_sort(in, g, nullptr, subset, S, scratch1, sc, s))) return rc;
         uint32_t* h = pinned_scalar(forward_ctx());     // the synchronous-check words: free between calls of this thread
         if (!h) { set_error("cudaMallocHost failed"); return 2; }
-        OGS_CUDA(cudaMemcpyAsync(h, sc.offsets + P, 8, cudaMemcpyDeviceToHost, s));
+        OGS_CUDA(cudaMemcpyAsync(h, sc.offsets + f.P, 8, cudaMemcpyDeviceToHost, s));
         OGS_CUDA(cudaStreamSynchronize(s));
-        if (h[1]) { set_error("more than 2^32 - 1 (Gaussian, tile) duplicates in one frame: 32-bit offsets overflow"); return -7; }
-        N = (int64_t)h[0];
+        if ((rc = read_count(h, N))) return rc;
     }
 
     // binning: the frame's lists and ranges, then the partitioned lists and the [S][tiles] segment bounds
-    const SubsetBinLayout bl = SubsetBinLayout::make(N, tiles, S);
+    const SubsetBinLayout bl = SubsetBinLayout::make(N, f.tiles, S);
     char* binning = (char*)alloc(alloc_user, bl.total, "binning");
     if (!binning) { set_error("allocation callback returned NULL"); return -6; }
     uint32_t* point_list = (uint32_t*)(binning + bl.frame.point_list);
@@ -282,33 +366,18 @@ static int forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, i
     uint32_t* seg_list = (uint32_t*)(binning + bl.seg_list);
     uint2* sub_ranges = (uint2*)(binning + bl.sub_ranges);
     if (N > 0) {
-        AsyncScratch scratch2(s);
-        const size_t k2 = align_up((size_t)N * 2, 256), v4 = align_up((size_t)N * 4, 256);
-        const size_t tb = align_up(tile_sort_temp_bytes(N), 256);
-        OGS_CUDA(scratch2.alloc(2 * k2 + v4 + tb));
-        char* s2 = (char*)scratch2.p;
-        sc.cub_temp = s2 + 2 * k2 + v4;
-        sc.cub_temp_bytes = tb;
-        rc = emit_sort_ranges(P, W, H, sc.offsets + P, N, g, sc, (uint16_t*)s2, (uint32_t*)(s2 + 2 * k2),
-                              (uint16_t*)(s2 + k2), point_list, ranges, s, in->debug);
-        if (rc) return rc;
+        if ((rc = build_tile_lists(f, sc.offsets + f.P, N, g, sc, point_list, ranges, s, in->debug))) return rc;
         prof_begin(PF_RANGES, s);
-        rc = launch_subset_partition(tiles, S, ranges, point_list, subset, seg_list, sub_ranges, s);
+        rc = launch_subset_partition(f.tiles, S, ranges, point_list, subset, seg_list, sub_ranges, s);
         prof_end(PF_RANGES, s);
         if (rc) return rc;
         OGS_KERNEL_CHECK("subset_partition", in->debug, s);
     } else {
-        OGS_CUDA(cudaMemsetAsync(sub_ranges, 0, (size_t)S * tiles * sizeof(uint2), s));
+        OGS_CUDA(cudaMemsetAsync(sub_ranges, 0, (size_t)S * f.tiles * sizeof(uint2), s));
     }
 
-    BlendFwdArgs ba;
-    ba.W = W; ba.H = H; ba.C = C;
-    ba.ranges = sub_ranges; ba.point_list = seg_list; ba.rec0 = g.rec0; ba.rec1 = g.rec1;
-    ba.base = has_sh ? g.rgb : in->colors_precomp;
-    ba.extra = in->extra; ba.bg = in->bg;
-    ba.out_color = out->color; ba.out_depth = out->depth; ba.out_alpha = out->alpha;
-    ba.final_T = image ? (float*)((char*)image + il.final_T) : nullptr;
-    ba.n_contrib = image ? (uint32_t*)((char*)image + il.n_contrib) : nullptr;
+    const BlendFwdArgs ba = blend_fwd_args(f, in, g, nullptr, sub_ranges, seg_list, out->color, out->depth, out->alpha,
+                                           image);
     prof_begin(PF_BLEND_FWD, s);
     rc = launch_blend_forward_subsets(ba, S, s);
     prof_end(PF_BLEND_FWD, s);
@@ -318,7 +387,7 @@ static int forward_subsets(const ogs_raster_inputs* in, const int32_t* subset, i
         memset(st, 0, sizeof *st);
         st->geom = geom; st->binning = binning; st->image = image;
         st->num_rendered = N;
-        st->geom_bytes = (int64_t)gl.total; st->binning_bytes = (int64_t)bl.total; st->image_bytes = (int64_t)il.total;
+        st->geom_bytes = (int64_t)f.gl.total; st->binning_bytes = (int64_t)bl.total; st->image_bytes = (int64_t)f.il.total;
     }
     return 0;
 }
@@ -379,22 +448,14 @@ int ogs_raster_forward(const ogs_raster_inputs* in, const ogs_raster_outputs* ou
     }
     cudaStream_t s = (cudaStream_t)stream_;
     if ((rc = ensure_pool())) return rc;
-    const int P = in->P, W = in->W, H = in->H, C = 3 + in->n_extra;
-    const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
-    const bool has_sh = in->shs != nullptr;
-
-    const int n_feat_act = (in->act_flags & OGS_ACT_EXTRA_UNIT_HALF) ? in->n_extra : 0;
-    const GeomLayout gl = GeomLayout::make(P, has_sh, n_feat_act);
-    const ImgLayout il = ImgLayout::make(W, H);
+    const Frame f = Frame::of(in);
     memset(st, 0, sizeof *st);
-    st->geom = alloc(alloc_user, gl.total, "geom");
-    st->image = alloc(alloc_user, il.total, "image");
-    st->geom_bytes = (int64_t)gl.total;
-    st->image_bytes = (int64_t)il.total;
+    st->geom = alloc(alloc_user, f.gl.total, "geom");
+    st->image = alloc(alloc_user, f.il.total, "image");
+    st->geom_bytes = (int64_t)f.gl.total;
+    st->image_bytes = (int64_t)f.il.total;
     if (!st->geom || !st->image) { set_error("allocation callback returned NULL"); return -6; }
-    const GeomPtrs g = GeomPtrs::from(st->geom, gl);
-    float* final_T = (float*)((char*)st->image + il.final_T);
-    uint32_t* n_contrib = (uint32_t*)((char*)st->image + il.n_contrib);
+    const GeomPtrs g = GeomPtrs::from(st->geom, f.gl);
 
     int64_t N = 0, cap = 0;
     bool speculative = false;
@@ -406,35 +467,8 @@ int ogs_raster_forward(const ogs_raster_inputs* in, const ogs_raster_outputs* ou
     AsyncScratch scratch1(s);          // freed (stream-ordered) on every exit path
     BinScratch sc;
     memset(&sc, 0, sizeof sc);
-    if (P > 0) {
-        const size_t pw = align_up((size_t)(P + 2) * 4, 256);      // offsets carries two extra words: N and the overflow flag
-        sc.cub_temp_bytes = align_up(depth_sort_temp_bytes(P), 256);
-        OGS_CUDA(scratch1.alloc(pw * 5 + sc.cub_temp_bytes));
-        char* s1 = (char*)scratch1.p;
-        sc.dkeys_in = (uint32_t*)(s1);
-        sc.dvals_in = (uint32_t*)(s1 + pw);
-        sc.dkeys_out = (uint32_t*)(s1 + 2 * pw);
-        sc.dvals_out = (uint32_t*)(s1 + 3 * pw);
-        sc.offsets = (uint32_t*)(s1 + 4 * pw);
-        sc.cub_temp = s1 + 5 * pw;
-
-        PreprocessArgs pa;
-        pa.P = P; pa.D = in->sh_degree; pa.M = in->M; pa.W = W; pa.H = H;
-        pa.act_flags = in->act_flags; pa.n_extra = in->n_extra; pa.shs_rest = in->shs_rest; pa.extra = in->extra;
-        pa.means3D = in->means3D; pa.scales = in->scales; pa.rotations = in->rotations;
-        pa.cov3D_precomp = in->cov3D_precomp; pa.opacities = in->opacities; pa.shs = in->shs;
-        pa.scale_modifier = in->scale_modifier; pa.tanfovx = in->tanfovx; pa.tanfovy = in->tanfovy;
-        pa.view = in->viewmatrix; pa.proj = in->projmatrix; pa.campos = in->campos;
-        pa.radii = out->radii; pa.g = g; pa.depth_keys = sc.dkeys_in; pa.depth_vals = sc.dvals_in;
-        prof_begin(PF_PREPROCESS_FWD, s);
-        rc = launch_preprocess_forward(pa, s);
-        prof_end(PF_PREPROCESS_FWD, s);
-        if (rc) return rc;
-        OGS_KERNEL_CHECK("preprocess_forward", in->debug, s);
-        prof_begin(PF_DEPTH_SORT_SCAN, s);
-        rc = depth_sort_and_scan(P, g, sc, s, in->debug);
-        prof_end(PF_DEPTH_SORT_SCAN, s);
-        if (rc) return rc;
+    if (f.P > 0) {
+        if ((rc = preprocess_and_sort(in, g, out->radii, nullptr, 0, scratch1, sc, s))) return rc;
         h = pinned_scalar(fc);
         if (!h) { set_error("cudaMallocHost failed"); return 2; }
         if (in->defer_capacity_check && fc.cap_hint != 0 && !in->debug) {
@@ -442,7 +476,7 @@ int ogs_raster_forward(const ogs_raster_inputs* in, const ogs_raster_outputs* ou
                 if (!fc.pending[k].live) deferred = &fc.pending[k];
             if (deferred) h += 2 * (1 + (deferred - fc.pending));
         }
-        n_ptr = sc.offsets + P;
+        n_ptr = sc.offsets + f.P;
         OGS_CUDA(cudaMemcpyAsync(h, n_ptr, 8, cudaMemcpyDeviceToHost, s));     // [N, overflow flag]
         // Capacity speculation: the binning buffers are sized from the running estimate cap_hint and
         // the N-dependent kernels take N from device memory, so emit/sort/blend are queued WITHOUT
@@ -450,8 +484,7 @@ int ogs_raster_forward(const ogs_raster_inputs* in, const ogs_raster_outputs* ou
         // finished by then).  If the estimate was too small the binning + blend are redone (rare).
         if (fc.cap_hint == 0 || in->debug) {
             OGS_CUDA(cudaStreamSynchronize(s));
-            if (h[1]) { set_error("more than 2^32 - 1 (Gaussian, tile) duplicates in one frame: 32-bit offsets overflow"); return -7; }
-            N = (int64_t)*h;
+            if ((rc = read_count(h, N))) return rc;
             cap = N;
         } else if (deferred) {
             if (!deferred->ev) OGS_CUDA(cudaEventCreateWithFlags(&deferred->ev, cudaEventDisableTiming));
@@ -471,35 +504,22 @@ int ogs_raster_forward(const ogs_raster_inputs* in, const ogs_raster_outputs* ou
     uint32_t* point_list = nullptr;
     uint2* ranges = nullptr;
     for (;;) {
-        const BinLayout bl = BinLayout::make(cap, tiles);
+        const BinLayout bl = BinLayout::make(cap, f.tiles);
         st->binning = alloc(alloc_user, bl.total, "binning");
         st->binning_bytes = (int64_t)bl.total;
         if (!st->binning) { set_error("allocation callback returned NULL"); return -6; }
         point_list = (uint32_t*)((char*)st->binning + bl.point_list);
         ranges = (uint2*)((char*)st->binning + bl.ranges);
-        if (cap > 0 && P > 0) {
-            AsyncScratch scratch2(s);
-            const size_t k2 = align_up((size_t)cap * 2, 256), v4 = align_up((size_t)cap * 4, 256);
-            const size_t tb = align_up(tile_sort_temp_bytes(cap), 256);
-            OGS_CUDA(scratch2.alloc(2 * k2 + v4 + tb));
-            char* s2 = (char*)scratch2.p;
-            sc.cub_temp = s2 + 2 * k2 + v4;
-            sc.cub_temp_bytes = tb;
-            rc = emit_sort_ranges(P, W, H, n_ptr, cap, g, sc, (uint16_t*)s2, (uint32_t*)(s2 + 2 * k2),
-                                  (uint16_t*)(s2 + k2), point_list, ranges, s, in->debug);
+        if (cap > 0 && f.P > 0) {
+            rc = build_tile_lists(f, n_ptr, cap, g, sc, point_list, ranges, s, in->debug);
         } else {
-            cudaError_t e = cudaMemsetAsync(ranges, 0, (size_t)tiles * sizeof(uint2), s);
+            cudaError_t e = cudaMemsetAsync(ranges, 0, (size_t)f.tiles * sizeof(uint2), s);
             if (e != cudaSuccess) rc = cuda_fail(e, "memset ranges");
         }
         if (rc) return rc;
 
-        BlendFwdArgs ba;
-        ba.W = W; ba.H = H; ba.C = C;
-        ba.ranges = ranges; ba.point_list = point_list; ba.rec0 = g.rec0; ba.rec1 = g.rec1;
-        ba.base = has_sh ? g.rgb : in->colors_precomp;
-        ba.extra = n_feat_act ? g.feat : in->extra; ba.bg = in->bg;
-        ba.out_color = out->color; ba.out_depth = out->depth; ba.out_alpha = out->alpha;
-        ba.final_T = final_T; ba.n_contrib = n_contrib;
+        const BlendFwdArgs ba = blend_fwd_args(f, in, g, g.feat, ranges, point_list, out->color, out->depth,
+                                               out->alpha, st->image);
         prof_begin(PF_BLEND_FWD, s);
         rc = launch_blend_forward(ba, s);
         prof_end(PF_BLEND_FWD, s);
@@ -511,14 +531,13 @@ int ogs_raster_forward(const ogs_raster_inputs* in, const ogs_raster_outputs* ou
             break;
         }
         OGS_CUDA(cudaEventSynchronize(n_event));
-        if (h[1]) { set_error("more than 2^32 - 1 (Gaussian, tile) duplicates in one frame: 32-bit offsets overflow"); return -7; }
-        N = (int64_t)*h;
+        if ((rc = read_count(h, N))) return rc;
         speculative = false;
         if (N <= cap) break;
         cap = N;                       // estimate too small: redo binning + blend with the exact size
     }
     scratch1.release();
-    if (P > 0 && N >= 0) fc.grow_hint(N);
+    if (f.P > 0 && N >= 0) fc.grow_hint(N);
     st->num_rendered = N;
     return 0;
 }
@@ -545,50 +564,33 @@ int ogs_raster_backward_subsets(const ogs_raster_inputs* in, int32_t S, const og
     if (gin->dL_dfeat && in->n_extra <= 0) { set_error("dL_dfeat needs n_extra > 0"); return -1; }
     if (go->accumulate) { set_error("backward_subsets: accumulate is not supported"); return -1; }
     if (go->dL_dshs_rest && !go->dL_dshs) { set_error("dL_dshs_rest needs dL_dshs"); return -1; }
-    const int P = in->P, W = in->W, H = in->H, C = 3 + in->n_extra;
-    const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
-    const bool has_sh = in->shs != nullptr;
-    const GeomLayout gl = GeomLayout::make(P, has_sh, 0);
-    const ImgLayout il = subset_img_layout(W, H, S);
-    if (!st->geom || !st->binning || !st->image || st->num_rendered < 0 || st->geom_bytes != (int64_t)gl.total ||
-        st->image_bytes != (int64_t)il.total ||
-        st->binning_bytes != (int64_t)SubsetBinLayout::make(st->num_rendered, tiles, S).total) {
+    const Frame f = Frame::of(in, S);
+    if (!st->geom || !st->binning || !st->image || st->num_rendered < 0 || st->geom_bytes != (int64_t)f.gl.total ||
+        st->image_bytes != (int64_t)f.il.total ||
+        st->binning_bytes != (int64_t)SubsetBinLayout::make(st->num_rendered, f.tiles, S).total) {
         set_error("backward_subsets: state does not belong to a forward_subsets_state of these sizes (P=%d, S=%d, %dx%d)",
-                  P, S, W, H);
+                  f.P, S, f.W, f.H);
         return -1;
     }
-    if (P == 0) return 0;
+    if (f.P == 0) return 0;
     cudaStream_t s = (cudaStream_t)stream_;
-    const SubsetBinLayout bl = SubsetBinLayout::make(st->num_rendered, tiles, S);
-    const GeomPtrs g = GeomPtrs::from(st->geom, gl);
-    const int geom = (go->dL_dmeans3D || go->dL_dmeans2D || go->dL_dopacities || go->dL_dshs || go->dL_dshs_rest ||
-                      go->dL_dscales || go->dL_drotations || go->dL_dcov3D) ? 1 : 0;
-    BlendBwdArgs ba;
-    ba.P = P; ba.W = W; ba.H = H; ba.C = C;
-    ba.ranges = (const uint2*)((char*)st->binning + bl.sub_ranges);
-    ba.point_list = (const uint32_t*)((char*)st->binning + bl.seg_list);
-    ba.rec0 = g.rec0; ba.rec1 = g.rec1;
-    ba.base = has_sh ? g.rgb : in->colors_precomp;
-    ba.extra = in->extra; ba.bg = in->bg;
-    ba.final_T = (const float*)((char*)st->image + il.final_T);
-    ba.n_contrib = (const uint32_t*)((char*)st->image + il.n_contrib);
-    ba.dL_dcolor = gin->dL_dcolor; ba.dL_ddepth = gin->dL_ddepth; ba.dL_dalpha = gin->dL_dalpha; ba.dL_dfeat = gin->dL_dfeat;
-    ba.geom = geom;
-    ba.acc = (float*)go->scratch;
-    ba.stride = blend_bwd_stride(C, geom);
+    const SubsetBinLayout bl = SubsetBinLayout::make(st->num_rendered, f.tiles, S);
+    const GeomPtrs g = GeomPtrs::from(st->geom, f.gl);
+    const BlendBwdArgs ba = blend_bwd_args(f, in, g, nullptr, (const uint2*)((char*)st->binning + bl.sub_ranges),
+                                           (const uint32_t*)((char*)st->binning + bl.seg_list), st->image, gin, go);
     prof_begin(PF_BLEND_BWD, s);
     rc = launch_blend_backward_subsets(ba, S, s);
     prof_end(PF_BLEND_BWD, s);
     if (rc) return rc;
     OGS_KERNEL_CHECK("blend_backward_subsets", in->debug, s);
-    return preprocess_backward(in, g, go, ba.acc, ba.stride, geom, s);
+    return preprocess_backward(in, g, go, ba.acc, ba.stride, ba.geom, s);
 }
 
 int ogs_raster_cached_bytes(const ogs_raster_inputs* in, int64_t num_rendered, int64_t* geom_bytes, int64_t* binning_bytes) {
     if (!in || num_rendered < 0 || in->P < 0 || in->W <= 0 || in->H <= 0) { set_error("cached_bytes: bad arguments"); return -1; }
-    const int tiles = ((in->W + 15) / 16) * ((in->H + 15) / 16);
-    if (geom_bytes) *geom_bytes = (int64_t)GeomLayout::make(in->P, in->shs != nullptr, 0).total;
-    if (binning_bytes) *binning_bytes = (int64_t)BinLayout::make(num_rendered, tiles).total;
+    const Frame f = Frame::of(in);
+    if (geom_bytes) *geom_bytes = (int64_t)GeomLayout::make(f.P, f.has_sh, 0).total;
+    if (binning_bytes) *binning_bytes = (int64_t)BinLayout::make(num_rendered, f.tiles).total;
     return 0;
 }
 
@@ -601,49 +603,38 @@ int ogs_raster_forward_cached(const ogs_raster_inputs* in, const ogs_raster_outp
         return -1;
     }
     cudaStream_t s = (cudaStream_t)stream_;
-    const int P = in->P, W = in->W, H = in->H, C = 3 + in->n_extra;
-    const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
-    const bool has_sh = in->shs != nullptr;
-    const int n_feat_act = (in->act_flags & OGS_ACT_EXTRA_UNIT_HALF) ? in->n_extra : 0;
+    const Frame f = Frame::of(in);
     // the activated channels sit last in the geometry layout: every other offset is the same with and without them
-    const GeomLayout gl = GeomLayout::make(P, has_sh, 0);
-    const ImgLayout il = ImgLayout::make(W, H);
-    if (!cached->geom || !cached->binning || cached->num_rendered < 0 || cached->geom_bytes < (int64_t)gl.total ||
-        cached->binning_bytes < (int64_t)BinLayout::make(cached->num_rendered, tiles).total) {
-        set_error("cached state does not belong to a finished forward of these sizes (P=%d, %d tiles, N=%lld)", P, tiles,
-                  (long long)cached->num_rendered);
+    if (!cached->geom || !cached->binning || cached->num_rendered < 0 ||
+        cached->geom_bytes < (int64_t)GeomLayout::make(f.P, f.has_sh, 0).total ||
+        cached->binning_bytes < (int64_t)BinLayout::make(cached->num_rendered, f.tiles).total) {
+        set_error("cached state does not belong to a finished forward of these sizes (P=%d, %d tiles, N=%lld)", f.P,
+                  f.tiles, (long long)cached->num_rendered);
         return -1;
     }
     *st = *cached;
-    st->image = alloc(alloc_user, il.total, "image");
-    st->image_bytes = (int64_t)il.total;
+    st->image = alloc(alloc_user, f.il.total, "image");
+    st->image_bytes = (int64_t)f.il.total;
     st->feat = nullptr;
     if (!st->image) { set_error("allocation callback returned NULL"); return -6; }
-    const GeomPtrs g = GeomPtrs::from(st->geom, gl);
-    const BinLayout bl = BinLayout::make(st->num_rendered, tiles);
-    if (n_feat_act && P > 0) {
-        st->feat = alloc(alloc_user, (size_t)P * n_feat_act * sizeof(float), "feat");
+    const GeomPtrs g = GeomPtrs::from(st->geom, f.gl);
+    const BinLayout bl = BinLayout::make(st->num_rendered, f.tiles);
+    if (f.n_feat_act && f.P > 0) {
+        st->feat = alloc(alloc_user, (size_t)f.P * f.n_feat_act * sizeof(float), "feat");
         if (!st->feat) { set_error("allocation callback returned NULL"); return -6; }
         prof_begin(PF_PREPROCESS_FWD, s);
-        rc = launch_feat_refresh(P, n_feat_act, g.rec1, in->extra, (float*)st->feat, s);
+        rc = launch_feat_refresh(f.P, f.n_feat_act, g.rec1, in->extra, (float*)st->feat, s);
         prof_end(PF_PREPROCESS_FWD, s);
         if (rc) return rc;
         OGS_KERNEL_CHECK("feat_refresh", in->debug, s);
     }
-    if (out->radii && P > 0) {          // radius = rec1.w as int bits; culled Gaussians hold 0 there
-        cudaError_t e = cudaMemcpy2DAsync(out->radii, 4, &g.rec1[0].w, 16, 4, (size_t)P, cudaMemcpyDeviceToDevice, s);
+    if (out->radii && f.P > 0) {        // radius = rec1.w as int bits; culled Gaussians hold 0 there
+        cudaError_t e = cudaMemcpy2DAsync(out->radii, 4, &g.rec1[0].w, 16, 4, (size_t)f.P, cudaMemcpyDeviceToDevice, s);
         if (e != cudaSuccess) return cuda_fail(e, "radii copy");
     }
-    BlendFwdArgs ba;
-    ba.W = W; ba.H = H; ba.C = C;
-    ba.ranges = (uint2*)((char*)st->binning + bl.ranges);
-    ba.point_list = (uint32_t*)((char*)st->binning + bl.point_list);
-    ba.rec0 = g.rec0; ba.rec1 = g.rec1;
-    ba.base = has_sh ? g.rgb : in->colors_precomp;
-    ba.extra = n_feat_act ? (const float*)st->feat : in->extra; ba.bg = in->bg;
-    ba.out_color = out->color; ba.out_depth = out->depth; ba.out_alpha = out->alpha;
-    ba.final_T = (float*)((char*)st->image + il.final_T);
-    ba.n_contrib = (uint32_t*)((char*)st->image + il.n_contrib);
+    const BlendFwdArgs ba = blend_fwd_args(f, in, g, (const float*)st->feat, (uint2*)((char*)st->binning + bl.ranges),
+                                           (uint32_t*)((char*)st->binning + bl.point_list), out->color, out->depth,
+                                           out->alpha, st->image);
     prof_begin(PF_BLEND_FWD, s);
     rc = launch_blend_forward(ba, s);
     prof_end(PF_BLEND_FWD, s);
@@ -668,13 +659,9 @@ int ogs_raster_capacity_check(void) {
         pf.live = false;
         cudaError_t e = cudaEventSynchronize(pf.ev);
         if (e != cudaSuccess) { result = cuda_fail(e, "capacity check"); continue; }
-        const uint32_t* h = fc.pinned + 2 * (1 + k);
-        if (h[1]) {
-            set_error("more than 2^32 - 1 (Gaussian, tile) duplicates in one frame: 32-bit offsets overflow");
-            result = -7;
-            continue;
-        }
-        const int64_t N = (int64_t)h[0];
+        int64_t N = 0;
+        const int rc = read_count(fc.pinned + 2 * (1 + k), N);
+        if (rc) { result = rc; continue; }
         fc.grow_hint(N);
         if (N > pf.cap && result == 0) result = 1;
     }
@@ -688,38 +675,21 @@ int ogs_raster_backward(const ogs_raster_inputs* in, const ogs_raster_state* st,
     if (!st || !gin || !go || (!gin->dL_dcolor && !gin->dL_dfeat) || !go->scratch) { set_error("state/grads/scratch must be set"); return -1; }
     if (gin->dL_dfeat && in->n_extra <= 0) { set_error("dL_dfeat needs n_extra > 0"); return -1; }
     cudaStream_t s = (cudaStream_t)stream_;
-    const int P = in->P, W = in->W, H = in->H, C = 3 + in->n_extra;
-    if (P == 0) return 0;
-    const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
-    const bool has_sh = in->shs != nullptr;
-    const int n_feat_act = (in->act_flags & OGS_ACT_EXTRA_UNIT_HALF) ? in->n_extra : 0;
-    const GeomLayout gl = GeomLayout::make(P, has_sh, n_feat_act);
-    const ImgLayout il = ImgLayout::make(W, H);
-    const BinLayout bl = BinLayout::make(st->num_rendered, tiles);
-    const GeomPtrs g = GeomPtrs::from(st->geom, gl);
+    const Frame f = Frame::of(in);
+    if (f.P == 0) return 0;
+    const BinLayout bl = BinLayout::make(st->num_rendered, f.tiles);
+    const GeomPtrs g = GeomPtrs::from(st->geom, f.gl);
 
-    const int geom = (go->dL_dmeans3D || go->dL_dmeans2D || go->dL_dopacities || go->dL_dshs || go->dL_dshs_rest ||
-                      go->dL_dscales || go->dL_drotations || go->dL_dcov3D) ? 1 : 0;
     if (go->dL_dshs_rest && !go->dL_dshs) { set_error("dL_dshs_rest needs dL_dshs"); return -1; }
-    BlendBwdArgs ba;
-    ba.P = P; ba.W = W; ba.H = H; ba.C = C;
-    ba.ranges = (const uint2*)((char*)st->binning + bl.ranges);
-    ba.point_list = (const uint32_t*)((char*)st->binning + bl.point_list);
-    ba.rec0 = g.rec0; ba.rec1 = g.rec1;
-    ba.base = has_sh ? g.rgb : in->colors_precomp;
-    ba.extra = n_feat_act ? (st->feat ? (const float*)st->feat : g.feat) : in->extra; ba.bg = in->bg;
-    ba.final_T = (const float*)((char*)st->image + il.final_T);
-    ba.n_contrib = (const uint32_t*)((char*)st->image + il.n_contrib);
-    ba.dL_dcolor = gin->dL_dcolor; ba.dL_ddepth = gin->dL_ddepth; ba.dL_dalpha = gin->dL_dalpha; ba.dL_dfeat = gin->dL_dfeat;
-    ba.geom = geom;
-    ba.acc = (float*)go->scratch;
-    ba.stride = blend_bwd_stride(C, geom);
+    const BlendBwdArgs ba = blend_bwd_args(f, in, g, st->feat ? (const float*)st->feat : g.feat,
+                                           (const uint2*)((char*)st->binning + bl.ranges),
+                                           (const uint32_t*)((char*)st->binning + bl.point_list), st->image, gin, go);
     prof_begin(PF_BLEND_BWD, s);
     rc = launch_blend_backward(ba, s);
     prof_end(PF_BLEND_BWD, s);
     if (rc) return rc;
     OGS_KERNEL_CHECK("blend_backward", in->debug, s);
-    return preprocess_backward(in, g, go, ba.acc, ba.stride, geom, s);
+    return preprocess_backward(in, g, go, ba.acc, ba.stride, ba.geom, s);
 }
 
 int ogs_mark_visible(int32_t P, const float* means3D, const float* viewmatrix, uint8_t* present, void* stream_) {
@@ -736,23 +706,20 @@ int ogs_raster_export(const ogs_raster_inputs* in, const ogs_raster_state* st, u
                       uint32_t* tiles_touched, float* final_T, uint32_t* n_contrib, void* stream_) {
     if (!in || !st) { set_error("export: NULL inputs/state"); return -1; }
     cudaStream_t s = (cudaStream_t)stream_;
-    const int P = in->P, W = in->W, H = in->H;
-    const int gx = (W + 15) / 16, gy = (H + 15) / 16, tiles = gx * gy;
-    const bool has_sh = in->shs != nullptr;
-    const GeomLayout gl = GeomLayout::make(P, has_sh, (in->act_flags & OGS_ACT_EXTRA_UNIT_HALF) ? in->n_extra : 0);
-    const ImgLayout il = ImgLayout::make(W, H);
-    const BinLayout bl = BinLayout::make(st->num_rendered, tiles);
-    const GeomPtrs g = GeomPtrs::from(st->geom, gl);
+    const Frame f = Frame::of(in);
+    const BinLayout bl = BinLayout::make(st->num_rendered, f.tiles);
+    const GeomPtrs g = GeomPtrs::from(st->geom, f.gl);
     const uint32_t* pl = (const uint32_t*)((char*)st->binning + bl.point_list);
     const uint2* rg = (const uint2*)((char*)st->binning + bl.ranges);
     const int64_t N = st->num_rendered;
-    if (keys && N > 0) export_keys_kernel<<<tiles, 128, 0, s>>>(tiles, rg, pl, g.rec1, keys);
+    const size_t plane = (size_t)f.W * f.H * 4;
+    if (keys && N > 0) export_keys_kernel<<<f.tiles, 128, 0, s>>>(f.tiles, rg, pl, g.rec1, keys);
     if (point_list && N > 0) OGS_CUDA(cudaMemcpyAsync(point_list, pl, (size_t)N * 4, cudaMemcpyDeviceToDevice, s));
-    if (ranges) OGS_CUDA(cudaMemcpyAsync(ranges, rg, (size_t)tiles * 8, cudaMemcpyDeviceToDevice, s));
-    if (P > 0 && (xy || depth || conic_opacity || rgb || tiles_touched))
-        export_geom_kernel<<<(P + 255) / 256, 256, 0, s>>>(P, g, has_sh, xy, depth, conic_opacity, rgb, tiles_touched);
-    if (final_T) OGS_CUDA(cudaMemcpyAsync(final_T, (char*)st->image + il.final_T, (size_t)W * H * 4, cudaMemcpyDeviceToDevice, s));
-    if (n_contrib) OGS_CUDA(cudaMemcpyAsync(n_contrib, (char*)st->image + il.n_contrib, (size_t)W * H * 4, cudaMemcpyDeviceToDevice, s));
+    if (ranges) OGS_CUDA(cudaMemcpyAsync(ranges, rg, (size_t)f.tiles * 8, cudaMemcpyDeviceToDevice, s));
+    if (f.P > 0 && (xy || depth || conic_opacity || rgb || tiles_touched))
+        export_geom_kernel<<<(f.P + 255) / 256, 256, 0, s>>>(f.P, g, f.has_sh, xy, depth, conic_opacity, rgb, tiles_touched);
+    if (final_T) OGS_CUDA(cudaMemcpyAsync(final_T, (char*)st->image + f.il.final_T, plane, cudaMemcpyDeviceToDevice, s));
+    if (n_contrib) OGS_CUDA(cudaMemcpyAsync(n_contrib, (char*)st->image + f.il.n_contrib, plane, cudaMemcpyDeviceToDevice, s));
     OGS_KERNEL_CHECK("export", 0, s);
     return 0;
 }

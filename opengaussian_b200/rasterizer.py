@@ -263,7 +263,7 @@ class _CacheSwitch:
 
 
 view_cache = ViewCache()
-_BG_FULL = {}         # device index -> (signature, [bg | extra_bg | 0] tensor, bg, extra_bg) of the last forward with extra channels
+_BG_FULL = {}         # (device index, n_extra) -> (signature, [bg | extra_bg | 0] tensor, bg, extra_bg) of the last such forward
 _CAPTURE_PINS = {}    # device index -> list that receives the cache buffers a CUDA-graph capture reads (graphs.GraphedViewStep)
 
 
@@ -384,69 +384,121 @@ def _fusable_grad(t, shape):
             and tuple(g.shape) == tuple(shape))
 
 
+def _check_inputs(means3D, shs, colors_precomp, scales, rotations, cov3D_precomp):
+    """Upstream's argument rules (and messages) -> (shs, colors_precomp, scales, rotations, cov3D_precomp), an empty
+    tensor standing for "not given" as upstream passes them."""
+    if means3D.shape[0] > 0:
+        shs, colors_precomp = _none_if_empty(shs), _none_if_empty(colors_precomp)
+        scales, rotations, cov3D_precomp = _none_if_empty(scales), _none_if_empty(rotations), _none_if_empty(cov3D_precomp)
+    if (shs is None and colors_precomp is None) or (shs is not None and colors_precomp is not None):
+        raise Exception('Please provide excatly one of either SHs or precomputed colors!')
+    if ((scales is None or rotations is None) and cov3D_precomp is None) or \
+            ((scales is not None or rotations is not None) and cov3D_precomp is not None):
+        raise Exception('Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!')
+    return shs, colors_precomp, scales, rotations, cov3D_precomp
+
+
+def _pad_extra(extra, act_flags=0):
+    """The extra channels padded with zero channels up to a compiled width (3 + F in _SUPPORTED_C) -> (extra, F padded).
+    Raw channels (ACT_EXTRA_UNIT_HALF) are normalised as a whole, so they cannot be padded."""
+    n = 0 if extra is None else int(extra.shape[1])
+    if not n:
+        return extra, 0
+    c_tot = next((c for c in _SUPPORTED_C if c >= 3 + n), None)
+    if c_tot is None:
+        raise _lib.OgsError(f"extra_feats: at most {_SUPPORTED_C[-1] - 3} channels are supported")
+    if c_tot == 3 + n:
+        return extra, n
+    if act_flags & _lib.ACT_EXTRA_UNIT_HALF:
+        raise _lib.OgsError(f"raw extra_feats need 3 + F in {_SUPPORTED_C} (got F = {n})")
+    return torch.cat([extra, extra.new_zeros(extra.shape[0], c_tot - 3 - n)], 1).contiguous(), c_tot - 3
+
+
+def _bg_full(bg, extra_bg, n_extra):
+    """The background of all 3 + n_extra channels, [bg | extra_bg | 0...] (extra_bg None: zeros); with extra channels
+    cached per device and width, rebuilt only when bg or extra_bg changes (storage, version counter)."""
+    bg = _f32c(bg).reshape(-1)
+    if n_extra == 0:
+        return bg
+    dev = bg.device
+    sig = (_sig(bg), _sig(extra_bg))
+    hit = _BG_FULL.get((dev.index, n_extra))
+    if hit is None or hit[0] != sig:
+        if extra_bg is None:
+            full = torch.cat([bg, bg.new_zeros(n_extra)])
+        else:
+            eb = _f32c(extra_bg).reshape(-1).to(dev)
+            full = torch.cat([bg, eb, bg.new_zeros(n_extra - eb.numel())])
+        hit = (sig, full, bg, extra_bg)            # the sources stay alive, so their addresses stay theirs
+        _BG_FULL[(dev.index, n_extra)] = hit
+    pin_for_capture(dev, hit[1])
+    return hit[1]
+
+
+def _prepare(rs, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, extra_bg,
+             sh_rest=None, act_flags=0):
+    """The C-ABI arguments of a forward -> (inputs, F as given, F padded, background, camera key, camera, settings,
+    inputs struct).  inputs: (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra,
+    sh_rest) as contiguous float32, extra padded (_pad_extra); camera: camera_inputs(), which the settings now hold."""
+    if means3D.device.type != "cuda":
+        raise _lib.OgsError("GaussianRasterizer needs CUDA tensors (there is no CPU fallback)")
+    means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, sh_rest = (
+        _f32c(t) for t in (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, sh_rest))
+    if sh_rest is not None and shs is None:
+        raise _lib.OgsError("shs_rest needs shs (= _features_dc)")
+    n_extra_user = 0 if extra is None else int(extra.shape[1])
+    extra, n_extra = _pad_extra(extra, act_flags)
+    bg = _bg_full(rs.bg, extra_bg, n_extra)
+    cam_key, cam = camera_inputs(rs.viewmatrix, rs.projmatrix, rs.campos)
+    rs = rs._replace(viewmatrix=cam[0], projmatrix=cam[1], campos=cam[2])
+    ri = _fill_inputs(rs, bg, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, n_extra,
+                      sh_rest, act_flags)
+    inputs = (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, sh_rest)
+    return inputs, n_extra_user, n_extra, bg, cam_key, cam, rs, ri
+
+
+def _grad_planes(grad_color, grad_feat, n_extra, shape, dev):
+    """The image gradients of a backward for the C ABI -> (dL_dcolor, dL_dfeat), channels at dim -3 of images of
+    `shape` without its channels ([H,W] or [S,H,W]).  With extra channels the feature gradient is always passed, with
+    zero planes for the channels padded up to a compiled width or absent from the loss; with neither gradient, zero
+    colour planes."""
+    def planes(c):
+        return (*shape[:-2], c, *shape[-2:])
+
+    gc = _f32c(grad_color)
+    gf = None
+    if n_extra and grad_feat is not None and grad_feat.shape[-3] > 0:
+        gf = _f32c(grad_feat)
+        if gf.shape[-3] != n_extra:
+            gf = torch.cat([gf, gf.new_zeros(planes(n_extra - gf.shape[-3]))], -3)
+    if n_extra and gf is None:
+        gf = torch.zeros(planes(n_extra), dtype=torch.float32, device=dev)
+    if gc is None and gf is None:
+        gc = torch.zeros(planes(3), dtype=torch.float32, device=dev)
+    return gc, gf
+
+
 class _RasterizeGaussians(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, extra,
                 raster_settings, extra_bg=None, sh_rest=None, act_flags=0):
         L = _lib.lib()
-        rs = raster_settings
-        dev = means3D.device
         means2D_in = means2D
-        if dev.type != "cuda":
-            raise _lib.OgsError("GaussianRasterizer needs CUDA tensors (there is no CPU fallback)")
-        means3D = _f32c(means3D)
-        sh = _f32c(sh)
-        colors_precomp = _f32c(colors_precomp)
-        opacities = _f32c(opacities)
-        scales = _f32c(scales)
-        rotations = _f32c(rotations)
-        cov3Ds_precomp = _f32c(cov3Ds_precomp)
-        extra = _f32c(extra)
-        sh_rest = _f32c(sh_rest)
         act_flags = int(act_flags)
-        if sh_rest is not None and sh is None:
-            raise _lib.OgsError("shs_rest needs shs (= _features_dc)")
+        (means3D, opacities, sh, colors_precomp, scales, rotations, cov3Ds_precomp, extra, sh_rest), n_extra_user, \
+            n_extra, bg_full, cam_sig, cam, rs, ri = _prepare(
+                raster_settings, means3D, opacities, sh, colors_precomp, scales, rotations, cov3Ds_precomp, extra,
+                extra_bg, sh_rest, act_flags)
+        cam_src = (raster_settings.viewmatrix, raster_settings.projmatrix, raster_settings.campos)
+        dev = means3D.device
         P = means3D.shape[0]
         H, W = int(rs.image_height), int(rs.image_width)
-        n_extra_user = 0 if extra is None else int(extra.shape[1])
-        n_extra = n_extra_user
-        if n_extra_user:
-            c_tot = next((c for c in _SUPPORTED_C if c >= 3 + n_extra_user), None)
-            if c_tot is None:
-                raise _lib.OgsError(f"extra_feats: at most {_SUPPORTED_C[-1] - 3} channels are supported")
-            if c_tot != 3 + n_extra_user and (act_flags & _lib.ACT_EXTRA_UNIT_HALF):
-                raise _lib.OgsError(f"raw extra_feats need 3 + F in {_SUPPORTED_C} (got F = {n_extra_user})")
-            if c_tot != 3 + n_extra_user:   # pad with zero channels up to a compiled width
-                extra = torch.cat([extra, extra.new_zeros(P, c_tot - 3 - n_extra_user)], 1).contiguous()
-                n_extra = c_tot - 3
-        bg = _f32c(rs.bg).reshape(-1)
-        if n_extra == 0:
-            bg_full = bg
-        else:
-            # [bg | extra_bg | 0...]: rebuilt only when one of the two tensors changes (storage, version counter)
-            sig = (_sig(bg), _sig(extra_bg), n_extra)
-            hit = _BG_FULL.get(dev.index)
-            if hit is None or hit[0] != sig:
-                if extra_bg is None:
-                    full = torch.cat([bg, bg.new_zeros(n_extra)])
-                else:
-                    eb = _f32c(extra_bg).reshape(-1).to(dev)
-                    full = torch.cat([bg, eb, bg.new_zeros(n_extra - eb.numel())])
-                hit = (sig, full, bg, extra_bg)            # the sources stay alive, so their addresses stay theirs
-                _BG_FULL[dev.index] = hit
-            bg_full = hit[1]
-            pin_for_capture(dev, bg_full)
-        cam_src = (rs.viewmatrix, rs.projmatrix, rs.campos)
-        cam_sig, cam = camera_inputs(*cam_src)
-        rs = rs._replace(viewmatrix=cam[0], projmatrix=cam[1], campos=cam[2])
 
         color_all = torch.empty(3 + n_extra, H, W, dtype=torch.float32, device=dev)
         depth = torch.empty(1, H, W, dtype=torch.float32, device=dev)
         alpha = torch.empty(1, H, W, dtype=torch.float32, device=dev)
         radii = torch.empty(P, dtype=torch.int32, device=dev)
 
-        ri = _fill_inputs(rs, bg_full, means3D, opacities, sh, colors_precomp, scales, rotations, cov3Ds_precomp,
-                          extra, n_extra, sh_rest, act_flags)
         st = _lib.RasterState()
         alloc = _Alloc(dev)
         # Frozen geometry (OpenGaussian stages 1-3, train.py:431-436): reuse the camera's records and tile lists
@@ -526,18 +578,8 @@ class _RasterizeGaussians(torch.autograd.Function):
         H, W = int(rs.image_height), int(rs.image_width)
         need = ctx.needs_input_grad   # means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3D, extra
 
-        gc = _f32c(grad_color) if grad_color is not None else None
-        gf = None
-        if n_extra and grad_feat is not None and grad_feat.shape[0] > 0:
-            gf = _f32c(grad_feat)
-            if gf.shape[0] != n_extra:        # zero planes for the padding channels
-                gf = torch.cat([gf, gf.new_zeros(n_extra - gf.shape[0], H, W)], 0)
-        if n_extra and gf is None:            # features rendered but not in the loss: the split form needs their planes
-            gf = torch.zeros(n_extra, H, W, dtype=torch.float32, device=dev)
-        if gc is None and gf is None:
-            gc = torch.zeros(3, H, W, dtype=torch.float32, device=dev)
-        gd = _f32c(grad_depth) if grad_depth is not None else None
-        ga = _f32c(grad_alpha) if grad_alpha is not None else None
+        gc, gf = _grad_planes(grad_color, grad_feat, n_extra, (H, W), dev)
+        gd, ga = _f32c(grad_depth), _f32c(grad_alpha)
 
         # All parameter gradients are carved out of ONE flat buffer (64-float aligned slices): autograd
         # adopts the views as .grad, and opengaussian_b200.dist.allreduce_gradients then reduces the whole
@@ -638,41 +680,39 @@ class _RasterizeGaussians(torch.autograd.Function):
         return g_means3D, g_means2D, g_sh, g_colors, g_opac, g_scales, g_rot, g_cov, g_extra, None, None, g_sh_rest, None
 
 
-def _subset_prepare(rs, means3D, opacities, subset, num_subsets, shs, colors_precomp, scales, rotations, cov3D_precomp,
-                    extra, extra_bg):
-    """The C-ABI arguments of a subset call: (S, int32 subset, F as given, F padded to a compiled width, the padded extra
-    channels, [bg | extra_bg | 0], settings with the camera as the C ABI needs it, inputs struct)."""
+def _forward_subsets(ctx, rs, subset, num_subsets, means3D, opacities, shs, colors_precomp, scales, rotations,
+                     cov3D_precomp, extra, extra_bg):
+    """One subset call -> (color [S,3,H,W], depth [S,1,H,W], alpha [S,1,H,W], feats [S,F,H,W]).  ctx None:
+    ogs_raster_forward_subsets, forward only; else ogs_raster_forward_subsets_state, and ctx keeps what the backward
+    needs."""
+    inputs, n_extra_user, n_extra, bg, _, _, rs, ri = _prepare(
+        rs, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, extra_bg)
+    means3D = inputs[0]
     dev = means3D.device
     P = means3D.shape[0]
     S = int(num_subsets)
     if tuple(subset.shape) != (P,):
         raise _lib.OgsError(f"subset must have shape [{P}], got {tuple(subset.shape)}")
     subset = subset.to(device=dev, dtype=torch.int32).contiguous()
-    n_extra_user = 0 if extra is None else int(extra.shape[1])
-    n_extra = n_extra_user
-    if n_extra_user:
-        c_tot = next((c for c in _SUPPORTED_C if c >= 3 + n_extra_user), None)
-        if c_tot is None:
-            raise _lib.OgsError(f"extra_feats: at most {_SUPPORTED_C[-1] - 3} channels are supported")
-        if c_tot != 3 + n_extra_user:   # pad with zero channels up to a compiled width
-            extra = torch.cat([extra, extra.new_zeros(P, c_tot - 3 - n_extra_user)], 1).contiguous()
-            n_extra = c_tot - 3
-    bg = _f32c(rs.bg).reshape(-1)
-    if n_extra:
-        eb = bg.new_zeros(0) if extra_bg is None else _f32c(extra_bg).reshape(-1).to(dev)
-        bg = torch.cat([bg, eb, bg.new_zeros(n_extra - eb.numel())])
-    _, cam = camera_inputs(rs.viewmatrix, rs.projmatrix, rs.campos)
-    rs = rs._replace(viewmatrix=cam[0], projmatrix=cam[1], campos=cam[2])
-    ri = _fill_inputs(rs, bg, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, n_extra)
     ri.defer_capacity_check = 0
-    return S, subset, n_extra_user, n_extra, extra, bg, rs, ri
-
-
-def _subset_outputs(S, C, H, W, dev):
-    color_all = torch.empty(max(S, 0), C, H, W, dtype=torch.float32, device=dev)
+    H, W = int(rs.image_height), int(rs.image_width)
+    color_all = torch.empty(max(S, 0), 3 + n_extra, H, W, dtype=torch.float32, device=dev)
     depth = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
     alpha = torch.empty(max(S, 0), 1, H, W, dtype=torch.float32, device=dev)
-    return color_all, depth, alpha, _lib.SubsetOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha))
+    so = _lib.SubsetOutputs(_lib.ptr(color_all), _lib.ptr(depth), _lib.ptr(alpha))
+    alloc = _Alloc(dev)
+    args = (C.byref(ri), _lib.ptr(subset), S, C.byref(so), alloc.fn, alloc.user)
+    if ctx is None:
+        _lib.launch("ogs_raster_forward_subsets", dev, *args)
+    else:
+        st = _lib.RasterState()
+        _lib.launch("ogs_raster_forward_subsets_state", dev, *args, C.byref(st))
+        ctx.set_materialize_grads(False)
+        ctx.rs, ctx.bg, ctx.state, ctx.bufs = rs, bg, st, alloc.bufs     # bufs: the state's geom/binning/image buffers
+        ctx.S, ctx.n_extra, ctx.n_extra_user = S, n_extra, n_extra_user
+        ctx.save_for_backward(*inputs[:8])
+    feat = color_all[:, 3:3 + n_extra_user] if n_extra_user else color_all.new_empty(max(S, 0), 0, H, W)
+    return color_all[:, :3], depth, alpha, feat
 
 
 class _RasterizeSubsets(torch.autograd.Function):
@@ -682,23 +722,8 @@ class _RasterizeSubsets(torch.autograd.Function):
     @staticmethod
     def forward(ctx, means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, subset, S, rs,
                 extra_bg):
-        dev = means3D.device
-        means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra = (
-            _f32c(t) for t in (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra))
-        S, subset, n_extra_user, n_extra, extra, bg, rs, ri = _subset_prepare(
-            rs, means3D, opacities, subset, S, shs, colors_precomp, scales, rotations, cov3D_precomp, extra, extra_bg)
-        H, W = int(rs.image_height), int(rs.image_width)
-        color_all, depth, alpha, so = _subset_outputs(S, 3 + n_extra, H, W, dev)
-        st = _lib.RasterState()
-        alloc = _Alloc(dev)
-        _lib.launch("ogs_raster_forward_subsets_state", dev, C.byref(ri), _lib.ptr(subset), S, C.byref(so), alloc.fn,
-                    alloc.user, C.byref(st))
-        ctx.set_materialize_grads(False)
-        ctx.rs, ctx.bg, ctx.state, ctx.bufs = rs, bg, st, alloc.bufs     # bufs: the state's geom/binning/image buffers
-        ctx.S, ctx.n_extra, ctx.n_extra_user = S, n_extra, n_extra_user
-        ctx.save_for_backward(means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra)
-        feat = color_all[:, 3:3 + n_extra_user] if n_extra_user else color_all.new_empty(max(S, 0), 0, H, W)
-        return color_all[:, :3], depth, alpha, feat
+        return _forward_subsets(ctx, rs, subset, S, means3D, opacities, shs, colors_precomp, scales, rotations,
+                                cov3D_precomp, extra, extra_bg)
 
     @staticmethod
     @once_differentiable
@@ -710,19 +735,8 @@ class _RasterizeSubsets(torch.autograd.Function):
         H, W = int(rs.image_height), int(rs.image_width)
         need = ctx.needs_input_grad   # means3D, opacities, shs, colors_precomp, scales, rotations, cov3D, extra
 
-        # the padding rules of _RasterizeGaussians.backward, per slot
-        gc = _f32c(grad_color) if grad_color is not None else None
-        gf = None
-        if n_extra and grad_feat is not None and grad_feat.shape[1] > 0:
-            gf = _f32c(grad_feat)
-            if gf.shape[1] != n_extra:        # zero planes for the padding channels
-                gf = torch.cat([gf, gf.new_zeros(S, n_extra - gf.shape[1], H, W)], 1)
-        if n_extra and gf is None:
-            gf = torch.zeros(S, n_extra, H, W, dtype=torch.float32, device=dev)
-        if gc is None and gf is None:
-            gc = torch.zeros(S, 3, H, W, dtype=torch.float32, device=dev)
-        gd = _f32c(grad_depth) if grad_depth is not None else None
-        ga = _f32c(grad_alpha) if grad_alpha is not None else None
+        gc, gf = _grad_planes(grad_color, grad_feat, n_extra, (S, H, W), dev)
+        gd, ga = _f32c(grad_depth), _f32c(grad_alpha)
 
         def out(flag, t, *shape):
             return torch.empty(*(shape or t.shape), dtype=torch.float32, device=dev) if flag and t is not None else None
@@ -786,32 +800,14 @@ class GaussianRasterizer(nn.Module):
         ``extra_bg [F]``: F extra channels composited in the same pass (background ``extra_bg``,
         default 0).  Returns ``(color, radii, depth, alpha)`` or, with extra_feats, a fifth
         ``feats [F,H,W]``."""
-        rs = self.raster_settings
-        if means3D.shape[0] > 0:     # upstream passes torch.Tensor([]) for "not given"
-            shs, colors_precomp = _none_if_empty(shs), _none_if_empty(colors_precomp)
-            scales, rotations, cov3D_precomp = _none_if_empty(scales), _none_if_empty(rotations), _none_if_empty(cov3D_precomp)
-        if (shs is None and colors_precomp is None) or (shs is not None and colors_precomp is not None):
-            raise Exception('Please provide excatly one of either SHs or precomputed colors!')
-        if ((scales is None or rotations is None) and cov3D_precomp is None) or \
-                ((scales is not None or rotations is not None) and cov3D_precomp is not None):
-            raise Exception('Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!')
+        shs, colors_precomp, scales, rotations, cov3D_precomp = _check_inputs(
+            means3D, shs, colors_precomp, scales, rotations, cov3D_precomp)
         color, radii, depth, alpha, feat = rasterize_gaussians(
-            means3D, means2D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp, rs, extra_feats,
-            extra_bg)
+            means3D, means2D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp, self.raster_settings,
+            extra_feats, extra_bg)
         if extra_feats is None:
             return color, radii, depth, alpha
         return color, radii, depth, alpha, feat
-
-    def _subset_check(self, shs, colors_precomp, scales, rotations, cov3D_precomp, means3D):
-        if means3D.shape[0] > 0:
-            shs, colors_precomp = _none_if_empty(shs), _none_if_empty(colors_precomp)
-            scales, rotations, cov3D_precomp = _none_if_empty(scales), _none_if_empty(rotations), _none_if_empty(cov3D_precomp)
-        if (shs is None and colors_precomp is None) or (shs is not None and colors_precomp is not None):
-            raise Exception('Please provide excatly one of either SHs or precomputed colors!')
-        if ((scales is None or rotations is None) and cov3D_precomp is None) or \
-                ((scales is not None or rotations is not None) and cov3D_precomp is not None):
-            raise Exception('Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!')
-        return shs, colors_precomp, scales, rotations, cov3D_precomp
 
     def forward_subsets(self, means3D, opacities, subset, num_subsets, shs=None, colors_precomp=None, scales=None,
                         rotations=None, cov3D_precomp=None, extra_feats=None, extra_bg=None):
@@ -820,27 +816,14 @@ class GaussianRasterizer(nn.Module):
         bit for bit, ``forward()`` on the rows with ``subset == k``.  Activated inputs as for ``forward()``; forward
         only (no backward, no radii: ``forward_subsets_grad`` is the differentiable form) and outside the view cache.
         Returns ``(color [S,3,H,W], depth [S,1,H,W], alpha [S,1,H,W], feats [S,F,H,W] or None)``."""
-        rs = self.raster_settings
-        shs, colors_precomp, scales, rotations, cov3D_precomp = self._subset_check(
-            shs, colors_precomp, scales, rotations, cov3D_precomp, means3D)
+        shs, colors_precomp, scales, rotations, cov3D_precomp = _check_inputs(
+            means3D, shs, colors_precomp, scales, rotations, cov3D_precomp)
         inputs = (means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra_feats)
         if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs):
             raise _lib.OgsError("forward_subsets has no backward: call it under torch.no_grad() or with inputs that "
                                 "do not require grad")
-        dev = means3D.device
-        if dev.type != "cuda":
-            raise _lib.OgsError("GaussianRasterizer needs CUDA tensors (there is no CPU fallback)")
-        means3D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp, extra = (_f32c(t) for t in inputs)
-        S, subset, n_extra_user, n_extra, extra, bg, rs, ri = _subset_prepare(
-            rs, means3D, opacities, subset, num_subsets, shs, colors_precomp, scales, rotations, cov3D_precomp, extra,
-            extra_bg)
-        H, W = int(rs.image_height), int(rs.image_width)
-        color_all, depth, alpha, so = _subset_outputs(S, 3 + n_extra, H, W, dev)
-        alloc = _Alloc(dev)
-        _lib.launch("ogs_raster_forward_subsets", dev, C.byref(ri), _lib.ptr(subset), S, C.byref(so), alloc.fn,
-                    alloc.user)
-        feats = color_all[:, 3:3 + n_extra_user] if n_extra_user else None
-        return color_all[:, :3], depth, alpha, feats
+        color, depth, alpha, feats = _forward_subsets(None, self.raster_settings, subset, num_subsets, *inputs, extra_bg)
+        return color, depth, alpha, (feats if feats.shape[1] > 0 else None)
 
     def forward_subsets_grad(self, means3D, opacities, subset, num_subsets, shs=None, colors_precomp=None, scales=None,
                              rotations=None, cov3D_precomp=None, extra_feats=None, extra_bg=None):
@@ -851,10 +834,8 @@ class GaussianRasterizer(nn.Module):
         of no slot get zero), as ``forward()`` + backward on each slot's rows would give.  There is no ``means2D``
         input, hence no screen-space gradient: a caller that needs one renders each slot with ``forward()``.  Plain
         gradient tensors (no gradient arena, no fused accumulation), outside the view cache; no double backward."""
-        shs, colors_precomp, scales, rotations, cov3D_precomp = self._subset_check(
-            shs, colors_precomp, scales, rotations, cov3D_precomp, means3D)
-        if means3D.device.type != "cuda":
-            raise _lib.OgsError("GaussianRasterizer needs CUDA tensors (there is no CPU fallback)")
+        shs, colors_precomp, scales, rotations, cov3D_precomp = _check_inputs(
+            means3D, shs, colors_precomp, scales, rotations, cov3D_precomp)
         color, depth, alpha, feats = _RasterizeSubsets.apply(means3D, opacities, shs, colors_precomp, scales, rotations,
                                                              cov3D_precomp, extra_feats, subset, num_subsets,
                                                              self.raster_settings, extra_bg)

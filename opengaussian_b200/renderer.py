@@ -58,14 +58,34 @@ def _zero_sink(xyz):
 
 def _tiled_bg(bg3, nb):
     """bg_color repeated over the feature channels (the reference reuses one rasterizer, hence one background, for all
-    its 3-channel passes); cached per device on the background tensor's storage and version counter."""
-    sig = (bg3.data_ptr(), bg3._version, nb)
-    hit = _TILED_BG.get(bg3.device)
+    its 3-channel passes); cached per device and width on the background tensor's storage and version counter."""
+    sig = (bg3.data_ptr(), bg3._version)
+    hit = _TILED_BG.get((bg3.device, nb))
     if hit is None or hit[0] != sig:
         hit = (sig, torch.cat([bg3] * ((nb + 2) // 3))[:nb].contiguous(), bg3)     # keeps bg3 alive: the address stays its own
-        _TILED_BG[bg3.device] = hit
+        _TILED_BG[(bg3.device, nb)] = hit
     pin_for_capture(bg3.device, hit[1])
     return hit[1]
+
+
+def _feat_args(bg3, feat, shs):
+    """The colour arguments of a feature pass: the SH colours (seg_rgb), `feat` as colours, or its first 3 channels as
+    colours and the rest as extra channels."""
+    if shs is not None:
+        return dict(shs=shs)
+    if feat.shape[-1] > 3:
+        return dict(colors_precomp=feat[:, :3], extra_feats=feat[:, 3:], extra_bg=_tiled_bg(bg3, feat.shape[-1] - 3))
+    return dict(colors_precomp=feat)
+
+
+def _feat_image(color, extra, shs, dim):
+    """The image of a feature pass from the rasterizer's colour and extra channels (channels at `dim`): with shs the RGB
+    image duplicated, as the reference does."""
+    if shs is not None:
+        return torch.cat((color, color), dim=dim)
+    if extra is not None:
+        return torch.cat((color, extra), dim=dim)
+    return color
 
 
 def _feat_pass(rasterizer, bg3, means3D, means2D, opacity, scales, rotations, cov3D_precomp, feat, shs=None,
@@ -81,21 +101,10 @@ def _feat_pass(rasterizer, bg3, means3D, means2D, opacity, scales, rotations, co
                                        opacities=opacity, scales=scales, rotations=rotations,
                                        cov3D_precomp=cov3D_precomp)
         return torch.cat((img, img2), dim=0), alpha
-    if shs is not None:
-        img, _, _, alpha = rasterizer(means3D=means3D, means2D=means2D, shs=shs, colors_precomp=None,
-                                      opacities=opacity, scales=scales, rotations=rotations,
-                                      cov3D_precomp=cov3D_precomp)
-        return torch.cat((img, img), dim=0), alpha
-    if feat.shape[-1] > 3:
-        nb = feat.shape[-1] - 3
-        ebg = torch.cat([bg3] * ((nb + 2) // 3))[:nb]
-        img, _, _, alpha, img2 = rasterizer(means3D=means3D, means2D=means2D, shs=None, colors_precomp=feat[:, :3],
-                                            opacities=opacity, scales=scales, rotations=rotations,
-                                            cov3D_precomp=cov3D_precomp, extra_feats=feat[:, 3:], extra_bg=ebg)
-        return torch.cat((img, img2), dim=0), alpha
-    img, _, _, alpha = rasterizer(means3D=means3D, means2D=means2D, shs=None, colors_precomp=feat,
-                                  opacities=opacity, scales=scales, rotations=rotations, cov3D_precomp=cov3D_precomp)
-    return img, alpha
+    img, _, _, alpha, *extra = rasterizer(means3D=means3D, means2D=means2D, opacities=opacity, scales=scales,
+                                          rotations=rotations, cov3D_precomp=cov3D_precomp,
+                                          **_feat_args(bg3, feat, shs))
+    return _feat_image(img, extra[0] if extra else None, shs, 0), alpha
 
 
 # ---- the coarse-cluster and leaf passes of render(): a planning step and a render step ----
@@ -196,8 +205,11 @@ def _plan_leaves(leaf_cluster_idx, lerf_range, selected_leaf_id, pre_mask, viewe
     return [cand[k] for k in kept], subset
 
 
-def _needs_grad(*inputs):
-    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs)
+def _slot_route(fused, batched, means2D, *inputs):
+    """_subset_route in the current grad mode: a gradient is needed when grad is enabled and one of `inputs` requires
+    it."""
+    needs_grad = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in inputs)
+    return _subset_route(fused, batched, needs_grad, means2D.requires_grad)
 
 
 def _subset_route(fused, batched, needs_grad, means2D_grad):
@@ -215,24 +227,17 @@ def _subset_route(fused, batched, needs_grad, means2D_grad):
     return "loop" if means2D_grad else "batched_grad"
 
 
-def _use_batched(fused, batched, means2D, *inputs):
-    """One subset call for all slots (forward_subsets, or forward_subsets_grad when an input needs a gradient) unless
-    _subset_route keeps the loop."""
-    return _subset_route(fused, batched, _needs_grad(*inputs), means2D.requires_grad) != "loop"
-
-
 def _render_slots(rasterizer, bg3, ids, subset, means3D, means2D, opacity, scales, rotations, cov3D_precomp, feat, shs,
                   fused, keep_min_alpha=None, batched=True):
     """The images of the planned slots -> (images, silhouettes), lists in slot order, each entry as _feat_pass returns it.
     keep_min_alpha: keep only the slots whose silhouette exceeds it somewhere (the coarse loop's test, :222), and
     remove the others from `ids` in place.  batched=False: the loop (pipe.batched_subsets)."""
     imgs, sils = [], []
-    inputs = (means3D, opacity, scales, rotations, cov3D_precomp, feat, shs)
-    if _use_batched(fused, batched, means2D, *inputs):
-        grad = _needs_grad(*inputs)
+    route = _slot_route(fused, batched, means2D, means3D, opacity, scales, rotations, cov3D_precomp, feat, shs)
+    if route != "loop":
         keep_ids = []
         for a, b, img, sil in _render_slots_batched(rasterizer, bg3, len(ids), subset, means3D, opacity, scales,
-                                                    rotations, cov3D_precomp, feat, shs, grad):
+                                                    rotations, cov3D_precomp, feat, shs, route == "batched_grad"):
             if keep_min_alpha is not None:
                 keep = (sil.amax(dim=(1, 2, 3)) > keep_min_alpha).tolist()       # one host read per launch
                 sel = [k for k in range(b - a) if keep[k]]
@@ -271,13 +276,8 @@ def _render_slots_batched(rasterizer, bg3, S, subset, means3D, opacity, scales, 
     _feat_pass."""
     rs = rasterizer.raster_settings
     H, W = int(rs.image_height), int(rs.image_width)
-    if shs is not None:
-        nb, kw = 0, dict(shs=shs)
-    elif feat.shape[-1] > 3:
-        nb = feat.shape[-1] - 3
-        kw = dict(colors_precomp=feat[:, :3], extra_feats=feat[:, 3:], extra_bg=torch.cat([bg3] * ((nb + 2) // 3))[:nb])
-    else:
-        nb, kw = 0, dict(colors_precomp=feat)
+    kw = _feat_args(bg3, feat, shs)
+    nb = kw["extra_feats"].shape[-1] if "extra_feats" in kw else 0
     per_launch = max(1, SUBSET_BATCH_BYTES // (((3 + nb + 2) * 4 + (8 if grad else 0)) * H * W))
     call = rasterizer.forward_subsets_grad if grad else rasterizer.forward_subsets
     for a in range(0, S, per_launch):
@@ -285,13 +285,7 @@ def _render_slots_batched(rasterizer, bg3, S, subset, means3D, opacity, scales, 
         sub = subset if (a == 0 and b == S) else torch.where((subset >= a) & (subset < b), subset - a, -1)
         color, _, alpha, extra = call(means3D, opacity, sub, b - a, scales=scales, rotations=rotations,
                                       cov3D_precomp=cov3D_precomp, **kw)
-        if shs is not None:
-            img = torch.cat((color, color), dim=1)
-        elif extra is not None:
-            img = torch.cat((color, extra), dim=1)
-        else:
-            img = color.contiguous()
-        yield a, b, img, alpha
+        yield a, b, _feat_image(color, extra, shs, 1), alpha
 
 
 def render(viewpoint_camera, pc, pipe, bg_color: torch.Tensor, iteration,

@@ -67,11 +67,11 @@ class Counter:
 
 def run(cams, model, calls, batched):
     """render() of every call on every camera; returns the last camera's outputs."""
-    renderer._use_batched = (lambda fused, *t: fused) if batched else (lambda fused, *t: False)
+    pipe = types.SimpleNamespace(batched_subsets=batched, **vars(PIPE))
     out = None
     with torch.no_grad():
         for cam in cams:
-            out = [renderer.render(cam, model, PIPE, BG, 1000, **kw) for kw in calls]
+            out = [renderer.render(cam, model, pipe, BG, 1000, **kw) for kw in calls]
     return out
 
 

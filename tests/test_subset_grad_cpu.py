@@ -88,14 +88,15 @@ def test_subset_route():
     assert route(True, False, True, False) == "loop"
 
 
-def test_use_batched_reads_grad_mode():
+def test_slot_route_reads_grad_mode():
     import torch
     x = torch.zeros(3, 3)
     feat = torch.zeros(3, 6, requires_grad=True)
     sink = torch.zeros(3, 3, requires_grad=True)
-    assert renderer._use_batched(True, True, x, x, feat)                 # grad flows to feat: forward_subsets_grad
-    assert not renderer._use_batched(True, True, sink, x, feat)          # trainable screen-space points: the loop
-    assert not renderer._use_batched(True, False, x, x, feat)            # pipe.batched_subsets = False
+    route = renderer._slot_route
+    assert route(True, True, x, x, feat) == "batched_grad"               # grad flows to feat: forward_subsets_grad
+    assert route(True, True, sink, x, feat) == "loop"                    # trainable screen-space points: the loop
+    assert route(True, False, x, x, feat) == "loop"                      # pipe.batched_subsets = False
     with torch.no_grad():
-        assert renderer._use_batched(True, True, sink, x, feat)          # no gradient at all: forward_subsets
-        assert not renderer._use_batched(False, True, x, x, feat)
+        assert route(True, True, sink, x, feat) == "batched"             # no gradient at all: forward_subsets
+        assert route(False, True, x, x, feat) == "loop"
