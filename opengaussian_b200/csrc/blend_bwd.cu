@@ -45,11 +45,21 @@ struct HalvingReduce {
             if constexpr (CUR > 1) {
                 constexpr int HALF = CUR / 2;
                 const bool upper = (lane & M) != 0;
+                if constexpr (HALF == 1) {
+                    const float send = upper ? v[0] : v[1];
+                    const float keep = upper ? v[1] : v[0];
+                    v[0] = keep + __shfl_xor_sync(0xffffffffu, send, M);
+                } else {
+                    // two values per FADD2
 #pragma unroll
-                for (int k = 0; k < HALF; k++) {
-                    const float send = upper ? v[k] : v[k + HALF];
-                    const float keep = upper ? v[k + HALF] : v[k];
-                    v[k] = keep + __shfl_xor_sync(0xffffffffu, send, M);
+                    for (int k = 0; k < HALF; k += 2) {
+                        const float2 keep = upper ? make_float2(v[k + HALF], v[k + 1 + HALF]) : make_float2(v[k], v[k + 1]);
+                        const float2 send = upper ? make_float2(v[k], v[k + 1]) : make_float2(v[k + HALF], v[k + 1 + HALF]);
+                        const float2 sum = __fadd2_rn(keep, make_float2(__shfl_xor_sync(0xffffffffu, send.x, M),
+                                                                        __shfl_xor_sync(0xffffffffu, send.y, M)));
+                        v[k] = sum.x;
+                        v[k + 1] = sum.y;
+                    }
                 }
                 HalvingReduce<HALF, M / 2>::run(v, lane);
             } else {
@@ -64,12 +74,14 @@ constexpr int floor_pow2(int v) { return v >= 16 ? 16 : (v >= 8 ? 8 : (v >= 4 ? 
 constexpr int log2c(int v) { return v <= 1 ? 0 : 1 + log2c(v / 2); }
 
 // Sums v[BASE..BASE+N) over the 32 lanes, chunk by chunk (largest power of two first), and stores
-// the totals to row[BASE..BASE+N): after a chunk of S values, lane l with (l % (32/S)) == 0 holds
-// the total of value l / (32/S).
+// the totals to row[BASE..BASE+N): after a chunk of S values, every lane l holds the total of value
+// l / (32/S) (the last log2(32/S) steps are butterflies, and the 32/S lanes of a value add the same
+// partial sums in commuted order, so their totals are bit-identical).  They all store it: no predicate
+// and no lane test per store.
 template <int N, int BASE>
 struct ChunkReduceStore {
     template <int VT>
-    __device__ __forceinline__ static void run(const float (&v)[VT], int lane, float* row) {
+    __device__ __forceinline__ static void run(const float (&v)[VT], int lane, uint32_t row) {   // row: shared address
         if constexpr (N > 0) {
             constexpr int S = floor_pow2(N);
             constexpr int SH = 5 - log2c(S);
@@ -77,7 +89,7 @@ struct ChunkReduceStore {
 #pragma unroll
             for (int k = 0; k < S; k++) t[k] = v[BASE + k];
             HalvingReduce<S, 16>::run(t, lane);
-            if ((lane & ((1 << SH) - 1)) == 0) row[BASE + (lane >> SH)] = t[0];
+            asm volatile("st.shared.f32 [%0], %1;" :: "r"(row + 4u * (BASE + (lane >> SH))), "f"(t[0]) : "memory");
             ChunkReduceStore<N - S, BASE + S>::run(v, lane, row);
         }
     }
@@ -92,7 +104,23 @@ int blend_bwd_stride(int C, int geom) { return geom ? C + 7 : C; }
 // registers without spills, which lets 12 CTAs of 64 threads share an SM instead of 10.  Measured on B200 (ncu,
 // profiles/r2_kernels_full.csv): warps active 28 -> 33 %, issue active 67 -> 70 %, but 7 % more instructions
 // (rematerialisation), so the net is small: 0.517 ms capped vs 0.531 ms uncapped in the same bench run.
-constexpr int bwd_min_blocks(int C, int pairs, bool geom = true) { return (pairs == 2 && (C <= 4 || (!geom && C <= 6))) ? 12 : 1; }
+// The per-warp survivor records (below) make ptxas take 4-9 more registers where it is not capped.  The instantiations
+// that launch_cg picks by default are held to the CTAs per SM they had without the records (register-limited, 64 or
+// 128 threads): 12 for the 3- and 4-channel geometry backward, 14 / 16 / 10 / 14 / 12 for the colour backwards, 4 for
+// the 12- and 16-channel geometry backward and 5-7 for their colour backwards.  The 6- and 9-channel geometry
+// backwards keep 6 CTAs on their own.
+constexpr int bwd_min_blocks(int C, int C0, bool geom, int pairs) {
+    if (pairs == 2 && C <= 9) {
+        if (geom) return C <= 4 ? 12 : 1;
+        if (C0 > 0) return C - C0 <= 1 ? 16 : (C - C0 <= 3 ? 14 : 12);
+        return C <= 4 ? 14 : 10;
+    }
+    if (pairs == 1 && C >= 12) {
+        if (geom) return 4;
+        return C0 > 0 ? (C <= 12 ? 7 : 5) : (C <= 12 ? 6 : 5);
+    }
+    return 1;   // the other combinations are reached only through OGS_BWD_PAIRS
+}
 
 // C0 > 0 (colour-only backward, GEOM = false): channels [0, C0) carry no incoming gradient -- OpenGaussian's Stage 1
 // back-propagates through the 6 feature channels only (train.py:441-456), the RGB planes of the fused pass have no
@@ -100,7 +128,7 @@ constexpr int bwd_min_blocks(int C, int pairs, bool geom = true) { return (pairs
 // (6 of 9 values: a third of the FFMA2s and of the reduction of every evaluated entry).  The accumulator rows keep
 // their C columns (preprocess_bwd reads them by column); columns [0, C0) stay zero.
 template <int C, bool GEOM, int PAIRS, int C0 = 0, bool SUBSETS = false>
-__global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEOM || C0 == 0)) blend_bwd_kernel(BlendBwdArgs a) {
+__global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C, C0, GEOM, PAIRS)) blend_bwd_kernel(BlendBwdArgs a) {
     static_assert(C0 == 0 || !GEOM, "the geometry gradients need every channel");
     constexpr int BWD_THREADS = 128 / PAIRS, BWD_WARPS = 4 / PAIRS, NPX = 2 * PAIRS;
     constexpr int V = GEOM ? C + 7 : C;
@@ -114,6 +142,10 @@ __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEO
     __shared__ float2 s_b2[2][BB];
     __shared__ __align__(16) float s_ch2[2][BB * CH];
     __shared__ uint32_t s_id3[3][BB];     // ids live until the batch's flush, i.e. while batch b-2 is already being staged: 3 slots
+    // per warp, the current group's surviving entries back to front, two float4 each: the staged sa and {sb, list
+    // position, shared addresses of the entry's accumulator row and channels}.  The entry loop walks consecutive
+    // records instead of locating each set bit of the ballot and re-deriving the addresses from it.
+    __shared__ float4 s_hit[BWD_WARPS][32 * 2];
     __shared__ int s_max_last;
 
     const int gx = (a.W + 15) / 16;
@@ -220,14 +252,24 @@ __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEO
                 const int idx = grp + lane;
                 bool hit = false;
                 if (idx < nw) hit = ogs_rect_hit_s(s_a[idx], s_b[idx], bx0, by0, bx0 + 7.0f, by0 + (float)(8 * PAIRS - 1));
-                unsigned mask = __ballot_sync(0xffffffffu, hit);
-                while (mask) {
-                    const int bit = 31 - __clz(mask);
-                    mask &= ~(1u << bit);
-                    const int j = grp + bit;
-                    const int pos = start + j;
-                    const float4 ra = s_a[j];
-                    const float2 rb = s_b[j];
+                const unsigned mask = __ballot_sync(0xffffffffu, hit);
+                float4* hits = s_hit[warp];
+                if (hit) {   // (re-read: keeping the record live across the test costs spills at the 80-register cap)
+                    float4* h = hits + 2 * __popc(mask & ~((2u << lane) - 1u));   // rank among the later survivors
+                    const float2 rb = s_b[idx];
+                    // shared addresses of the accumulator row (4-byte aligned, < 2^18) and of the channels (16-byte
+                    // aligned), packed into one word: the loop loads and stores through them with no base to rebuild
+                    const uint32_t row = (uint32_t)__cvta_generic_to_shared(my_acc + idx * V + C0);
+                    const uint32_t chs = GEOM ? (uint32_t)__cvta_generic_to_shared(s_ch + idx * CH) : 0u;   // unread without GEOM: s_ch2 stays unallocated
+                    h[0] = s_a[idx];
+                    h[1] = make_float4(rb.x, rb.y, __int_as_float(start + idx), __uint_as_float((row >> 2) | ((chs >> 4) << 16)));
+                }
+                __syncwarp();
+                const float4* const hend = hits + 2 * __popc(mask);
+                for (const float4* h = hits; h != hend; h += 2) {
+                    const float4 ra = h[0];
+                    const float4 rb = h[1];
+                    const int pos = __float_as_int(rb.z);
                     const float dx = ra.x - pxf;
                     const float adx = __fmul_rn(__fmul_rn(ra.z, dx), dx), bdx = __fmul_rn(ra.w, dx);
                     float2 dy[PAIRS], G[PAIRS], al[PAIRS];
@@ -249,8 +291,11 @@ __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEO
                     if constexpr (GEOM) {
 #pragma unroll
                         for (int q = 0; q < CH / 4; q++) {
-                            const float4 t = reinterpret_cast<const float4*>(s_ch + j * CH)[q];
-                            chv[4 * q] = t.x; chv[4 * q + 1] = t.y; chv[4 * q + 2] = t.z; chv[4 * q + 3] = t.w;
+                            // s_ch2[sb] is written by stage() before the __syncthreads that precedes this traversal;
+                            // the "memory" clobber keeps the load behind that barrier if the staging ever moves
+                            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
+                                         : "=f"(chv[4 * q]), "=f"(chv[4 * q + 1]), "=f"(chv[4 * q + 2]), "=f"(chv[4 * q + 3])
+                                         : "r"(((__float_as_uint(rb.w) >> 16) << 4) + 16u * q) : "memory");
                         }
                     }
                     // packed sums over the lane's pairs; .x + .y is taken once at the end
@@ -299,8 +344,9 @@ __global__ void __launch_bounds__(128 / PAIRS, bwd_min_blocks(C - C0, PAIRS, GEO
                         v[C + 5] = suy * dx;
                         v[C + 6] = suyy2.x + suyy2.y;
                     }
-                    ChunkReduceStore<VG, 0>::run(v, lane, my_acc + j * V + C0);
+                    ChunkReduceStore<VG, 0>::run(v, lane, (__float_as_uint(rb.w) & 0xffffu) << 2);
                 }
+                __syncwarp();   // the records are read before the next group overwrites them
             }
         }
         __syncthreads();   // batch b fully traversed by every warp; batch b-1 fully staged

@@ -122,19 +122,21 @@ __global__ void __launch_bounds__(128 / PAIRS) blend_fwd_kernel(BlendFwdArgs a) 
                         al.y = fminf(0.99f, al.y);
                         const bool oka = pw.x <= 0.0f && al.x >= (1.0f / 255.0f);
                         const bool okb = pw.y <= 0.0f && al.y >= (1.0f / 255.0f);
+                        // a skipped entry gets alpha 0, so tT = T exactly and the one floor test below also covers it
+                        const float2 alm = make_float2(oka ? al.x : 0.0f, okb ? al.y : 0.0f);
                         const float2 T = T2[p];
-                        const float2 tT = __fmul2_rn(T, __fadd2_rn(s2(1.0f), make_float2(-al.x, -al.y)));
-                        const float2 w = __fmul2_rn(al, T);
-                        // apply: valid alpha and the pixel stays above the transmittance floor (false once T <= 0)
-                        const bool apa = oka && tT.x >= 0.0001f, apb = okb && tT.y >= 0.0001f;
-                        const float2 wm = make_float2(apa ? w.x : 0.0f, apb ? w.y : 0.0f);
+                        const float2 tT = __fmul2_rn(T, __fadd2_rn(s2(1.0f), make_float2(-alm.x, -alm.y)));
+                        const float2 w = __fmul2_rn(alm, T);
+                        // live: the pixel stays above the transmittance floor (false once T <= 0); a live skipped entry
+                        // adds w = 0 and keeps T, a valid alpha that reaches the floor stops the pixel without being
+                        // applied (T <- -|T|, which leaves a finished pixel's T as it is)
+                        const bool lva = tT.x >= 0.0001f, lvb = tT.y >= 0.0001f;
+                        const float2 wm = make_float2(lva ? w.x : 0.0f, lvb ? w.y : 0.0f);
 #pragma unroll
                         for (int c = 0; c <= C; c++) acc[p][c] = __ffma2_rn(s2(chv[c]), wm, acc[p][c]);
-                        // stop (valid alpha, floor reached): this Gaussian is NOT applied, T <- -|T|
-                        T2[p] = make_float2((oka && !apa) ? -fabsf(T.x) : (apa ? tT.x : T.x),
-                                            (okb && !apb) ? -fabsf(T.y) : (apb ? tT.y : T.y));
-                        last[2 * p] = apa ? pos : last[2 * p];
-                        last[2 * p + 1] = apb ? pos : last[2 * p + 1];
+                        T2[p] = make_float2(lva ? tT.x : -fabsf(T.x), lvb ? tT.y : -fabsf(T.y));
+                        last[2 * p] = (oka && lva) ? pos : last[2 * p];
+                        last[2 * p + 1] = (okb && lvb) ? pos : last[2 * p + 1];
                     }
                 }
                 if (__all_sync(0xffffffffu, all_done())) break;
