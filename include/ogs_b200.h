@@ -54,6 +54,8 @@
  *   ogs_cohesion_forward/backward
  *                                train.py:102-121 (cohesion_loss)
  *   ogs_separation_loss          train.py:123-155 (separation_loss)
+ *   ogs_knn_segmented            pytorch3d.ops.knn_points, which gaussian_renderer/__init__.py's post_process calls once
+ *                                per leaf (:315-322): here for all leaves of a view, or all clouds of a batch, at once
  */
 #ifndef OGS_B200_H
 #define OGS_B200_H
@@ -456,6 +458,23 @@ typedef struct ogs_adam_tensor {
     float reserved_;
 } ogs_adam_tensor;
 int ogs_adam_step(int32_t n_tensors, const ogs_adam_tensor* tensors, float grad_scale, void* stream);
+
+/* ---- exact k-nearest neighbours within segments (pytorch3d.ops.knn_points; render()'s post_process for all leaves) ----
+ * q [Q,3] queries, q_seg int32 [Q] the segment of each query; p [M,3] the candidates in segment order with CSR offsets
+ * p_off int64 [S+1] (segment s = rows [p_off[s], p_off[s+1]) of p); k_seg int32 [S] the K of each segment (device: no
+ * host read).  A query sees only its own segment's candidates, itself included when it is one of them.  Squared
+ * distance = (dx*dx + dy*dy) + dz*dz in float32, every operation rounded on its own (no FMA).  The K used for a query
+ * is min(k_seg, segment size), and with a neighbour list also min(., k_max); a query whose segment is outside [0, S) or
+ * whose K is 0 gets 0 in kth_dist / dist_sum / dist_sumsq and no list entries.  Outputs, each may be NULL (not all):
+ *   kth_dist [Q]         the K-th smallest squared distance
+ *   dist_sum, dist_sumsq double [Q]: sum and sum of squares of the K smallest squared distances, accumulated in fp64
+ *   nn_dist [Q,k_max], nn_idx int64 [Q,k_max] (both or neither): the K nearest ordered by (distance, index), the index
+ *                        relative to the segment's first row; entries K..k_max-1 of a row are not written.
+ * One warp per query: a radix select of the K-th distance (three passes over the segment), then one collect pass.
+ * With a neighbour list and k_max > 1024 the call takes Q * k_max * 8 bytes from the stream-ordered pool. */
+int ogs_knn_segmented(int64_t Q, const float* q, const int32_t* q_seg, int32_t S, const float* p, const int64_t* p_off,
+                      const int32_t* k_seg, int32_t k_max, float* kth_dist, double* dist_sum, double* dist_sumsq,
+                      float* nn_dist, int64_t* nn_idx, void* stream);
 
 #ifdef __cplusplus
 }

@@ -125,6 +125,8 @@ EXPORTS = {
     "ogs_adam_step": (C.c_int, [C.c_int32, C.c_void_p, C.c_float, C.c_void_p]),
     "ogs_mask_iou_scratch_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int64]),
     "ogs_mask_pair_counts": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, _fp, _fp, _fp, _fp, _fp, C.c_void_p]),
+    "ogs_knn_segmented": (C.c_int, [C.c_int64, _fp, _fp, C.c_int32, _fp, _fp, _fp, C.c_int32, _fp, _fp, _fp, _fp, _fp,
+                                    C.c_void_p]),
 }
 
 _LIB = None

@@ -16,7 +16,8 @@ OBJ = os.path.join(CSRC, "build")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
           "--expt-relaxed-constexpr", "-Xptxas", "-v"]
-# translation units; preprocess.cu / binning.cu carry the bit-exact arithmetic contract (no FMA contraction)
+# translation units; preprocess.cu / binning.cu carry the bit-exact arithmetic contract (no FMA contraction), knn.cu
+# computes its distances in the direct form with every operation rounded on its own
 UNITS = {
     "preprocess.cu": ["--fmad=false"],
     "binning.cu": ["--fmad=false"],
@@ -34,6 +35,7 @@ UNITS = {
     "adam.cu": [],
     "footprint.cu": [],
     "subsets.cu": [],
+    "knn.cu": ["--fmad=false"],
     "capi.cu": [],
 }
 

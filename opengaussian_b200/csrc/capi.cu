@@ -1005,4 +1005,24 @@ int ogs_adam_step(int32_t n_tensors, const ogs_adam_tensor* tensors, float grad_
     return 0;
 }
 
+int ogs_knn_segmented(int64_t Q, const float* q, const int32_t* q_seg, int32_t S, const float* p, const int64_t* p_off,
+                      const int32_t* k_seg, int32_t k_max, float* kth_dist, double* dist_sum, double* dist_sumsq,
+                      float* nn_dist, int64_t* nn_idx, void* stream_) {
+    const bool nn = nn_dist || nn_idx;
+    if (Q < 0 || S < 0 || Q > (int64_t)INT32_MAX * 4 || (Q > 0 && (!q || !q_seg)) || (S > 0 && (!p || !p_off || !k_seg))) {
+        set_error("knn_segmented: bad sizes or pointers (Q=%lld S=%d)", (long long)Q, S);
+        return -1;
+    }
+    if (nn && (!nn_dist || !nn_idx || k_max < 1)) {
+        set_error("knn_segmented: a neighbour list needs nn_dist, nn_idx and k_max >= 1 (k_max=%d)", k_max);
+        return -1;
+    }
+    if (!nn && !kth_dist && !dist_sum && !dist_sumsq) { set_error("knn_segmented: no output requested"); return -1; }
+    if (Q == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream_;
+    int rc = ensure_pool();
+    if (rc) return rc;
+    return launch_knn_segmented(Q, q, q_seg, S, p, p_off, k_seg, k_max, kth_dist, dist_sum, dist_sumsq, nn_dist, nn_idx, s);
+}
+
 }  // extern "C"

@@ -355,4 +355,9 @@ int launch_footprint_votes(int P, int W, int H, const GeomPtrs& g, const int32_t
 // optimiser step (adam.cu)
 int launch_adam_step(int n_tensors, const ogs_adam_tensor* tensors, float grad_scale, cudaStream_t s);
 
+// exact k-nearest-neighbour selection within segments (knn.cu)
+int launch_knn_segmented(int64_t Q, const float* q, const int32_t* q_seg, int32_t S, const float* p, const int64_t* p_off,
+                         const int32_t* k_seg, int32_t k_max, float* kth, double* sum, double* sumsq, float* nn_dist,
+                         int64_t* nn_idx, cudaStream_t s);
+
 }  // namespace ogs

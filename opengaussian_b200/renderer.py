@@ -23,6 +23,7 @@ import math
 
 import torch
 
+from . import knn
 from .rasterizer import GaussianRasterizationSettings, GaussianRasterizer, pin_for_capture
 from .rasterizer import view_cache as _view_cache
 
@@ -145,6 +146,27 @@ def _post_process(filter_idx, means3D):
     return filter_idx
 
 
+def _post_process_slots(subset, S, means3D):
+    """_post_process for every slot of the slot map `subset` at once (CUDA tensors) -> (subset with the removed points
+    at -1, kept points per slot as a host list).  Per slot: K = int(n ** 0.5) as the reference computes it, mean and
+    unbiased std over all n * K distances of the slot's kNN matrix (from fp64 per-point sums), keep a point when its
+    mean over K is below mean + std.  One kNN launch for all slots and one host read.  An empty slot keeps 0 points
+    (where _post_process raises, as the reference's kNN does on an empty cloud)."""
+    if S == 0:
+        return subset, []
+    s1, s2, n, k = knn.slot_knn_sums(means3D.detach(), subset, S)
+    inside = subset >= 0
+    seg = subset.long().clamp_min(0)                  # the points of no slot have zero sums
+    tot = torch.zeros(S, dtype=torch.float64, device=subset.device).index_add_(0, seg, s1)
+    tot2 = torch.zeros_like(tot).index_add_(0, seg, s2)
+    cnt = (n * k).double()
+    mean = tot / cnt
+    std = ((tot2 - tot * mean) / (cnt - 1)).clamp_min(0).sqrt()      # NaN for one value, as torch.std: nothing kept
+    keep = inside & (s1 / k[seg] < (mean + std)[seg])
+    kept = torch.zeros(S, dtype=torch.int64, device=subset.device).index_add_(0, seg, keep.long()).tolist()
+    return torch.where(keep, subset, -1).to(torch.int32), kept
+
+
 def _plan_clusters(cluster_idx, num_cluster, viewed_pts, scale_filter, better_vis, selected_root_id, cluster_occur_cam):
     """Coarse clusters of the loop :173-236 that reach the rasterizer, in loop order -> (cluster ids, slot map).  Filter of
     cluster idx: cluster_idx == idx, visible, and with better_vis all scales < 0.5 and at least 100 such points (the
@@ -169,7 +191,9 @@ def _plan_leaves(leaf_cluster_idx, lerf_range, selected_leaf_id, pre_mask, viewe
     Filter of leaf idx: leaf_cluster_idx == idx (with selected_leaf_id: any of those leaves), & pre_mask, visible; with
     better_vis all scales < 0.1 and at least 100 points; then post_process's outlier removal; then at least 10 points.
     With selected_leaf_id every iteration has the same filter and the loop stops after the first pass: at most one
-    slot.  Without post_process the counts of all leaves come from one bincount."""
+    slot.  Without post_process the counts of all leaves come from one bincount.  On CUDA tensors post_process runs for
+    all leaves at once (_post_process_slots); there a leaf with no points is dropped, where the per-leaf loop (CPU
+    tensors) raises as the reference does."""
     base = viewed_pts if pre_mask is None else pre_mask & viewed_pts
     if better_vis:
         base = base & scale_filter
@@ -177,9 +201,13 @@ def _plan_leaves(leaf_cluster_idx, lerf_range, selected_leaf_id, pre_mask, viewe
         filt = (leaf_cluster_idx.unsqueeze(1) == selected_leaf_id).any(dim=1) & base
         if not lerf_range or (better_vis and filt.sum() < 100):
             return [], _slot_map(leaf_cluster_idx, filt, [])
-        if post_process:
+        n_kept = None
+        if post_process and filt.is_cuda:
+            sub, (n_kept,) = _post_process_slots(torch.where(filt, 0, -1).to(torch.int32), 1, means3D)
+            filt = sub == 0
+        elif post_process:
             filt = _post_process(filt, means3D)
-        if filt.sum() < 10:
+        if (filt.sum() if n_kept is None else n_kept) < 10:
             return [], _slot_map(leaf_cluster_idx, filt, [])
         return [lerf_range[0]], torch.where(filt, 0, -1).to(torch.int32)
     if not lerf_range:
@@ -191,13 +219,17 @@ def _plan_leaves(leaf_cluster_idx, lerf_range, selected_leaf_id, pre_mask, viewe
         cand = [idx for idx in cand if count(idx) >= 10]
         return cand, _slot_map(leaf_cluster_idx, base, cand)
     subset = _slot_map(leaf_cluster_idx, base, cand)
-    kept = []
-    for k, idx in enumerate(cand):
-        filt = subset == k
-        post = _post_process(filt, means3D)
-        subset = torch.where(filt & ~post, -1, subset).to(torch.int32)
-        if post.sum() >= 10:
-            kept.append(k)
+    if subset.is_cuda:
+        subset, counts = _post_process_slots(subset, len(cand), means3D)
+        kept = [k for k, c in enumerate(counts) if c >= 10]
+    else:
+        kept = []
+        for k, idx in enumerate(cand):
+            filt = subset == k
+            post = _post_process(filt, means3D)
+            subset = torch.where(filt & ~post, -1, subset).to(torch.int32)
+            if post.sum() >= 10:
+                kept.append(k)
     lut = torch.full((len(cand) + 1,), -1, dtype=torch.int32, device=subset.device)     # renumber the kept slots
     lut[torch.tensor(kept, dtype=torch.long, device=subset.device)] = torch.arange(len(kept), dtype=torch.int32,
                                                                                   device=subset.device)
